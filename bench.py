@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the driver's measurement contract for the per-pixel render path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c3|c4|c5] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c3|c4|c5] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one frame of the configured scene: zero the float4 accumulator, render `spp` samples per pixel into it
 (wavefront pipeline, librt_b200.so), sum the accumulators of all ranks and finalise (/spp, saturate, sqrt, Y-flip +
@@ -21,6 +21,11 @@ samples per pixel split across the ranks).
 stated baseline — the reference ships no CPU renderer) for c1, and the reference harness for the other configs; that arm
 never loads librt_b200.so: the scenes are flat files written at build time (oracle/_ref/scenes/) and read with pure ctypes.
 The `cpu_baseline` leg times the reference headers compiled for the host cores on a bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step handed its caller on rank 0 as DIR/<name>.npy (float32): `rgb` (the
+finished frame), `rgb8` (its 8-bit pixels) and, with one GPU, `accum` (the float4 accumulator).  The scenes are built in and
+the random numbers are keyed on pixel, sample and bounce, so the same arguments give the same inputs on every run and two
+builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -307,10 +312,41 @@ class FrameLoop:
         ms_finish = float(np.mean([e[2].elapsed_time(e[3]) for e in ev]))
         return ms, ms_render, ms_finish, rays, launches, iters
 
+    def outputs(self) -> dict:
+        """what the last step handed its caller on rank 0: the frame as floats and as 8-bit pixels, and with one rank the
+        accumulator it was finalised from (with several, each rank's accumulator holds only its own samples)"""
+        if self.group is not None:
+            rgb, rgb8 = np.empty((self.H, self.W, 3), np.float32), np.empty((self.H, self.W, 3), np.uint8)
+            self.group.read_frame(rgb, rgb8)
+            out = {"rgb": rgb, "rgb8": rgb8}
+        else:
+            self.stream.synchronize()
+            out = {"rgb": self.rgb.cpu().numpy(), "rgb8": self.rgb8.cpu().numpy()}
+        if self.world == 1:
+            out["accum"] = self.accum.cpu().numpy()
+        return out
+
     def close(self):
         if self.group is not None:
             self.group.close()
         self.scene.close()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes [H, W, C] arrays as <name>.npy in float32.  When they exceed DUMP_BYTES together, every array keeps the
+    same fixed, seeded sample of pixels in ascending order ([n, C]), so that dumps of two builds still line up."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    h, w = next(iter(arrays.values())).shape[:2]
+    bytes_per_pixel = 4 * sum(a.shape[2] for a in arrays.values())
+    n = min(h * w, (DUMP_BYTES - 4096) // bytes_per_pixel)  # (4096: room for the .npy headers)
+    pick = None if n == h * w else np.sort(np.random.default_rng(0).choice(h * w, n, replace=False))
+    for name, a in arrays.items():
+        a = a.astype(np.float32)
+        np.save(out / f"{name}.npy", a if pick is None else a.reshape(h * w, -1)[pick])
 
 
 def roofline_of(cfg_key, rays_rank, ms_render, n_step_launches, peaks, l2_gbs, kernel_name):
@@ -377,6 +413,11 @@ def run_ours(args) -> None:
         ms_step, ms_render, ms_finish, rays_rank, launches_render, iters = loop.timed(args.steps, args.warmup, flush)
         t_wall = time.perf_counter() - t_wall0
         clocks = sampler.stop() if sampler else None
+        if args.dump_outputs:
+            if rank == 0:
+                dump_outputs(args.dump_outputs, loop.outputs())
+            if world > 1:
+                dist.barrier()  # the other ranks' next rt_group barrier waits a bounded time only
         launches_finish = (3 if loop.group is not None or loop.symm is not None else 1) if (world > 1 or rank == 0) else 0
         launches_step = launches_render + launches_finish
 
@@ -657,10 +698,11 @@ def run_reference(args) -> None:
         print(json.dumps(line), flush=True)
         return
     if not (ref / "ref_main").exists() or not (ref / "ref_harness").exists():
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/ref_main not built (needs /root/reference at build time)"}))
+        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref/ref_main not built (needs the reference's sources: make -C oracle ref REF=<dir>)"}))
         return
     spp = args.spp or cfg["spp"]
     took_ms, kernel_ms, rays = [], None, None
+    steps = args.steps
     how = ""
     if args.config == "c1" and not args.spp:
         # the UNCHANGED binary: its own timing window (init_rand_state + render + syncs, main.cu:431-454)
@@ -684,8 +726,9 @@ def run_reference(args) -> None:
                 if child_json("--child", "dump-scene", "--config", args.config, "--scene-n", str(n_over), "--out", str(sp)) is None:
                     print(json.dumps({"impl": "reference", "unavailable": "could not write the scene file"}))
                     return
+            steps = min(args.steps, 3)  # the reference's frames of the larger configs take seconds to minutes each
             o = subprocess.run([str(ref / "ref_harness"), "render", str(sp), str(W), str(H), str(spp), str(Path(td) / "o.f32"), "1", "1",
-                                str(max(1, min(args.steps, 3)))], capture_output=True, text=True, timeout=1500)
+                                str(steps)], capture_output=True, text=True, timeout=1500)
             if o.returncode != 0:
                 print(json.dumps({"impl": "reference", "unavailable": "ref_harness failed: " + o.stderr[-200:]}))
                 return
@@ -697,7 +740,7 @@ def run_reference(args) -> None:
     ms = float(np.mean(took_ms))
     paths = float(W) * H * spp
     value = paths / ms / 1e3
-    line = {"impl": "reference", "metric": "Mpaths/s", "value": value, "unit": "Mpaths/s", "n_gpus": args.gpus, "steps": args.steps,
+    line = {"impl": "reference", "metric": "Mpaths/s", "value": value, "unit": "Mpaths/s", "n_gpus": args.gpus, "steps": steps,
             "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "ms_per_frame": ms, "mrays_per_s": (rays / ms / 1e3) if rays else None,
             "kernel_ms_cuda_events": kernel_ms,
@@ -736,10 +779,16 @@ def main() -> None:
     ap.add_argument("--collective", choices=["auto", "ipc", "multimem", "peer", "nccl"], default="auto",
                     help="N > 1: rt_group of the C-ABI (auto / ipc), or the A/B forms: torch symmetric memory with NVLS multimem / "
                          "peer loads in the fused kernel, or the plain NCCL reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame (and, with one GPU, the accumulator) of the last timed step as DIR/<name>.npy")
     ap.add_argument("--child", choices=["cpu-baseline", "dump-scene"], default=None, help=argparse.SUPPRESS)
     ap.add_argument("--scene-n", type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument("--out", default="", help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.child:
         run_child(args)
         return

@@ -323,6 +323,10 @@ class Context:
         self._h = _VP()
         _check(self.lib, self.lib.rt_context_create(device, C.byref(self._h)))
         self.device = device
+        # open scenes and groups of this context, handle -> destroy entry: they must be destroyed before the context, and
+        # when the garbage collector finds a context and its scenes unreachable together it finalises them in no
+        # particular order
+        self._open: dict[int, object] = {}
 
     def set_stream(self, cuda_stream: int) -> None:
         _check(self.lib, self.lib.rt_context_set_stream(self._h, _VP(cuda_stream)))
@@ -332,6 +336,9 @@ class Context:
 
     def close(self) -> None:
         if self._h:
+            for h, destroy in self._open.items():
+                destroy(_VP(h))
+            self._open.clear()
             self.lib.rt_context_destroy(self._h)
             self._h = _VP()
 
@@ -348,6 +355,7 @@ class Scene:
         self.lib = ctx.lib
         self._h = _VP()
         _check(self.lib, self.lib.rt_scene_create(ctx._h, desc._ptr, C.byref(self._h)))
+        ctx._open[self._h.value] = self.lib.rt_scene_destroy
 
     def info(self) -> rt_scene_info:
         i = rt_scene_info()
@@ -417,7 +425,8 @@ class Scene:
 
     def close(self) -> None:
         if self._h:
-            self.lib.rt_scene_destroy(self._h)
+            if self.ctx._open.pop(self._h.value, None):  # (else the context has been closed and destroyed the scene with it)
+                self.lib.rt_scene_destroy(self._h)
             self._h = _VP()
 
     def __del__(self):
@@ -508,6 +517,7 @@ class Group:
         self.lib, self.ctx, self.rank, self.world, self.width, self.height = ctx.lib, ctx, rank, world, width, height
         self._h = _VP()
         _check(self.lib, self.lib.rt_group_create(ctx._h, rank, world, width, height, C.byref(self._h)))
+        ctx._open[self._h.value] = self.lib.rt_group_destroy
         blob = C.create_string_buffer(RT_GROUP_HANDLE_BYTES)
         _check(self.lib, self.lib.rt_group_export(self._h, blob))
         if world > 1:
@@ -535,7 +545,8 @@ class Group:
 
     def close(self) -> None:
         if self._h:
-            self.lib.rt_group_destroy(self._h)
+            if self.ctx._open.pop(self._h.value, None):  # (else the context has been closed and destroyed the group with it)
+                self.lib.rt_group_destroy(self._h)
             self._h = _VP()
 
 

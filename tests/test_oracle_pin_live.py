@@ -1,6 +1,6 @@
 """Live pin of the oracle against the reference's own headers (oracle/_ref/libref_cpu.so).  Only where the
-reference has been compiled (this container); elsewhere tests/test_oracle_golden.py carries the same
-comparison through committed vectors."""
+reference has been compiled (`make -C oracle ref REF=<reference checkout>`); elsewhere tests/test_oracle_golden.py
+carries the same comparison through committed vectors."""
 import numpy as np
 import pytest
 
@@ -9,7 +9,7 @@ from raytracing_renderer_cuda_b200 import capi
 from tests.conftest import SCENES
 from tests.oracle_api import REFCPU_SO, RefCpu, camera_rays, secondary_rays
 
-pytestmark = pytest.mark.skipif(not REFCPU_SO.exists(), reason="oracle/_ref/libref_cpu.so not built (no /root/reference here)")
+needs_reference = pytest.mark.skipif(not REFCPU_SO.exists(), reason="oracle/_ref/libref_cpu.so not built (the reference's sources are not here)")
 
 
 @pytest.fixture(scope="module")
@@ -17,6 +17,7 @@ def ref():
     return RefCpu()
 
 
+@needs_reference
 @pytest.mark.parametrize("name", SCENES)
 def test_trace_matches_reference_headers(oracle, ref, scene_descs, name):
     d = scene_descs[name]
@@ -34,6 +35,7 @@ def test_trace_matches_reference_headers(oracle, ref, scene_descs, name):
         assert np.array_equal(b["id"], w["id"]) and np.array_equal(b["t"], w["t"])
 
 
+@needs_reference
 @pytest.mark.parametrize("name,size", [("earth_emitter", (96, 48, 8)), ("book1_final", (64, 36, 4)), ("perlin_motion", (64, 32, 4))])
 def test_render_matches_reference_headers(oracle, ref, scene_descs, name, size):
     w, h, spp = size
