@@ -6,7 +6,7 @@
 //   render_scene [scene] [width height spp] [out] [earth.ppm]            (positional, as before)
 //   render_scene --scene <name | file.json> [--width W --height H --spp N --depth D --seed S]
 //                [--out render.jpg|.ppm] [--quality 100] [--earth assets/earth_stb.ppm] [--passes K] [--emitter-sampling]
-//                [--gpus N]
+//                [--gpus N] [--denoise]
 //     scene: earth_emitter (default) | book1_final | perlin_motion | random_spheres:N | a JSON document
 //            (include/rt/scene_json.hpp; the reference's compile-time scene and WIDTH/HEIGHT/SAMPLES_PER_PIXEL/SEED
 //            macros, main.cu:15,188-356, common.h:13-20, become runtime input)
@@ -20,6 +20,8 @@
 //            NVLink peer memory.  The output file is written from the 8-bit frame (JPEG through rt_jpeg_encode).
 //     --passes K: progressive accumulation, K passes of --spp samples each into one accumulator; the output file is
 //            rewritten after every pass (PPM only)
+//     --denoise: rt_render_denoised with rt_default_denoise_params — first-hit features and the edge-avoiding à-trous
+//            filter on the device after the render; the frame is then written as without it.  One device, one pass.
 //
 // The earth texture: --earth textures/earth.jpg (decoded by rt_image_load exactly as stbi_loadf does) or a binary PPM
 // of the stb-decoded bytes (assets/earth_stb.ppm, written by __graft_entry__.build()).
@@ -51,6 +53,7 @@ int main(int argc, char** argv) {
     int passes = 1;
     int gpus = 1; // 1: the single-device path below; anything else: rt_multi_*
     bool emitter_sampling = false;
+    bool denoise = false;
     rt_render_params p;
     rt_default_render_params(&p); // 1200x600x100, depth 50, seed 1000, tmin 1e-5 (common.h:13-20, main.cu:15,45)
     bool size_given = false;
@@ -76,9 +79,10 @@ int main(int argc, char** argv) {
         else if (a == "--passes") passes = atoi(next("--passes"));
         else if (a == "--gpus") gpus = atoi(next("--gpus"));
         else if (a == "--emitter-sampling") emitter_sampling = true;
+        else if (a == "--denoise") denoise = true;
         else if (a == "--help" || a == "-h") {
             printf("render_scene --scene <name|file.json> [--width W --height H --spp N --depth D --seed S] [--out f.jpg|f.ppm] "
-                   "[--quality Q] [--earth earth.ppm] [--passes K] [--emitter-sampling] [--gpus N]\n");
+                   "[--quality Q] [--earth earth.ppm] [--passes K] [--emitter-sampling] [--gpus N] [--denoise]\n");
             return 0;
         } else pos.push_back(a);
     }
@@ -91,6 +95,10 @@ int main(int argc, char** argv) {
     }
     if (pos.size() > 4) out_path = pos[4];
     if (pos.size() > 5) earth_path = pos[5];
+    if (denoise && (gpus != 1 || passes > 1)) {
+        fprintf(stderr, "--denoise renders one pass on one device: it cannot be combined with --gpus or --passes\n");
+        return 2;
+    }
 
     rt_context* ctx = nullptr;
     CHECK(rt_context_create(0, &ctx));
@@ -174,6 +182,17 @@ int main(int argc, char** argv) {
         };
         CHECK(rt_render_progressive(ctx, scene, &p, passes, fb.data(), on_pass, &sink, &st));
         printf("took %.0fus on the device for %d passes (%.1f Mpaths/s)\n", st.ms_total * 1e3, passes, st.paths / st.ms_total / 1e3);
+    } else if (denoise) {
+        std::vector<float> fb(size_t(p.width) * p.height * 3);
+        rt_denoise_params d;
+        rt_default_denoise_params(&d);
+        CHECK(rt_render_denoised(ctx, scene, &p, &d, fb.data(), &st));
+        printf("took %.0fus.  (%.1f Mpaths/s, %.1f Mrays/s; features + %d filter levels + finalisation %.3f ms)\n", st.ms_total * 1e3,
+               st.paths / st.ms_total / 1e3, st.rays / st.ms_total / 1e3, d.iterations, st.ms_tonemap);
+        std::vector<uint8_t> img(fb.size());
+        CHECK(rt_quantize_rgb8(fb.data(), p.width, p.height, img.data())); // main.cu:475-488
+        if (ends_with(out_path, ".jpg") || ends_with(out_path, ".jpeg")) CHECK(rt_write_jpg(ctx, out_path.c_str(), p.width, p.height, img.data(), quality));
+        else CHECK(rt_write_ppm(out_path.c_str(), p.width, p.height, img.data()));
     } else if (ends_with(out_path, ".jpg") || ends_with(out_path, ".jpeg")) {
         // device output stage: finalise, flip, quantise and JPEG-encode on the GPU; only the file comes back
         std::vector<uint8_t> file(rt_jpeg_max_bytes(p.width, p.height));

@@ -325,7 +325,41 @@ rt_status rt_reduce_tonemap_peers(rt_context* ctx, const void* const* peer_accum
                                   const void* multicast_accum, int32_t width, int32_t height, int32_t row_begin,
                                   int32_t row_end, void* out_rgb_dev, void* out_rgb8_dev, void* out_sum_dev);
 
-/* ---- multi-GPU (SURVEY.md 8e; BASELINE.json north_star (4)) ---------------------------------------------------
+/* ---- denoiser -------------------------------------------------------------------------------------------------
+ * A post-pass over the float4 accumulator of any render entry: first-hit feature buffers and the edge-avoiding à-trous
+ * wavelet filter (Dammertz et al., HPG 2010), then the pixel finalisation of rt_tonemap_device.  No render kernel is
+ * involved.
+ * Features: 2*width*height float4, two planes in the accumulator's layout (index j*width+i, j = 0 the bottom row):
+ *   plane 0 [0, W*H):      mean outward unit normal (not renormalised) and mean hit distance t*|d| over the camera
+ *                          samples that hit (0 when none does);
+ *   plane 1 [W*H, 2*W*H):  mean albedo over all samples (scatter()'s attenuation; emit for an emitter; the world colour
+ *                          for a miss) and the fraction of samples that hit.
+ * Filter level i (0 <= i < iterations) is a 5x5 B3-spline kernel with taps 2^i pixels apart, each tap weighted by
+ *   exp(-|c_p-c_q|^2/(sigma_color 2^-i)^2) exp(-|n_p-n_q|^2/sigma_normal^2) exp(-|z_p-z_q|/(sigma_depth max(z_p,z_q,1e-4)))
+ *   exp(-(|a_p-a_q|^2 + (f_p-f_q)^2)/sigma_albedo^2)
+ * on the mean colour accum.rgb/accum.w saturated to [0, 1].  Pixels without samples are finalised as rt_tonemap_device
+ * finalises them.  The colour is not divided by the albedo: the estimator's first-hit attenuation multiplies only what the
+ * path gathers after that hit, not the pixel value. */
+typedef struct rt_denoise_params {
+    int32_t iterations;  /* à-trous levels, 0..8; 0 = no filtering (== rt_tonemap_device) */
+    int32_t feature_spp; /* camera samples per pixel of the feature pass, >= 1 */
+    float sigma_color, sigma_normal, sigma_depth, sigma_albedo; /* > 0, finite */
+} rt_denoise_params;
+void rt_default_denoise_params(rt_denoise_params* d); /* 3 levels, 4 feature samples, sigmas 0.5, 1, 0.3, 1 */
+/* features of p's camera samples [p->sample_offset, p->sample_offset + feature_spp) into features_dev (device memory,
+ * layout above); p->spp is not used.  Asynchronous on the context stream. */
+rt_status rt_render_features_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
+                                    int32_t feature_spp, void* features_dev);
+/* filter + finalisation of a device accumulator: out_rgb_dev / out_rgb8_dev (either may be NULL, not both) as
+ * rt_tonemap_device writes them.  Asynchronous on the context stream; scratch comes from the context's memory pool. */
+rt_status rt_denoise_device(rt_context* ctx, const void* accum_dev, const void* features_dev, int32_t width,
+                            int32_t height, const rt_denoise_params* d, void* out_rgb_dev, void* out_rgb8_dev);
+/* rt_render + features (d->feature_spp samples from p->sample_offset) + filter + finalisation; out_rgb: HOST, layout of
+ * rt_render.  stats->ms_tonemap = device time of features + filter + finalisation. */
+rt_status rt_render_denoised(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
+                             const rt_denoise_params* d, float* out_rgb, rt_stats* stats);
+
+/* ---- multi-GPU (SURVEY.md 8e; BASELINE.json north_star (4))---------------------------------------------------
  * Samples per pixel are split across the GPUs of one box: GPU r renders sample indices [first_r, first_r + count_r) of
  * EVERY pixel (rt_render_params.sample_offset; the Philox keys use the global sample index, so the image does not depend
  * on the number of GPUs) into its own float4 accumulator; the accumulators are summed in rank order and finalised by

@@ -114,6 +114,11 @@ class rt_shade_sample(C.Structure):
                 ("attenuation", C.c_float * 3), ("scattered", rt_ray)]
 
 
+class rt_denoise_params(C.Structure):
+    _fields_ = [("iterations", C.c_int32), ("feature_spp", C.c_int32), ("sigma_color", C.c_float), ("sigma_normal", C.c_float),
+                ("sigma_depth", C.c_float), ("sigma_albedo", C.c_float)]
+
+
 RAY_DTYPE = np.dtype([("origin", "<f4", 3), ("direction", "<f4", 3), ("time", "<f4")])
 HIT_DTYPE = np.dtype([("t", "<f4"), ("id", "<u4"), ("p", "<f4", 3), ("n", "<f4", 3), ("u", "<f4"), ("v", "<f4")])
 SHADE_DTYPE = np.dtype([("id", "<u4"), ("continues", "<u4"), ("t", "<f4"), ("emitted", "<f4", 3), ("attenuation", "<f4", 3),
@@ -143,6 +148,10 @@ _SIGNATURES = {
     "rt_render_accum_device": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), _VP, C.POINTER(rt_stats)]),
     "rt_render_progressive": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.c_int32, _VP, _VP, _VP, C.POINTER(rt_stats)]),
     "rt_tonemap_device": (C.c_int, [_VP, _VP, C.c_int32, C.c_int32, _VP, _VP]),
+    "rt_default_denoise_params": (None, [C.POINTER(rt_denoise_params)]),
+    "rt_render_features_device": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.c_int32, _VP]),
+    "rt_denoise_device": (C.c_int, [_VP, _VP, _VP, C.c_int32, C.c_int32, C.POINTER(rt_denoise_params), _VP, _VP]),
+    "rt_render_denoised": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_denoise_params), _VP, C.POINTER(rt_stats)]),
     "rt_reduce_tonemap_peers": (C.c_int, [_VP, C.POINTER(_VP), C.c_int32, _VP, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                           _VP, _VP, _VP]),
     "rt_shard_samples": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
@@ -215,7 +224,7 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
 
 def check_layout(lib: C.CDLL) -> None:
     for cls in (rt_jpeg_component, rt_jpeg_coefficients, rt_sphere, rt_material, rt_texture, rt_image, rt_camera, rt_scene_desc, rt_render_params, rt_stats,
-                rt_scene_info, rt_ray, rt_hit, rt_shade_sample):
+                rt_scene_info, rt_ray, rt_hit, rt_shade_sample, rt_denoise_params):
         want = lib.rt_abi_sizeof(cls.__name__.encode())
         if want != C.sizeof(cls):
             raise RuntimeError(f"ABI drift: sizeof({cls.__name__}) is {want} in the library, {C.sizeof(cls)} here")
@@ -313,6 +322,16 @@ def default_params(**kw) -> rt_render_params:
         else:
             setattr(p, k, v)
     return p
+
+
+def default_denoise_params(**kw) -> rt_denoise_params:
+    """rt_default_denoise_params with fields overridden by keyword."""
+    lib = load_library()
+    d = rt_denoise_params()
+    lib.rt_default_denoise_params(C.byref(d))
+    for k, v in kw.items():
+        setattr(d, k, v)
+    return d
 
 
 class Context:
@@ -423,6 +442,19 @@ class Scene:
                                                  C.byref(n), C.byref(st)))
         return out[:n.value], st
 
+    def render_denoised(self, params: rt_render_params, denoise: "rt_denoise_params | None" = None):
+        """rt_render_denoised: render + features + à-trous filter + finalisation; HOST float RGB [H, W, 3] (layout of render)."""
+        d = denoise if denoise is not None else default_denoise_params()
+        out = np.empty((params.height, params.width, 3), dtype=np.float32)
+        st = rt_stats()
+        _check(self.lib, self.lib.rt_render_denoised(self.ctx._h, self._h, C.byref(params), C.byref(d), out.ctypes.data, C.byref(st)))
+        return out, st
+
+    def render_features_device(self, params: rt_render_params, feature_spp: int, features_ptr: int) -> None:
+        """rt_render_features_device: first-hit features of feature_spp camera samples per pixel into 2*W*H float4 of device
+        memory (plane 0: mean normal, mean distance; plane 1: mean albedo, hit fraction)."""
+        _check(self.lib, self.lib.rt_render_features_device(self.ctx._h, self._h, C.byref(params), feature_spp, _VP(features_ptr)))
+
     def close(self) -> None:
         if self._h:
             if self.ctx._open.pop(self._h.value, None):  # (else the context has been closed and destroyed the scene with it)
@@ -439,6 +471,14 @@ class Scene:
 def tonemap_device(ctx: Context, accum_ptr: int, width: int, height: int, out_rgb_ptr: int = 0, out_rgb8_ptr: int = 0):
     _check(ctx.lib, ctx.lib.rt_tonemap_device(ctx._h, _VP(accum_ptr), width, height, _VP(out_rgb_ptr or None),
                                               _VP(out_rgb8_ptr or None)))
+
+
+def denoise_device(ctx: Context, accum_ptr: int, features_ptr: int, width: int, height: int, denoise: "rt_denoise_params | None" = None,
+                   out_rgb_ptr: int = 0, out_rgb8_ptr: int = 0):
+    """rt_denoise_device: à-trous filter of a device accumulator guided by device features, finalised as tonemap_device."""
+    d = denoise if denoise is not None else default_denoise_params()
+    _check(ctx.lib, ctx.lib.rt_denoise_device(ctx._h, _VP(accum_ptr), _VP(features_ptr), width, height, C.byref(d),
+                                              _VP(out_rgb_ptr or None), _VP(out_rgb8_ptr or None)))
 
 
 RT_GROUP_HANDLE_BYTES = 192

@@ -1067,6 +1067,127 @@ rt_status rt_render_progressive(rt_context* ctx, const rt_scene* scene, const rt
     return RT_OK;
 } RT_API_CATCH
 
+void rt_default_denoise_params(rt_denoise_params* d) {
+    if (!d) return;
+    d->iterations = 3;
+    d->feature_spp = 4;
+    // the best worst case over C1 / C2 / C3 at 4 spp of a sweep of 216 settings (profiles/r03_denoise.md)
+    d->sigma_color = 0.5f;
+    d->sigma_normal = 1.0f;
+    d->sigma_depth = 0.3f;
+    d->sigma_albedo = 1.0f;
+}
+
+} // extern "C"
+
+namespace {
+
+rt_status check_denoise(const rt_denoise_params* d) {
+    ARG_CHECK(d != nullptr, "denoise params is NULL");
+    ARG_CHECK(d->iterations >= 0 && d->iterations <= 8, "iterations must be in [0, 8]");
+    ARG_CHECK(d->feature_spp >= 1, "feature_spp must be >= 1");
+    for (float s : {d->sigma_color, d->sigma_normal, d->sigma_depth, d->sigma_albedo})
+        ARG_CHECK(std::isfinite(s) && s > 0.f, "sigmas must be positive and finite");
+    return RT_OK;
+}
+
+rt_status features_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, int32_t feature_spp, float4* features) {
+    rtd::DRenderParams rp = to_device_params(*p);
+    rp.flags = 0; // the features describe the first hit of the reference estimator: no shadow rays
+    rtd::launch_features(scene->d, rp, scene->d.nodes != nullptr, feature_spp, features, ctx->stream);
+    CUDA_TRY(cudaGetLastError());
+    return RT_OK;
+}
+
+// d->iterations levels ping-ponging between two scratch planes, then the pixel finalisation of the last one
+rt_status denoise_into(rt_context* ctx, const float4* accum, const float4* features, int32_t width, int32_t height,
+                       const rt_denoise_params* d, float* out_rgb, uint8_t* out_rgb8) {
+    if (d->iterations == 0) {
+        rtd::launch_tonemap(accum, width, height, out_rgb, out_rgb8, ctx->sm_count, ctx->stream);
+        CUDA_TRY(cudaGetLastError());
+        return RT_OK;
+    }
+    const size_t npix = size_t(width) * size_t(height);
+    float4* scratch = nullptr;
+    CUDA_TRY(rtd::malloc_async(&scratch, 2 * npix * sizeof(float4), ctx->stream));
+    const float4* in = accum;
+    float4* out = scratch;
+    for (int32_t level = 0; level < d->iterations; ++level) {
+        rtd::launch_atrous(in, level == 0, features, width, height, level, d->sigma_color, d->sigma_normal, d->sigma_depth,
+                           d->sigma_albedo, out, ctx->stream);
+        in = out;
+        out = out == scratch ? scratch + npix : scratch;
+    }
+    rtd::launch_tonemap(in, width, height, out_rgb, out_rgb8, ctx->sm_count, ctx->stream);
+    const cudaError_t e = cudaGetLastError();
+    cudaFreeAsync(scratch, ctx->stream);
+    if (e != cudaSuccess) {
+        set_error("denoise: %s", cudaGetErrorString(e));
+        return RT_ERR_CUDA;
+    }
+    return RT_OK;
+}
+
+} // namespace
+
+extern "C" {
+
+rt_status rt_render_features_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, int32_t feature_spp,
+                                    void* features_dev) try {
+    ARG_CHECK(ctx && scene && features_dev, "ctx/scene/features_dev is NULL");
+    rt_status st = check_params(p);
+    if (st != RT_OK) return st;
+    ARG_CHECK(feature_spp >= 1, "feature_spp must be >= 1");
+    ARG_CHECK(int64_t(p->sample_offset) + feature_spp <= INT32_MAX, "sample indices exceed 2^31");
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    return features_into(ctx, scene, p, feature_spp, static_cast<float4*>(features_dev));
+} RT_API_CATCH
+
+rt_status rt_denoise_device(rt_context* ctx, const void* accum_dev, const void* features_dev, int32_t width, int32_t height,
+                            const rt_denoise_params* d, void* out_rgb_dev, void* out_rgb8_dev) try {
+    ARG_CHECK(ctx && accum_dev && features_dev, "ctx/accum_dev/features_dev is NULL");
+    ARG_CHECK(width > 0 && height > 0, "width/height must be positive");
+    ARG_CHECK(uint64_t(width) * uint64_t(height) < (1ull << 31), "frame has more than 2^31 pixels");
+    ARG_CHECK(out_rgb_dev || out_rgb8_dev, "no output buffer");
+    rt_status st = check_denoise(d);
+    if (st != RT_OK) return st;
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    return denoise_into(ctx, static_cast<const float4*>(accum_dev), static_cast<const float4*>(features_dev), width, height, d,
+                        static_cast<float*>(out_rgb_dev), static_cast<uint8_t*>(out_rgb8_dev));
+} RT_API_CATCH
+
+rt_status rt_render_denoised(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_denoise_params* d,
+                             float* out_rgb, rt_stats* stats) try {
+    ARG_CHECK(ctx && scene && out_rgb, "ctx/scene/out_rgb is NULL");
+    rt_status st = check_params(p);
+    if (st != RT_OK) return st;
+    if ((st = check_denoise(d)) != RT_OK) return st;
+    ARG_CHECK(int64_t(p->sample_offset) + d->feature_spp <= INT32_MAX, "sample indices exceed 2^31");
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    const size_t npix = size_t(p->width) * size_t(p->height);
+    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
+    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
+    rt_stats local;
+    if ((st = render_into(ctx, scene, p, ctx->accum, &local)) != RT_OK) return st;
+    float4* features = nullptr;
+    CUDA_TRY(rtd::malloc_async(&features, 2 * npix * sizeof(float4), ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
+    st = features_into(ctx, scene, p, d->feature_spp, features);
+    if (st == RT_OK) st = denoise_into(ctx, ctx->accum, features, p->width, p->height, d, ctx->out_rgb, nullptr);
+    cudaFreeAsync(features, ctx->stream);
+    if (st != RT_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    local.launches += 2 + uint32_t(d->iterations); // features, the levels, the finalisation
+    if (stats) *stats = local;
+    return RT_OK;
+} RT_API_CATCH
+
 namespace {
 struct OwnedCoefficients { // rt_jpeg_coefficients that owns its planes; `pub` must stay the first member
     rt_jpeg_coefficients pub;

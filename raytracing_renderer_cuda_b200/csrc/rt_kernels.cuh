@@ -37,6 +37,12 @@ void launch_tonemap(const float4* accum, int width, int height, float* out_rgb, 
 void launch_reduce_tonemap(const void* const* peer_accum, int n_peers, const void* multicast, int width, int height,
                            int row_begin, int row_end, float* out_rgb, uint8_t* out_rgb8, float4* out_sum, int sm_count, cudaStream_t st);
 
+// denoiser (rt_denoise.cu): first-hit features of feature_spp camera samples per pixel (2 float4 planes of width*height),
+// and one level of the edge-avoiding à-trous filter (taps 2^level apart); from_accum: `in` is a render's accumulator
+void launch_features(const DScene& sc, const DRenderParams& rp, bool use_bvh, int feature_spp, float4* features, cudaStream_t st);
+void launch_atrous(const float4* in, bool from_accum, const float4* features, int width, int height, int level, float sigma_color,
+                   float sigma_normal, float sigma_depth, float sigma_albedo, float4* out, cudaStream_t st);
+
 // self-test: out[4i..4i+3] = div_rz(x, y), __fdiv_rz(x, y), sqrt_rz(x), __fsqrt_rz(x)  (rt_device.cuh)
 void launch_selftest_rz(const float* x_dev, const float* y_dev, size_t n, float* out_dev, cudaStream_t st);
 
