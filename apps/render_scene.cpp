@@ -6,7 +6,7 @@
 //   render_scene [scene] [width height spp] [out] [earth.ppm]            (positional, as before)
 //   render_scene --scene <name | file.json> [--width W --height H --spp N --depth D --seed S]
 //                [--out render.jpg|.ppm] [--quality 100] [--earth assets/earth_stb.ppm] [--passes K] [--emitter-sampling]
-//                [--gpus N] [--denoise]
+//                [--gpus N] [--denoise] [--adaptive T [--max-spp N]]
 //     scene: earth_emitter (default) | book1_final | perlin_motion | random_spheres:N | a JSON document
 //            (include/rt/scene_json.hpp; the reference's compile-time scene and WIDTH/HEIGHT/SAMPLES_PER_PIXEL/SEED
 //            macros, main.cu:15,188-356, common.h:13-20, become runtime input)
@@ -22,6 +22,9 @@
 //            rewritten after every pass (PPM only)
 //     --denoise: rt_render_denoised with rt_default_denoise_params — first-hit features and the edge-avoiding à-trous
 //            filter on the device after the render; the frame is then written as without it.  One device, one pass.
+//     --adaptive T: adaptive sampling (rt_render_adaptive): every pixel gets --spp samples, then passes of --spp samples go
+//            to the pixels whose display-space noise estimate is still >= T, up to --max-spp (default 16 x --spp).  With
+//            --denoise the adaptive accumulator goes through the device entries (features, rt_denoise_device).  One device.
 //
 // The earth texture: --earth textures/earth.jpg (decoded by rt_image_load exactly as stbi_loadf does) or a binary PPM
 // of the stb-decoded bytes (assets/earth_stb.ppm, written by __graft_entry__.build()).
@@ -30,6 +33,8 @@
 #include <cstring>
 #include <string>
 #include <vector>
+
+#include <cuda_runtime.h>
 
 #include "../include/rt/scenes.hpp"
 
@@ -54,6 +59,9 @@ int main(int argc, char** argv) {
     int gpus = 1; // 1: the single-device path below; anything else: rt_multi_*
     bool emitter_sampling = false;
     bool denoise = false;
+    bool adaptive = false;
+    float threshold = 0.f;
+    int max_spp = 0; // 0: 16 x --spp
     rt_render_params p;
     rt_default_render_params(&p); // 1200x600x100, depth 50, seed 1000, tmin 1e-5 (common.h:13-20, main.cu:15,45)
     bool size_given = false;
@@ -80,9 +88,12 @@ int main(int argc, char** argv) {
         else if (a == "--gpus") gpus = atoi(next("--gpus"));
         else if (a == "--emitter-sampling") emitter_sampling = true;
         else if (a == "--denoise") denoise = true;
+        else if (a == "--adaptive") adaptive = true, threshold = float(atof(next("--adaptive")));
+        else if (a == "--max-spp") max_spp = atoi(next("--max-spp"));
         else if (a == "--help" || a == "-h") {
             printf("render_scene --scene <name|file.json> [--width W --height H --spp N --depth D --seed S] [--out f.jpg|f.ppm] "
-                   "[--quality Q] [--earth earth.ppm] [--passes K] [--emitter-sampling] [--gpus N] [--denoise]\n");
+                   "[--quality Q] [--earth earth.ppm] [--passes K] [--emitter-sampling] [--gpus N] [--denoise] "
+                   "[--adaptive T [--max-spp N]]\n");
             return 0;
         } else pos.push_back(a);
     }
@@ -97,6 +108,10 @@ int main(int argc, char** argv) {
     if (pos.size() > 5) earth_path = pos[5];
     if (denoise && (gpus != 1 || passes > 1)) {
         fprintf(stderr, "--denoise renders one pass on one device: it cannot be combined with --gpus or --passes\n");
+        return 2;
+    }
+    if (adaptive && (gpus != 1 || passes > 1)) {
+        fprintf(stderr, "--adaptive renders on one device and chooses its own passes: it cannot be combined with --gpus or --passes\n");
         return 2;
     }
 
@@ -165,7 +180,54 @@ int main(int argc, char** argv) {
            p.height, p.spp, info.n_spheres, info.n_nodes, info.bvh_mode, info.ms_build);
 
     rt_stats st;
-    if (passes > 1) { // progressive: the frame on disk sharpens pass by pass
+    auto write_frame = [&](const std::vector<float>& fb) -> int {
+        std::vector<uint8_t> img(fb.size());
+        CHECK(rt_quantize_rgb8(fb.data(), p.width, p.height, img.data())); // main.cu:475-488
+        if (ends_with(out_path, ".jpg") || ends_with(out_path, ".jpeg")) CHECK(rt_write_jpg(ctx, out_path.c_str(), p.width, p.height, img.data(), quality));
+        else CHECK(rt_write_ppm(out_path.c_str(), p.width, p.height, img.data()));
+        return 0;
+    };
+    if (adaptive) {
+        rt_adaptive_params a;
+        rt_default_adaptive_params(&a);
+        a.min_spp = a.step_spp = p.spp;
+        a.max_spp = max_spp > 0 ? max_spp : 16 * p.spp;
+        a.threshold = threshold;
+        const size_t npix = size_t(p.width) * p.height;
+        std::vector<float> fb(npix * 3);
+        int32_t n_passes = 0;
+        if (!denoise) {
+            std::vector<int32_t> spp_map(npix);
+            CHECK(rt_render_adaptive(ctx, scene, &p, &a, fb.data(), spp_map.data(), &st));
+            int32_t top = 0;
+            for (int32_t c : spp_map) top = c > top ? c : top;
+            n_passes = 1 + (top - a.min_spp) / a.step_spp;
+        } else { // adaptive accumulator -> first-hit features -> à-trous filter + finalisation, all on the device
+            rt_denoise_params d;
+            rt_default_denoise_params(&d);
+            void *accum = nullptr, *features = nullptr, *rgb = nullptr;
+            if (cudaMalloc(&accum, npix * 16) != cudaSuccess || cudaMalloc(&features, 2 * npix * 16) != cudaSuccess ||
+                cudaMalloc(&rgb, npix * 3 * sizeof(float)) != cudaSuccess) {
+                fprintf(stderr, "cudaMalloc failed\n");
+                return 1;
+            }
+            CHECK(rt_render_adaptive_device(ctx, scene, &p, &a, accum, nullptr, &n_passes, &st));
+            CHECK(rt_render_features_device(ctx, scene, &p, d.feature_spp, features));
+            CHECK(rt_denoise_device(ctx, accum, features, p.width, p.height, &d, rgb, nullptr));
+            CHECK(rt_context_synchronize(ctx));
+            if (cudaMemcpy(fb.data(), rgb, fb.size() * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess) {
+                fprintf(stderr, "cudaMemcpy failed\n");
+                return 1;
+            }
+            cudaFree(accum);
+            cudaFree(features);
+            cudaFree(rgb);
+        }
+        printf("took %.0fus.  (%d passes, mean %.2f samples per pixel of %d..%d, threshold %g; %.1f Mpaths/s, %.1f Mrays/s%s)\n",
+               st.ms_total * 1e3, n_passes, double(st.paths) / double(npix), a.min_spp, a.max_spp, double(a.threshold),
+               st.paths / st.ms_total / 1e3, st.rays / st.ms_total / 1e3, denoise ? "; denoised" : "");
+        if (write_frame(fb)) return 1;
+    } else if (passes > 1) { // progressive: the frame on disk sharpens pass by pass
         struct Sink {
             const rt_render_params* p;
             const char* path;

@@ -359,6 +359,41 @@ rt_status rt_denoise_device(rt_context* ctx, const void* accum_dev, const void* 
 rt_status rt_render_denoised(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
                              const rt_denoise_params* d, float* out_rgb, rt_stats* stats);
 
+/* ---- adaptive sampling --------------------------------------------------------------------------------------------
+ * Pixels stop sampling once their noise estimate falls below a threshold.  Pass 0 gives every pixel min_spp samples; each
+ * later pass gives step_spp samples to the pixels still listed, until the list is empty or max_spp is reached.  A path
+ * adds into plane A (even samples, counted from p->sample_offset) or plane B (odd samples) of a two-plane accumulator
+ * (2*W*H float4: plane A, then plane B).  After every pass but the last, the error of pixel p is, with g(x) =
+ * sqrt(saturate(x)),
+ *   e_p = (|g(A_r/A_w) - g(B_r/B_w)| + |g(A_g/A_w) - g(B_g/B_w)| + |g(A_b/A_w) - g(B_b/B_w)|) / 6      (+inf if A_w or B_w = 0)
+ * (half the mean over the channels of the difference of the two half means: the standard error of the full mean in
+ * display space), the windowed error ebar_p = (sum of e over the 3x3 neighbourhood, coordinates clamped to the frame,
+ * in row-major order) / 9, every step one IEEE float operation, and the list keeps, in its order (pixel order), the pixels
+ * with ebar_p >= threshold and count(p) < max_spp.  A pixel that stopped never restarts, so pixel p has exactly the samples
+ * [p->sample_offset, p->sample_offset + count(p)), count(p) = min_spp + k*step_spp: the samples a uniform render of
+ * count(p) spp gives it.  Stopping early carries the small bias of every adaptive sampler; threshold = 0 removes it. */
+typedef struct rt_adaptive_params {
+    int32_t min_spp;  /* first pass, every pixel; even, >= 2 */
+    int32_t step_spp; /* every later pass, listed pixels only; even, >= 2 */
+    int32_t max_spp;  /* cap: min_spp + k*step_spp for some k >= 0, <= 2^24 */
+    float threshold;  /* display-space standard-error target, finite, >= 0; 0 = never stop early */
+} rt_adaptive_params;
+void rt_default_adaptive_params(rt_adaptive_params* a); /* min 32, step 32, max 256, threshold 1/255 */
+/* windowed error map (ebar above) of a two-plane accumulator (2*W*H float4, device) into error_dev (W*H floats, device).
+ * Asynchronous on the context stream. */
+rt_status rt_adaptive_error_device(rt_context* ctx, const void* planes_dev, int32_t width, int32_t height, void* error_dev);
+/* p->spp is not used; samples start at p->sample_offset.  accum_dev (W*H float4, device) is WRITTEN (A + B), not added to;
+ * error_dev (W*H floats, device, may be NULL) receives the final windowed error; *passes (may be NULL) the passes run.
+ * stats (may be NULL): paths = samples actually traced, rays, launches, iterations, ms_total = device time of the whole
+ * call.  Returns when the frame is finished (the planes and lists live in the context's memory pool). */
+rt_status rt_render_adaptive_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
+                                    const rt_adaptive_params* a, void* accum_dev, void* error_dev, int32_t* passes,
+                                    rt_stats* stats);
+/* host convenience: out_rgb (HOST) as rt_render writes it; out_spp (HOST, may be NULL) W*H int32 samples per pixel in the
+ * same layout */
+rt_status rt_render_adaptive(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
+                             const rt_adaptive_params* a, float* out_rgb, int32_t* out_spp, rt_stats* stats);
+
 /* ---- multi-GPU (SURVEY.md 8e; BASELINE.json north_star (4))---------------------------------------------------
  * Samples per pixel are split across the GPUs of one box: GPU r renders sample indices [first_r, first_r + count_r) of
  * EVERY pixel (rt_render_params.sample_offset; the Philox keys use the global sample index, so the image does not depend

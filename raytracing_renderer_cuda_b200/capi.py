@@ -119,6 +119,10 @@ class rt_denoise_params(C.Structure):
                 ("sigma_depth", C.c_float), ("sigma_albedo", C.c_float)]
 
 
+class rt_adaptive_params(C.Structure):
+    _fields_ = [("min_spp", C.c_int32), ("step_spp", C.c_int32), ("max_spp", C.c_int32), ("threshold", C.c_float)]
+
+
 RAY_DTYPE = np.dtype([("origin", "<f4", 3), ("direction", "<f4", 3), ("time", "<f4")])
 HIT_DTYPE = np.dtype([("t", "<f4"), ("id", "<u4"), ("p", "<f4", 3), ("n", "<f4", 3), ("u", "<f4"), ("v", "<f4")])
 SHADE_DTYPE = np.dtype([("id", "<u4"), ("continues", "<u4"), ("t", "<f4"), ("emitted", "<f4", 3), ("attenuation", "<f4", 3),
@@ -152,6 +156,12 @@ _SIGNATURES = {
     "rt_render_features_device": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.c_int32, _VP]),
     "rt_denoise_device": (C.c_int, [_VP, _VP, _VP, C.c_int32, C.c_int32, C.POINTER(rt_denoise_params), _VP, _VP]),
     "rt_render_denoised": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_denoise_params), _VP, C.POINTER(rt_stats)]),
+    "rt_default_adaptive_params": (None, [C.POINTER(rt_adaptive_params)]),
+    "rt_adaptive_error_device": (C.c_int, [_VP, _VP, C.c_int32, C.c_int32, _VP]),
+    "rt_render_adaptive_device": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params), _VP, _VP,
+                                            C.POINTER(C.c_int32), C.POINTER(rt_stats)]),
+    "rt_render_adaptive": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params), _VP, _VP,
+                                     C.POINTER(rt_stats)]),
     "rt_reduce_tonemap_peers": (C.c_int, [_VP, C.POINTER(_VP), C.c_int32, _VP, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                           _VP, _VP, _VP]),
     "rt_shard_samples": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
@@ -224,7 +234,7 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
 
 def check_layout(lib: C.CDLL) -> None:
     for cls in (rt_jpeg_component, rt_jpeg_coefficients, rt_sphere, rt_material, rt_texture, rt_image, rt_camera, rt_scene_desc, rt_render_params, rt_stats,
-                rt_scene_info, rt_ray, rt_hit, rt_shade_sample, rt_denoise_params):
+                rt_scene_info, rt_ray, rt_hit, rt_shade_sample, rt_denoise_params, rt_adaptive_params):
         want = lib.rt_abi_sizeof(cls.__name__.encode())
         if want != C.sizeof(cls):
             raise RuntimeError(f"ABI drift: sizeof({cls.__name__}) is {want} in the library, {C.sizeof(cls)} here")
@@ -332,6 +342,16 @@ def default_denoise_params(**kw) -> rt_denoise_params:
     for k, v in kw.items():
         setattr(d, k, v)
     return d
+
+
+def default_adaptive_params(**kw) -> rt_adaptive_params:
+    """rt_default_adaptive_params with fields overridden by keyword."""
+    lib = load_library()
+    a = rt_adaptive_params()
+    lib.rt_default_adaptive_params(C.byref(a))
+    for k, v in kw.items():
+        setattr(a, k, v)
+    return a
 
 
 class Context:
@@ -455,6 +475,28 @@ class Scene:
         memory (plane 0: mean normal, mean distance; plane 1: mean albedo, hit fraction)."""
         _check(self.lib, self.lib.rt_render_features_device(self.ctx._h, self._h, C.byref(params), feature_spp, _VP(features_ptr)))
 
+    def render_adaptive(self, params: rt_render_params, adaptive: "rt_adaptive_params | None" = None):
+        """rt_render_adaptive: returns (HOST float RGB [H, W, 3] in the layout of render, samples per pixel [H, W] int32, stats,
+        passes run)."""
+        a = adaptive if adaptive is not None else default_adaptive_params()
+        out = np.empty((params.height, params.width, 3), dtype=np.float32)
+        spp = np.empty((params.height, params.width), dtype=np.int32)
+        st = rt_stats()
+        _check(self.lib, self.lib.rt_render_adaptive(self.ctx._h, self._h, C.byref(params), C.byref(a), out.ctypes.data, spp.ctypes.data,
+                                                     C.byref(st)))
+        return out, spp, st, 1 + (int(spp.max()) - a.min_spp) // a.step_spp  # one pass per sample level up to the largest count
+
+    def render_adaptive_device(self, params: rt_render_params, adaptive: "rt_adaptive_params | None", accum_ptr: int,
+                               error_ptr: int = 0, want_stats: bool = False):
+        """rt_render_adaptive_device: writes the finished accumulator (W*H float4) to accum_ptr and, if error_ptr, the final
+        windowed error map (W*H float) there.  Returns (passes run, stats or None)."""
+        a = adaptive if adaptive is not None else default_adaptive_params()
+        st = rt_stats() if want_stats else None
+        passes = C.c_int32(0)
+        _check(self.lib, self.lib.rt_render_adaptive_device(self.ctx._h, self._h, C.byref(params), C.byref(a), _VP(accum_ptr),
+                                                            _VP(error_ptr or None), C.byref(passes), C.byref(st) if st is not None else None))
+        return passes.value, st
+
     def close(self) -> None:
         if self._h:
             if self.ctx._open.pop(self._h.value, None):  # (else the context has been closed and destroyed the scene with it)
@@ -479,6 +521,11 @@ def denoise_device(ctx: Context, accum_ptr: int, features_ptr: int, width: int, 
     d = denoise if denoise is not None else default_denoise_params()
     _check(ctx.lib, ctx.lib.rt_denoise_device(ctx._h, _VP(accum_ptr), _VP(features_ptr), width, height, C.byref(d),
                                               _VP(out_rgb_ptr or None), _VP(out_rgb8_ptr or None)))
+
+
+def adaptive_error_device(ctx: Context, planes_ptr: int, width: int, height: int, error_ptr: int) -> None:
+    """rt_adaptive_error_device: windowed error map (W*H float) of a two-plane accumulator (2*W*H float4, plane A then B)."""
+    _check(ctx.lib, ctx.lib.rt_adaptive_error_device(ctx._h, _VP(planes_ptr), width, height, _VP(error_ptr)))
 
 
 RT_GROUP_HANDLE_BYTES = 192

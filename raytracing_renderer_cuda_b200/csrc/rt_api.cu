@@ -201,6 +201,9 @@ rtd::DRenderParams to_device_params(const rt_render_params& p) {
     d.world_b = p.world[2];
     d.bloom = p.bloom;
     d.flags = p.flags;
+    d.adapt_pixels = nullptr;
+    d.adapt_first = 0;
+    d.adapt_plane = 0;
     return d;
 }
 
@@ -267,23 +270,20 @@ rt_status jpeg_from_device(rt_context* ctx, const uint8_t* rgb8_dev, int32_t w, 
     return RT_OK;
 }
 
-// Core: adds p->spp samples per pixel into accum (device).  Fills stats if requested
-// (which synchronises the stream).
-rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float4* accum, rt_stats* stats) {
-    rtd::DRenderParams rp = to_device_params(*p);
+// One render pass: rp.spp samples of every pixel (of the rp.adapt_pixels list when it is set) added into accum (device);
+// rays are added to ctx->d_ray_counter.
+rt_status render_pass(rt_context* ctx, const rt_scene* scene, const rtd::DRenderParams& rp, uint32_t pipeline_param, float4* accum,
+                      uint32_t* launches_out, uint32_t* iterations_out) {
     const bool use_bvh = scene->d.nodes != nullptr;
-    uint32_t pipeline = p->pipeline == RT_PIPE_AUTO ? uint32_t(RT_PIPE_WAVEFRONT) : p->pipeline;
+    uint32_t pipeline = pipeline_param == RT_PIPE_AUTO ? uint32_t(RT_PIPE_WAVEFRONT) : pipeline_param;
     uint32_t launches = 0, iterations = 0;
-    if (stats) {
-        CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), ctx->stream));
-        CUDA_TRY(cudaEventRecord(ctx->ev[0], ctx->stream));
-    }
     if (pipeline == RT_PIPE_MEGAKERNEL) {
         rtd::launch_render_mega(scene->d, rp, use_bvh, accum, ctx->d_ray_counter, ctx->sm_count, ctx->stream);
         launches = 1;
         iterations = 1;
     } else {
-        const size_t npaths = size_t(p->width) * size_t(p->height) * size_t(p->spp);
+        const size_t npix = rp.adapt_pixels ? size_t(rp.div_npix.d) : size_t(rp.width) * size_t(rp.height);
+        const size_t npaths = npix * size_t(rp.spp);
         // pool of path slots (RT_WF_POOL overrides).  Measured on C1 (ms/frame): 256 Ki 18.7, 512 Ki 14.7, 1 Mi 13.5,
         // 2 Mi 12.6, 4 Mi 12.4 (before the later kernel work), then 4 Mi 11.0, 8 Mi 11.0, 16 Mi 10.5 — fewer, fuller
         // iterations beat keeping the 64-byte records L2-resident.  16 Mi slots = 1 GiB of records + 1 GiB of queues.
@@ -310,6 +310,21 @@ rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_pa
         }
     }
     CUDA_TRY(cudaGetLastError());
+    *launches_out = launches;
+    *iterations_out = iterations;
+    return RT_OK;
+}
+
+// Core: adds p->spp samples per pixel into accum (device).  Fills stats if requested
+// (which synchronises the stream).
+rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float4* accum, rt_stats* stats) {
+    uint32_t launches = 0, iterations = 0;
+    if (stats) {
+        CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), ctx->stream));
+        CUDA_TRY(cudaEventRecord(ctx->ev[0], ctx->stream));
+    }
+    rt_status st = render_pass(ctx, scene, to_device_params(*p), p->pipeline, accum, &launches, &iterations);
+    if (st != RT_OK) return st;
     if (stats) {
         CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
         unsigned long long rays = 0;
@@ -1184,6 +1199,168 @@ rt_status rt_render_denoised(rt_context* ctx, const rt_scene* scene, const rt_re
     CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
     CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
     local.launches += 2 + uint32_t(d->iterations); // features, the levels, the finalisation
+    if (stats) *stats = local;
+    return RT_OK;
+} RT_API_CATCH
+
+void rt_default_adaptive_params(rt_adaptive_params* a) {
+    if (!a) return;
+    // the best worst case over C1 / C2 / C3 of a 36-setting sweep at equal budget, up to 0.03 dB (profiles/r04_adaptive.md)
+    a->min_spp = 32;
+    a->step_spp = 32;
+    a->max_spp = 256;
+    a->threshold = 1.f / 255.f;
+}
+
+} // extern "C"
+
+namespace {
+
+rt_status check_adaptive(const rt_render_params* p, const rt_adaptive_params* a) {
+    ARG_CHECK(a != nullptr, "adaptive params is NULL");
+    ARG_CHECK(a->min_spp >= 2 && a->min_spp % 2 == 0, "min_spp must be even and >= 2");
+    ARG_CHECK(a->step_spp >= 2 && a->step_spp % 2 == 0, "step_spp must be even and >= 2");
+    ARG_CHECK(a->max_spp >= a->min_spp && (a->max_spp - a->min_spp) % a->step_spp == 0, "max_spp must be min_spp + k * step_spp, k >= 0");
+    ARG_CHECK(a->max_spp <= (1 << 24), "max_spp exceeds 2^24, up to which the float sample count is exact");
+    ARG_CHECK(std::isfinite(a->threshold) && a->threshold >= 0.f, "threshold must be finite and >= 0");
+    ARG_CHECK(int64_t(p->sample_offset) + a->max_spp <= INT32_MAX, "sample indices exceed 2^31");
+    return RT_OK;
+}
+
+// The adaptive render (rt_adaptive.cu): pass 0 gives every pixel min_spp samples, every later pass step_spp samples to the
+// pixels the selection kept; then accum = A + B (written) and, if error_dev, the final windowed error map.  Stream-ordered
+// on the context stream, with one 4-byte read-back of the list length per pass.
+rt_status adaptive_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_adaptive_params* a, float4* accum,
+                        float* error_dev, int32_t* passes_out, rt_stats* stats) {
+    cudaStream_t stream = ctx->stream;
+    const uint32_t npix = uint32_t(p->width) * uint32_t(p->height);
+    auto align = [](size_t b) { return (b + 255) & ~size_t(255); };
+    const size_t b_planes = align(2 * size_t(npix) * sizeof(float4)), b_px = align(size_t(npix) * sizeof(uint32_t));
+    const size_t b_words = align(rtd::adapt_select_scratch_words(npix) * sizeof(uint32_t));
+    char* base = nullptr; // planes A and B, the error map, two pixel lists, the selection's words, the list length
+    CUDA_TRY(rtd::malloc_async(&base, b_planes + 3 * b_px + b_words + 256, stream));
+    float4* planes = reinterpret_cast<float4*>(base);
+    float* e = reinterpret_cast<float*>(base + b_planes);
+    uint32_t* list[2] = {reinterpret_cast<uint32_t*>(base + b_planes + b_px), reinterpret_cast<uint32_t*>(base + b_planes + 2 * b_px)};
+    uint32_t* words = reinterpret_cast<uint32_t*>(base + b_planes + 3 * b_px);
+    uint32_t* n_dev = reinterpret_cast<uint32_t*>(base + b_planes + 3 * b_px + b_words);
+    const rt_status st = [&]() -> rt_status {
+        CUDA_TRY(cudaMemsetAsync(planes, 0, 2 * size_t(npix) * sizeof(float4), stream));
+        CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), stream));
+        CUDA_TRY(cudaEventRecord(ctx->ev[0], stream));
+        rtd::launch_adapt_iota(list[0], npix, stream);
+        rtd::DRenderParams rp = to_device_params(*p);
+        rp.adapt_first = uint32_t(p->sample_offset);
+        rp.adapt_plane = npix;
+        uint32_t n = npix, launches = 2, iterations = 0; // (iota and merge)
+        int32_t done = 0, passes = 0, cur = 0;          // samples of every listed pixel so far, passes run, current list
+        uint64_t paths = 0;
+        for (;;) {
+            rp.spp = passes == 0 ? a->min_spp : a->step_spp;
+            rp.sample_offset = p->sample_offset + done;
+            rp.adapt_pixels = list[cur];
+            rp.div_npix = rtd::make_fastdiv(n);
+            uint32_t l = 0, it = 0;
+            const rt_status s = render_pass(ctx, scene, rp, p->pipeline, planes, &l, &it);
+            if (s != RT_OK) return s;
+            launches += l;
+            iterations += it;
+            paths += uint64_t(n) * uint64_t(rp.spp);
+            done += rp.spp;
+            ++passes;
+            if (done >= a->max_spp) break;
+            CUDA_TRY(rtd::launch_adapt_select(planes, p->width, p->height, list[cur], n, a->threshold, a->max_spp, e, words, list[cur ^ 1],
+                                              n_dev, &l, stream));
+            launches += l;
+            uint32_t n_next = 0;
+            CUDA_TRY(cudaMemcpyAsync(&n_next, n_dev, sizeof n_next, cudaMemcpyDeviceToHost, stream));
+            CUDA_TRY(cudaStreamSynchronize(stream));
+            if (n_next == 0) break;
+            n = n_next;
+            cur ^= 1;
+        }
+        rtd::launch_adapt_merge(planes, npix, accum, stream);
+        if (error_dev) {
+            rtd::launch_adapt_error_map(planes, p->width, p->height, e, error_dev, stream);
+            launches += 2;
+        }
+        CUDA_TRY(cudaGetLastError());
+        if (passes_out) *passes_out = passes;
+        if (stats) {
+            CUDA_TRY(cudaEventRecord(ctx->ev[1], stream));
+            unsigned long long rays = 0;
+            CUDA_TRY(cudaMemcpyAsync(&rays, ctx->d_ray_counter, sizeof rays, cudaMemcpyDeviceToHost, stream));
+            CUDA_TRY(cudaStreamSynchronize(stream));
+            memset(stats, 0, sizeof *stats);
+            CUDA_TRY(cudaEventElapsedTime(&stats->ms_total, ctx->ev[0], ctx->ev[1]));
+            stats->paths = paths;
+            stats->rays = rays;
+            stats->launches = launches;
+            stats->iterations = iterations;
+        }
+        return RT_OK;
+    }();
+    cudaFreeAsync(base, stream);
+    return st;
+}
+
+} // namespace
+
+extern "C" {
+
+rt_status rt_adaptive_error_device(rt_context* ctx, const void* planes_dev, int32_t width, int32_t height, void* error_dev) try {
+    ARG_CHECK(ctx && planes_dev && error_dev, "ctx/planes_dev/error_dev is NULL");
+    ARG_CHECK(width > 0 && height > 0, "width/height must be positive");
+    ARG_CHECK(uint64_t(width) * uint64_t(height) < (1ull << 31), "frame has more than 2^31 pixels");
+    rt_status st = make_current(ctx);
+    if (st != RT_OK) return st;
+    float* e = nullptr;
+    CUDA_TRY(rtd::malloc_async(&e, size_t(width) * size_t(height) * sizeof(float), ctx->stream));
+    rtd::launch_adapt_error_map(static_cast<const float4*>(planes_dev), width, height, e, static_cast<float*>(error_dev), ctx->stream);
+    const cudaError_t err = cudaGetLastError();
+    cudaFreeAsync(e, ctx->stream);
+    if (err != cudaSuccess) {
+        set_error("adaptive error map: %s", cudaGetErrorString(err));
+        return RT_ERR_CUDA;
+    }
+    return RT_OK;
+} RT_API_CATCH
+
+rt_status rt_render_adaptive_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_adaptive_params* a,
+                                    void* accum_dev, void* error_dev, int32_t* passes, rt_stats* stats) try {
+    ARG_CHECK(ctx && scene && accum_dev, "ctx/scene/accum_dev is NULL");
+    rt_status st = check_params(p);
+    if (st != RT_OK) return st;
+    if ((st = check_adaptive(p, a)) != RT_OK) return st;
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    return adaptive_into(ctx, scene, p, a, static_cast<float4*>(accum_dev), static_cast<float*>(error_dev), passes, stats);
+} RT_API_CATCH
+
+rt_status rt_render_adaptive(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_adaptive_params* a,
+                             float* out_rgb, int32_t* out_spp, rt_stats* stats) try {
+    ARG_CHECK(ctx && scene && out_rgb, "ctx/scene/out_rgb is NULL");
+    rt_status st = check_params(p);
+    if (st != RT_OK) return st;
+    if ((st = check_adaptive(p, a)) != RT_OK) return st;
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    const size_t npix = size_t(p->width) * size_t(p->height);
+    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
+    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    rt_stats local;
+    if ((st = adaptive_into(ctx, scene, p, a, ctx->accum, nullptr, nullptr, &local)) != RT_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
+    rtd::launch_tonemap(ctx->accum, p->width, p->height, ctx->out_rgb, nullptr, ctx->sm_count, ctx->stream);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
+    std::vector<float4> acc(out_spp ? npix : 0);
+    if (out_spp) CUDA_TRY(cudaMemcpyAsync(acc.data(), ctx->accum, npix * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < acc.size(); ++i) out_spp[i] = int32_t(acc[i].w); // (exact: counts stay below 2^24)
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    local.launches += 1;
     if (stats) *stats = local;
     return RT_OK;
 } RT_API_CATCH

@@ -180,7 +180,19 @@ struct DRenderParams {
     float world_r, world_g, world_b;
     float bloom;
     uint32_t flags; // RT_RENDER_*
+    // Adaptive sampling (the ADAPT instantiations of the render kernels; nullptr / 0 otherwise): path x of a pass is pixel
+    // adapt_pixels[x mod n] of sample sample_offset + x / n with n = div_npix.d, and a finished path adds into plane
+    // (sample - adapt_first) & 1 of a two-plane accumulator whose planes are adapt_plane float4 apart (rt_adaptive.cu).
+    const uint32_t* adapt_pixels;
+    uint32_t adapt_first;
+    uint32_t adapt_plane;
 };
+
+// the float4 accumulator a path of `sample` adds into: the render's own, or in ADAPT instantiations the plane of the sample's parity
+template <bool ADAPT>
+RT_DEV float4* accum_plane(float4* accum, const DRenderParams& rp, uint32_t sample) {
+    return ADAPT ? accum + size_t((sample - rp.adapt_first) & 1u) * rp.adapt_plane : accum;
+}
 
 struct Ray {
     V3 o, d;

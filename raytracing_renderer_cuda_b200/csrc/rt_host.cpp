@@ -38,7 +38,7 @@ size_t rt_abi_sizeof(const char* name) {
     RT_SZ(rt_sphere); RT_SZ(rt_material); RT_SZ(rt_texture); RT_SZ(rt_image); RT_SZ(rt_camera); RT_SZ(rt_scene_desc);
     RT_SZ(rt_jpeg_component); RT_SZ(rt_jpeg_coefficients);
     RT_SZ(rt_render_params); RT_SZ(rt_stats); RT_SZ(rt_scene_info); RT_SZ(rt_ray); RT_SZ(rt_hit); RT_SZ(rt_shade_sample);
-    RT_SZ(rt_denoise_params);
+    RT_SZ(rt_denoise_params); RT_SZ(rt_adaptive_params);
 #undef RT_SZ
     return 0;
 }

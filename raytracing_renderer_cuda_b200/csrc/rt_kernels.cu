@@ -103,6 +103,8 @@ void launch_shade_probe(const DScene& sc, const DRenderParams& rp, const rt_ray*
 // covers 32 neighbouring pixels of one sample.  This is the reference's structure
 // (render + color(), main.cu:35-74,97-132) on the flat scene; it is kept as the
 // RT_PIPE_MEGAKERNEL pipeline and as the yardstick the wavefront pipeline is measured against.
+// ADAPT: adaptive sampling, path -> pixel rp.adapt_pixels[path mod n] (n = div_npix.d), values into the sample's parity plane.
+template <bool ADAPT>
 __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp,
                                                      int use_bvh, float4* __restrict__ accum,
                                                      unsigned long long* __restrict__ ray_counter) {
@@ -111,12 +113,13 @@ __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DSc
     __syncthreads();
     PerlinTab pt{smem, threadIdx.x & 31u};
 
-    const unsigned long long npix = (unsigned long long)rp.width * rp.height;
+    const unsigned long long npix = ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
     unsigned long long nrays = 0;
     for (unsigned long long path = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; path < npaths; path += stride) {
         uint32_t pixel = uint32_t(path % npix);
+        if (ADAPT) pixel = __ldg(rp.adapt_pixels + pixel);
         uint32_t sample = uint32_t(path / npix) + uint32_t(rp.sample_offset);
         Ray r = camera_ray(sc, rp, pixel, sample);
         V3 A = mk(rp.world_r, rp.world_g, rp.world_b); // main.cu:40
@@ -144,7 +147,7 @@ __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DSc
             r = next;
         }
         nrays += shadow_rays;
-        atomicAdd(&accum[pixel], make_float4(result.x + direct.x, result.y + direct.y, result.z + direct.z, 1.f)); // RED.E.ADD.F32x4 (sm_90+)
+        atomicAdd(&accum_plane<ADAPT>(accum, rp, sample)[pixel], make_float4(result.x + direct.x, result.y + direct.y, result.z + direct.z, 1.f)); // RED.E.ADD.F32x4 (sm_90+)
     }
     // one counter update per warp
     for (int off = 16; off > 0; off >>= 1) nrays += __shfl_down_sync(0xffffffffu, nrays, off);
@@ -153,13 +156,15 @@ __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DSc
 
 void launch_render_mega(const DScene& sc, const DRenderParams& rp, bool use_bvh, float4* accum,
                         unsigned long long* ray_counter, int sm_count, cudaStream_t st) {
-    unsigned long long npaths = (unsigned long long)rp.width * rp.height * (unsigned long long)rp.spp;
+    const unsigned long long npix = rp.adapt_pixels ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
+    unsigned long long npaths = npix * (unsigned long long)rp.spp;
     if (npaths == 0) return;
     const size_t smem = RT_PERLIN_SMEM_WORDS * sizeof(uint32_t);
     unsigned long long want = (npaths + 255) / 256;
     unsigned long long cap = (unsigned long long)sm_count * 32; // several waves of resident CTAs, grid-stride beyond
     unsigned blocks = unsigned(want < cap ? want : cap);
-    k_render_mega<<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
+    if (rp.adapt_pixels) k_render_mega<true><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
+    else k_render_mega<false><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
 }
 
 // --------------------------------------------------------------- tonemap ----

@@ -43,6 +43,20 @@ void launch_features(const DScene& sc, const DRenderParams& rp, bool use_bvh, in
 void launch_atrous(const float4* in, bool from_accum, const float4* features, int width, int height, int level, float sigma_color,
                    float sigma_normal, float sigma_depth, float sigma_albedo, float4* out, cudaStream_t st);
 
+// adaptive sampling (rt_adaptive.cu).  planes: two float4 planes of width*height (A: even samples, B: odd samples).
+// Windowed error map of the planes into ebar (e_scratch: width*height floats)
+void launch_adapt_error_map(const float4* planes, int width, int height, float* e_scratch, float* ebar, cudaStream_t st);
+// uint32 words of scratch launch_adapt_select needs besides e_scratch
+size_t adapt_select_scratch_words(uint32_t npix);
+// next = the entries of list (n pixels) whose windowed error is >= tau and whose count is < max_spp, in list order; *n_next
+// (device) = their number; *launches = kernels launched
+cudaError_t launch_adapt_select(const float4* planes, int width, int height, const uint32_t* list, uint32_t n, float tau,
+                                int32_t max_spp, float* e_scratch, uint32_t* words, uint32_t* next, uint32_t* n_next, uint32_t* launches,
+                                cudaStream_t st);
+void launch_adapt_iota(uint32_t* list, uint32_t n, cudaStream_t st);
+// accum = A + B (written, not added)
+void launch_adapt_merge(const float4* planes, uint32_t npix, float4* accum, cudaStream_t st);
+
 // self-test: out[4i..4i+3] = div_rz(x, y), __fdiv_rz(x, y), sqrt_rz(x), __fsqrt_rz(x)  (rt_device.cuh)
 void launch_selftest_rz(const float* x_dev, const float* y_dev, size_t n, float* out_dev, cudaStream_t st);
 
