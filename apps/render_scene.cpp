@@ -6,7 +6,7 @@
 //   render_scene [scene] [width height spp] [out] [earth.ppm]            (positional, as before)
 //   render_scene --scene <name | file.json> [--width W --height H --spp N --depth D --seed S]
 //                [--out render.jpg|.ppm] [--quality 100] [--earth assets/earth_stb.ppm] [--passes K] [--emitter-sampling]
-//                [--gpus N] [--denoise] [--adaptive T [--max-spp N]]
+//                [--gpus N] [--denoise] [--adaptive T [--max-spp N]] [--frames N [--orbit DEG]]
 //     scene: earth_emitter (default) | book1_final | perlin_motion | random_spheres:N | a JSON document
 //            (include/rt/scene_json.hpp; the reference's compile-time scene and WIDTH/HEIGHT/SAMPLES_PER_PIXEL/SEED
 //            macros, main.cu:15,188-356, common.h:13-20, become runtime input)
@@ -25,6 +25,11 @@
 //     --adaptive T: adaptive sampling (rt_render_adaptive): every pixel gets --spp samples, then passes of --spp samples go
 //            to the pixels whose display-space noise estimate is still >= T, up to --max-spp (default 16 x --spp).  With
 //            --denoise the adaptive accumulator goes through the device entries (features, rt_denoise_device).  One device.
+//     --frames N: a sequence of N frames in one render (rt_render_frames_device): the cameras come from rt_orbit_cameras on
+//            the scene's camera, lookfrom turned by --orbit DEG degrees in all (default 0) about the axis through lookat
+//            along up, and the shutter split into N windows (so the moving spheres of perlin_motion move from frame to
+//            frame).  Frame k is written to <stem>_<kkkk><ext> (render_0000.jpg, ...) through rt_tonemap_device and the
+//            device JPEG writer (PPM for other extensions).  One device, one pass, no denoising or adaptive sampling.
 //
 // The earth texture: --earth textures/earth.jpg (decoded by rt_image_load exactly as stbi_loadf does) or a binary PPM
 // of the stb-decoded bytes (assets/earth_stb.ppm, written by __graft_entry__.build()).
@@ -62,6 +67,8 @@ int main(int argc, char** argv) {
     bool adaptive = false;
     float threshold = 0.f;
     int max_spp = 0; // 0: 16 x --spp
+    int frames = 0;  // 0: one frame of the scene's camera
+    float orbit = 0.f;
     rt_render_params p;
     rt_default_render_params(&p); // 1200x600x100, depth 50, seed 1000, tmin 1e-5 (common.h:13-20, main.cu:15,45)
     bool size_given = false;
@@ -90,10 +97,17 @@ int main(int argc, char** argv) {
         else if (a == "--denoise") denoise = true;
         else if (a == "--adaptive") adaptive = true, threshold = float(atof(next("--adaptive")));
         else if (a == "--max-spp") max_spp = atoi(next("--max-spp"));
+        else if (a == "--frames") {
+            frames = atoi(next("--frames"));
+            if (frames < 1) {
+                fprintf(stderr, "--frames needs N >= 1\n");
+                return 2;
+            }
+        } else if (a == "--orbit") orbit = float(atof(next("--orbit")));
         else if (a == "--help" || a == "-h") {
             printf("render_scene --scene <name|file.json> [--width W --height H --spp N --depth D --seed S] [--out f.jpg|f.ppm] "
                    "[--quality Q] [--earth earth.ppm] [--passes K] [--emitter-sampling] [--gpus N] [--denoise] "
-                   "[--adaptive T [--max-spp N]]\n");
+                   "[--adaptive T [--max-spp N]] [--frames N [--orbit DEG]]\n");
             return 0;
         } else pos.push_back(a);
     }
@@ -112,6 +126,10 @@ int main(int argc, char** argv) {
     }
     if (adaptive && (gpus != 1 || passes > 1)) {
         fprintf(stderr, "--adaptive renders on one device and chooses its own passes: it cannot be combined with --gpus or --passes\n");
+        return 2;
+    }
+    if (frames > 0 && (gpus != 1 || passes > 1 || denoise || adaptive)) {
+        fprintf(stderr, "--frames renders one pass per frame on one device: it cannot be combined with --gpus, --passes, --denoise or --adaptive\n");
         return 2;
     }
 
@@ -187,7 +205,51 @@ int main(int argc, char** argv) {
         else CHECK(rt_write_ppm(out_path.c_str(), p.width, p.height, img.data()));
         return 0;
     };
-    if (adaptive) {
+    if (frames > 0) { // one wavefront for the whole sequence, then per frame: finalisation -> 8-bit frame -> file
+        std::vector<rt_camera> cams(frames);
+        CHECK(rt_orbit_cameras(&desc.camera, frames, orbit, cams.data()));
+        const size_t npix = size_t(p.width) * p.height;
+        void *accum = nullptr, *rgb8 = nullptr;
+        if (cudaMalloc(&accum, size_t(frames) * npix * 16) != cudaSuccess || cudaMalloc(&rgb8, npix * 3) != cudaSuccess ||
+            cudaMemset(accum, 0, size_t(frames) * npix * 16) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) {
+            fprintf(stderr, "device allocation failed\n");
+            return 1;
+        }
+        CHECK(rt_render_frames_device(ctx, scene, &p, cams.data(), frames, accum, &st));
+        printf("took %.0fus for %d frames (%.3f ms per frame; %.1f Mpaths/s, %.1f Mrays/s, %u launches)\n", st.ms_total * 1e3, frames,
+               st.ms_total / frames, st.paths / st.ms_total / 1e3, st.rays / st.ms_total / 1e3, st.launches);
+        const size_t slash = out_path.find_last_of('/'), dot = out_path.find_last_of('.');
+        const bool has_ext = dot != std::string::npos && (slash == std::string::npos || dot > slash);
+        const std::string stem = has_ext ? out_path.substr(0, dot) : out_path, ext = has_ext ? out_path.substr(dot) : "";
+        const bool jpg = ext == ".jpg" || ext == ".jpeg";
+        std::vector<uint8_t> file(jpg ? rt_jpeg_max_bytes(p.width, p.height) : npix * 3);
+        for (int k = 0; k < frames; ++k) {
+            char num[16];
+            snprintf(num, sizeof num, "_%04d", k);
+            const std::string path = stem + num + ext;
+            CHECK(rt_tonemap_device(ctx, static_cast<char*>(accum) + size_t(k) * npix * 16, p.width, p.height, nullptr, rgb8));
+            if (jpg) {
+                size_t n = 0;
+                CHECK(rt_jpeg_encode_device(ctx, rgb8, p.width, p.height, quality, file.data(), file.size(), &n, nullptr));
+                FILE* f = fopen(path.c_str(), "wb");
+                const bool ok = f && fwrite(file.data(), 1, n, f) == n;
+                if (f) fclose(f);
+                if (!ok) {
+                    fprintf(stderr, "cannot write %s\n", path.c_str());
+                    return 1;
+                }
+            } else {
+                CHECK(rt_context_synchronize(ctx));
+                if (cudaMemcpy(file.data(), rgb8, npix * 3, cudaMemcpyDeviceToHost) != cudaSuccess) {
+                    fprintf(stderr, "cudaMemcpy failed\n");
+                    return 1;
+                }
+                CHECK(rt_write_ppm(path.c_str(), p.width, p.height, file.data()));
+            }
+        }
+        cudaFree(accum);
+        cudaFree(rgb8);
+    } else if (adaptive) {
         rt_adaptive_params a;
         rt_default_adaptive_params(&a);
         a.min_spp = a.step_spp = p.spp;

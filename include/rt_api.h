@@ -394,6 +394,32 @@ rt_status rt_render_adaptive_device(rt_context* ctx, const rt_scene* scene, cons
 rt_status rt_render_adaptive(rt_context* ctx, const rt_scene* scene, const rt_render_params* p,
                              const rt_adaptive_params* a, float* out_rgb, int32_t* out_spp, rt_stats* stats);
 
+/* ---- frame sequences ----------------------------------------------------------------------------------------------
+ * n_frames frames of one scene in one render: frame f looks through cameras[f] (its time0 / time1 shutter included; the
+ * scene's own camera is not used) and takes the sample indices [p->sample_offset + f*p->spp, p->sample_offset +
+ * (f+1)*p->spp), the convention of rt_render_progressive's passes: frames have independent noise under the same seed.
+ * So frame f is the frame rt_render_accum_device gives on a scene whose camera is cameras[f] with sample_offset =
+ * p->sample_offset + f*p->spp: equal sample counts and ray counts, sums equal up to the order of float additions.  Every
+ * pipeline and RT_RENDER_EMITTER_SAMPLING work as for one frame.  The paths of all frames share one wavefront, so the
+ * next frame's paths fill the thin end of the previous one.  The scene is not re-uploaded; the cameras are (n_frames *
+ * 84 bytes).  Checked before any device work: NULLs, n_frames >= 1, p, every camera finite, and sample_offset +
+ * n_frames*spp <= 2^31 - 1. */
+/* ADDS frame f's samples into accum_dev + f*W*H (n_frames*W*H float4, device, caller zeroes it).  Asynchronous on the
+ * context stream unless stats != NULL; stats: paths = W*H*spp*n_frames, rays, launches, iterations and ms_total of the
+ * whole batch. */
+rt_status rt_render_frames_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_camera* cameras,
+                                  int32_t n_frames, void* accum_dev, rt_stats* stats);
+/* host convenience: out_rgb (HOST) n_frames*W*H*3 floats, frame f from f*W*H*3 on in rt_render's layout; ms_tonemap is the
+ * finalisation of all frames */
+rt_status rt_render_frames(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_camera* cameras,
+                           int32_t n_frames, float* out_rgb, rt_stats* stats);
+/* Cameras of an orbit or a motion sequence (no device needed).  Frame k (0 <= k < n_frames) is *base with lookfrom rotated by
+ * k*degrees/n_frames degrees about the axis through lookat along up (right-hand rule) and the shutter
+ * [t0 + k*(t1-t0)/n_frames, t0 + (k+1)*(t1-t0)/n_frames] of base's [t0, t1] = [time0, time1]: the frames' windows tile
+ * base's.  Computed in double and rounded to float once.  degrees = 0 keeps lookfrom: the frames of a still camera over
+ * successive shutter windows.  Checks: NULLs, n_frames >= 1, degrees and base finite, up not zero. */
+rt_status rt_orbit_cameras(const rt_camera* base, int32_t n_frames, float degrees, rt_camera* out);
+
 /* ---- multi-GPU (SURVEY.md 8e; BASELINE.json north_star (4))---------------------------------------------------
  * Samples per pixel are split across the GPUs of one box: GPU r renders sample indices [first_r, first_r + count_r) of
  * EVERY pixel (rt_render_params.sample_offset; the Philox keys use the global sample index, so the image does not depend

@@ -162,6 +162,10 @@ _SIGNATURES = {
                                             C.POINTER(C.c_int32), C.POINTER(rt_stats)]),
     "rt_render_adaptive": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_adaptive_params), _VP, _VP,
                                      C.POINTER(rt_stats)]),
+    "rt_render_frames_device": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.c_int32, _VP,
+                                          C.POINTER(rt_stats)]),
+    "rt_render_frames": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), C.POINTER(rt_camera), C.c_int32, _VP, C.POINTER(rt_stats)]),
+    "rt_orbit_cameras": (C.c_int, [C.POINTER(rt_camera), C.c_int32, C.c_float, C.POINTER(rt_camera)]),
     "rt_reduce_tonemap_peers": (C.c_int, [_VP, C.POINTER(_VP), C.c_int32, _VP, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                           _VP, _VP, _VP]),
     "rt_shard_samples": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
@@ -497,6 +501,24 @@ class Scene:
                                                             _VP(error_ptr or None), C.byref(passes), C.byref(st) if st is not None else None))
         return passes.value, st
 
+    def render_frames(self, params: rt_render_params, cameras):
+        """rt_render_frames: frame f of the sequence looks through cameras[f] (a sequence of rt_camera, e.g. from orbit_cameras)
+        with samples params.sample_offset + f * params.spp + [0, spp).  Returns (HOST float RGB [K, H, W, 3], frame f in the
+        layout of render, stats)."""
+        cams = _camera_array(cameras)
+        out = np.empty((len(cams), params.height, params.width, 3), dtype=np.float32)
+        st = rt_stats()
+        _check(self.lib, self.lib.rt_render_frames(self.ctx._h, self._h, C.byref(params), cams, len(cams), out.ctypes.data, C.byref(st)))
+        return out, st
+
+    def render_frames_device(self, params: rt_render_params, cameras, accum_ptr: int, want_stats: bool = False):
+        """rt_render_frames_device: ADDS frame f into accum_ptr + f * W * H float4 (device).  Returns stats or None."""
+        cams = _camera_array(cameras)
+        st = rt_stats() if want_stats else None
+        _check(self.lib, self.lib.rt_render_frames_device(self.ctx._h, self._h, C.byref(params), cams, len(cams), _VP(accum_ptr),
+                                                          C.byref(st) if st is not None else None))
+        return st
+
     def close(self) -> None:
         if self._h:
             if self.ctx._open.pop(self._h.value, None):  # (else the context has been closed and destroyed the scene with it)
@@ -508,6 +530,20 @@ class Scene:
             self.close()
         except Exception:
             pass
+
+
+def _camera_array(cameras):
+    cams = list(cameras)
+    return (rt_camera * len(cams))(*cams)
+
+
+def orbit_cameras(base: rt_camera, n: int, degrees: float):
+    """rt_orbit_cameras: n cameras, frame k = base with lookfrom rotated by k * degrees / n about the axis through lookat along
+    up and the k-th of n equal shutter windows of [base.time0, base.time1].  Needs no device."""
+    lib = load_library()
+    out = (rt_camera * max(int(n), 1))()
+    _check(lib, lib.rt_orbit_cameras(C.byref(base), int(n), float(degrees), out))
+    return list(out)
 
 
 def tonemap_device(ctx: Context, accum_ptr: int, width: int, height: int, out_rgb_ptr: int = 0, out_rgb8_ptr: int = 0):

@@ -99,6 +99,17 @@ rt_status dev_alloc(rt_scene* s, T** out, size_t count) {
     return RT_OK;
 }
 
+} // namespace
+namespace rtd {
+// every parameter of a camera finite (scene descriptions, frame sequences, rt_orbit_cameras)
+bool camera_finite(const rt_camera& c) {
+    auto finite3 = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
+    return finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && std::isfinite(c.vfov) && std::isfinite(c.aspect) &&
+           std::isfinite(c.aperture) && std::isfinite(c.focus_dist) && std::isfinite(c.time0) && std::isfinite(c.time1);
+}
+} // namespace rtd
+namespace {
+
 // camera ctor (camera.h:7-31) in host float arithmetic
 void make_camera(const rt_camera& c, rtd::DCamera& out) {
     auto V = [](const float* p) { return rtd::V3{p[0], p[1], p[2]}; };
@@ -164,10 +175,7 @@ rt_status validate_desc(const rt_scene_desc* d) {
                       std::isfinite(sp.time1),
                   "sphere centre / radius / time is not finite");
     }
-    const rt_camera& c = d->camera;
-    ARG_CHECK(finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && std::isfinite(c.vfov) && std::isfinite(c.aspect) &&
-                  std::isfinite(c.aperture) && std::isfinite(c.focus_dist) && std::isfinite(c.time0) && std::isfinite(c.time1),
-              "camera parameter is not finite");
+    ARG_CHECK(rtd::camera_finite(d->camera), "camera parameter is not finite");
     return RT_OK;
 }
 
@@ -204,6 +212,8 @@ rtd::DRenderParams to_device_params(const rt_render_params& p) {
     d.adapt_pixels = nullptr;
     d.adapt_first = 0;
     d.adapt_plane = 0;
+    d.frame_cams = nullptr;
+    d.div_spp = rtd::make_fastdiv(1u);
     return d;
 }
 
@@ -315,15 +325,16 @@ rt_status render_pass(rt_context* ctx, const rt_scene* scene, const rtd::DRender
     return RT_OK;
 }
 
-// Core: adds p->spp samples per pixel into accum (device).  Fills stats if requested
+// Core: adds rp.spp samples per pixel into accum (device).  Fills stats if requested
 // (which synchronises the stream).
-rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float4* accum, rt_stats* stats) {
+rt_status render_rp(rt_context* ctx, const rt_scene* scene, const rtd::DRenderParams& rp, uint32_t pipeline, float4* accum,
+                    rt_stats* stats) {
     uint32_t launches = 0, iterations = 0;
     if (stats) {
         CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), ctx->stream));
         CUDA_TRY(cudaEventRecord(ctx->ev[0], ctx->stream));
     }
-    rt_status st = render_pass(ctx, scene, to_device_params(*p), p->pipeline, accum, &launches, &iterations);
+    rt_status st = render_pass(ctx, scene, rp, pipeline, accum, &launches, &iterations);
     if (st != RT_OK) return st;
     if (stats) {
         CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
@@ -332,12 +343,16 @@ rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_pa
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         memset(stats, 0, sizeof *stats);
         CUDA_TRY(cudaEventElapsedTime(&stats->ms_total, ctx->ev[0], ctx->ev[1]));
-        stats->paths = uint64_t(p->width) * uint64_t(p->height) * uint64_t(p->spp);
+        stats->paths = uint64_t(rp.width) * uint64_t(rp.height) * uint64_t(rp.spp);
         stats->rays = rays;
         stats->launches = launches;
         stats->iterations = iterations;
     }
     return RT_OK;
+}
+
+rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float4* accum, rt_stats* stats) {
+    return render_rp(ctx, scene, to_device_params(*p), p->pipeline, accum, stats);
 }
 
 } // namespace
@@ -1361,6 +1376,81 @@ rt_status rt_render_adaptive(rt_context* ctx, const rt_scene* scene, const rt_re
     CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
     CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
     local.launches += 1;
+    if (stats) *stats = local;
+    return RT_OK;
+} RT_API_CATCH
+
+} // extern "C"
+
+namespace {
+
+rt_status check_frames(const rt_render_params* p, const rt_camera* cameras, int32_t n_frames) {
+    ARG_CHECK(cameras != nullptr, "cameras is NULL");
+    ARG_CHECK(n_frames >= 1, "n_frames must be >= 1");
+    rt_status st = check_params(p);
+    if (st != RT_OK) return st;
+    for (int32_t f = 0; f < n_frames; ++f) ARG_CHECK(rtd::camera_finite(cameras[f]), "camera parameter is not finite");
+    ARG_CHECK(int64_t(p->sample_offset) + int64_t(n_frames) * int64_t(p->spp) <= INT32_MAX, "sample indices exceed 2^31 - 1");
+    return RT_OK;
+}
+
+// A frame sequence as ONE render of n_frames * spp samples per pixel: sample block f (frame_of, rt_device.cuh) looks through
+// cameras[f] and adds into accum + f * W * H, so the wavefront runs the frames back to back in one pool and one poll loop.
+rt_status frames_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_camera* cameras, int32_t n_frames,
+                      float4* accum, rt_stats* stats) {
+    std::vector<rtd::DCamera> cams(static_cast<size_t>(n_frames));
+    for (int32_t f = 0; f < n_frames; ++f) make_camera(cameras[f], cams[f]);
+    rtd::DCamera* d_cams = nullptr;
+    CUDA_TRY(rtd::malloc_async(&d_cams, cams.size() * sizeof(rtd::DCamera), ctx->stream));
+    const rt_status st = [&]() -> rt_status {
+        CUDA_TRY(cudaMemcpyAsync(d_cams, cams.data(), cams.size() * sizeof(rtd::DCamera), cudaMemcpyHostToDevice, ctx->stream));
+        rtd::DRenderParams rp = to_device_params(*p);
+        rp.spp = p->spp * n_frames; // <= 2^31 - 1: check_frames
+        rp.frame_cams = d_cams;
+        rp.div_spp = rtd::make_fastdiv(uint32_t(p->spp));
+        return render_rp(ctx, scene, rp, p->pipeline, accum, stats);
+    }();
+    cudaFreeAsync(d_cams, ctx->stream);
+    return st;
+}
+
+} // namespace
+
+extern "C" {
+
+rt_status rt_render_frames_device(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_camera* cameras,
+                                  int32_t n_frames, void* accum_dev, rt_stats* stats) try {
+    ARG_CHECK(ctx && scene && accum_dev, "ctx/scene/accum_dev is NULL");
+    rt_status st = check_frames(p, cameras, n_frames);
+    if (st != RT_OK) return st;
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    return frames_into(ctx, scene, p, cameras, n_frames, static_cast<float4*>(accum_dev), stats);
+} RT_API_CATCH
+
+rt_status rt_render_frames(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, const rt_camera* cameras,
+                           int32_t n_frames, float* out_rgb, rt_stats* stats) try {
+    ARG_CHECK(ctx && scene && out_rgb, "ctx/scene/out_rgb is NULL");
+    rt_status st = check_frames(p, cameras, n_frames);
+    if (st != RT_OK) return st;
+    if ((st = make_current(ctx)) != RT_OK) return st;
+    const size_t npix = size_t(p->width) * size_t(p->height), total = npix * size_t(n_frames);
+    if ((st = ensure_accum(ctx, total)) != RT_OK) return st;
+    if ((st = ensure_out(ctx, total)) != RT_OK) return st;
+    CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, total * sizeof(float4), ctx->stream));
+    rt_stats local;
+    if ((st = frames_into(ctx, scene, p, cameras, n_frames, ctx->accum, &local)) != RT_OK) return st;
+    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
+    for (int32_t f = 0; f < n_frames; ++f)
+        rtd::launch_tonemap(ctx->accum + size_t(f) * npix, p->width, p->height, ctx->out_rgb + size_t(f) * npix * 3, nullptr,
+                            ctx->sm_count, ctx->stream);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, total * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
+    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    local.launches += uint32_t(n_frames);
     if (stats) *stats = local;
     return RT_OK;
 } RT_API_CATCH

@@ -186,12 +186,27 @@ struct DRenderParams {
     const uint32_t* adapt_pixels;
     uint32_t adapt_first;
     uint32_t adapt_plane;
+    // Frame sequences (the FRAMES instantiations; nullptr otherwise): spp counts the samples of the whole batch, n_frames
+    // times div_spp.d per pixel.  Sample s belongs to frame f = (s - sample_offset) / div_spp.d, whose camera is
+    // frame_cams[f] and whose accumulator is the f-th width*height block of float4 (rt_api.cu, frames_into).
+    const DCamera* frame_cams;
+    FastDiv div_spp;
 };
 
-// the float4 accumulator a path of `sample` adds into: the render's own, or in ADAPT instantiations the plane of the sample's parity
-template <bool ADAPT>
+// Which paths a render kernel instantiation traces (its RM template argument): every pixel of the frame (RM_PLAIN), the
+// pixel list of an adaptive pass (RM_ADAPT), or the frames of a sequence (RM_FRAMES).
+enum : int { RM_PLAIN = 0, RM_ADAPT = 1, RM_FRAMES = 2 };
+
+// frame of a sample in FRAMES instantiations (computed at ray generation and at accumulation only, never per bounce)
+RT_DEV uint32_t frame_of(const DRenderParams& rp, uint32_t sample) { return fastdiv(sample - uint32_t(rp.sample_offset), rp.div_spp); }
+
+// the float4 accumulator a path of `sample` adds into: the render's own, in ADAPT instantiations the plane of the sample's
+// parity, in FRAMES instantiations the sample's frame
+template <int RM>
 RT_DEV float4* accum_plane(float4* accum, const DRenderParams& rp, uint32_t sample) {
-    return ADAPT ? accum + size_t((sample - rp.adapt_first) & 1u) * rp.adapt_plane : accum;
+    if (RM == RM_ADAPT) return accum + size_t((sample - rp.adapt_first) & 1u) * rp.adapt_plane;
+    if (RM == RM_FRAMES) return accum + size_t(frame_of(rp, sample)) * rp.div_npix.d;
+    return accum;
 }
 
 struct Ray {

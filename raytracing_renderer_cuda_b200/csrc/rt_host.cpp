@@ -1,5 +1,6 @@
 // rt_host.cpp — host-only entry points of the C-ABI: built-in scenes (through the
 // façade), scene-description files, and the reference's writer conversion.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -13,6 +14,7 @@
 
 namespace rtd {
 void set_error_message(const char* msg); // rt_api.cu
+bool camera_finite(const rt_camera& c); // rt_api.cu
 }
 
 namespace {
@@ -41,6 +43,36 @@ size_t rt_abi_sizeof(const char* name) {
     RT_SZ(rt_denoise_params); RT_SZ(rt_adaptive_params);
 #undef RT_SZ
     return 0;
+}
+
+rt_status rt_orbit_cameras(const rt_camera* base, int32_t n_frames, float degrees, rt_camera* out) {
+    auto fail = [](const char* msg) {
+        rtd::set_error_message((std::string("invalid argument: ") + msg).c_str());
+        return RT_ERR_INVALID_ARG;
+    };
+    if (!base || !out) return fail("base/out is NULL");
+    if (n_frames < 1) return fail("n_frames must be >= 1");
+    if (!std::isfinite(degrees) || !rtd::camera_finite(*base)) return fail("degrees / camera parameter is not finite");
+    const double ux = base->up[0], uy = base->up[1], uz = base->up[2], ul = std::sqrt(ux * ux + uy * uy + uz * uz);
+    if (!(ul > 0.0)) return fail("camera up is zero");
+    // Rodrigues' rotation of v = lookfrom - lookat about the unit axis a = up / |up|:
+    //   v' = v cos(th) + (a x v) sin(th) + a (a . v) (1 - cos(th))
+    const double ax = ux / ul, ay = uy / ul, az = uz / ul;
+    const double vx = double(base->lookfrom[0]) - base->lookat[0], vy = double(base->lookfrom[1]) - base->lookat[1],
+                 vz = double(base->lookfrom[2]) - base->lookat[2];
+    const double adv = ax * vx + ay * vy + az * vz;
+    const double t0 = base->time0, t1 = base->time1, n = n_frames;
+    for (int32_t k = 0; k < n_frames; ++k) {
+        const double th = double(degrees) * k / n * (M_PI / 180.0), c = std::cos(th), s = std::sin(th);
+        rt_camera cam = *base;
+        cam.lookfrom[0] = float(base->lookat[0] + (vx * c + (ay * vz - az * vy) * s + ax * adv * (1.0 - c)));
+        cam.lookfrom[1] = float(base->lookat[1] + (vy * c + (az * vx - ax * vz) * s + ay * adv * (1.0 - c)));
+        cam.lookfrom[2] = float(base->lookat[2] + (vz * c + (ax * vy - ay * vx) * s + az * adv * (1.0 - c)));
+        cam.time0 = float(t0 + (t1 - t0) * k / n);
+        cam.time1 = float(t0 + (t1 - t0) * (k + 1) / n);
+        out[k] = cam;
+    }
+    return RT_OK;
 }
 
 rt_status rt_quantize_rgb8(const float* rgb, int32_t width, int32_t height, uint8_t* out) {

@@ -103,8 +103,9 @@ void launch_shade_probe(const DScene& sc, const DRenderParams& rp, const rt_ray*
 // covers 32 neighbouring pixels of one sample.  This is the reference's structure
 // (render + color(), main.cu:35-74,97-132) on the flat scene; it is kept as the
 // RT_PIPE_MEGAKERNEL pipeline and as the yardstick the wavefront pipeline is measured against.
-// ADAPT: adaptive sampling, path -> pixel rp.adapt_pixels[path mod n] (n = div_npix.d), values into the sample's parity plane.
-template <bool ADAPT>
+// RM_ADAPT: adaptive sampling, path -> pixel rp.adapt_pixels[path mod n] (n = div_npix.d), values into the sample's parity plane.
+// RM_FRAMES: a frame sequence, the camera and the accumulator of the sample's frame (DRenderParams::frame_cams).
+template <int RM>
 __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp,
                                                      int use_bvh, float4* __restrict__ accum,
                                                      unsigned long long* __restrict__ ray_counter) {
@@ -113,15 +114,15 @@ __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DSc
     __syncthreads();
     PerlinTab pt{smem, threadIdx.x & 31u};
 
-    const unsigned long long npix = ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
+    const unsigned long long npix = RM == RM_ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
     unsigned long long nrays = 0;
     for (unsigned long long path = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; path < npaths; path += stride) {
         uint32_t pixel = uint32_t(path % npix);
-        if (ADAPT) pixel = __ldg(rp.adapt_pixels + pixel);
+        if (RM == RM_ADAPT) pixel = __ldg(rp.adapt_pixels + pixel);
         uint32_t sample = uint32_t(path / npix) + uint32_t(rp.sample_offset);
-        Ray r = camera_ray(sc, rp, pixel, sample);
+        Ray r = camera_ray<RM>(sc, rp, pixel, sample);
         V3 A = mk(rp.world_r, rp.world_g, rp.world_b); // main.cu:40
         V3 result = mk(0.f, 0.f, 0.f);                 // exceeded recursion (main.cu:70)
         V3 direct = mk(0.f, 0.f, 0.f);                 // shadow/emission rays of the path (RT_RENDER_EMITTER_SAMPLING)
@@ -147,7 +148,7 @@ __global__ void __launch_bounds__(256) k_render_mega(const __grid_constant__ DSc
             r = next;
         }
         nrays += shadow_rays;
-        atomicAdd(&accum_plane<ADAPT>(accum, rp, sample)[pixel], make_float4(result.x + direct.x, result.y + direct.y, result.z + direct.z, 1.f)); // RED.E.ADD.F32x4 (sm_90+)
+        atomicAdd(&accum_plane<RM>(accum, rp, sample)[pixel], make_float4(result.x + direct.x, result.y + direct.y, result.z + direct.z, 1.f)); // RED.E.ADD.F32x4 (sm_90+)
     }
     // one counter update per warp
     for (int off = 16; off > 0; off >>= 1) nrays += __shfl_down_sync(0xffffffffu, nrays, off);
@@ -163,8 +164,9 @@ void launch_render_mega(const DScene& sc, const DRenderParams& rp, bool use_bvh,
     unsigned long long want = (npaths + 255) / 256;
     unsigned long long cap = (unsigned long long)sm_count * 32; // several waves of resident CTAs, grid-stride beyond
     unsigned blocks = unsigned(want < cap ? want : cap);
-    if (rp.adapt_pixels) k_render_mega<true><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
-    else k_render_mega<false><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
+    if (rp.adapt_pixels) k_render_mega<RM_ADAPT><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
+    else if (rp.frame_cams) k_render_mega<RM_FRAMES><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
+    else k_render_mega<RM_PLAIN><<<blocks, 256, smem, st>>>(sc, rp, use_bvh ? 1 : 0, accum, ray_counter);
 }
 
 // --------------------------------------------------------------- tonemap ----

@@ -212,8 +212,7 @@ RT_DEV V3 texture_value(const DScene& sc, const PerlinTab& pt, int32_t ix, V3 n,
 // ------------------------------------------------------------------ camera ----
 // render()'s per-sample set-up (main.cu:116-118) + camera::get_ray (camera.h:33-38).
 // Draw order of the reference: jitter x, jitter y, lens disk, shutter time.
-RT_DEV Ray camera_ray(const DScene& sc, const DRenderParams& rp, uint32_t pixel, uint32_t sample) {
-    const DCamera& cam = sc.cam;
+RT_DEV Ray camera_ray_of(const DCamera& cam, const DRenderParams& rp, uint32_t pixel, uint32_t sample) {
     const uint32_t j = fastdiv(pixel, rp.div_width), i = pixel - j * uint32_t(rp.width);
     U4 r0 = rng_block(rp.seed, pixel, sample, 0, 0);
     float s = float(i + u01(r0.x)) / float(rp.width);
@@ -232,6 +231,21 @@ RT_DEV Ray camera_ray(const DScene& sc, const DRenderParams& rp, uint32_t pixel,
     r.d = cam.lower_left + s * cam.horizontal + t * cam.vertical - cam.origin - offset;
     r.time = time;
     return r;
+}
+
+// The camera ray of a path: through the scene's camera, or in FRAMES instantiations through the camera of the sample's frame
+template <int RM = RM_PLAIN>
+RT_DEV Ray camera_ray(const DScene& sc, const DRenderParams& rp, uint32_t pixel, uint32_t sample) {
+    if constexpr (RM == RM_FRAMES) {
+        DCamera cam;
+        const float* src = reinterpret_cast<const float*>(rp.frame_cams + frame_of(rp, sample));
+        float* dst = reinterpret_cast<float*>(&cam);
+#pragma unroll
+        for (int k = 0; k < int(sizeof(DCamera) / sizeof(float)); ++k) dst[k] = __ldg(src + k);
+        return camera_ray_of(cam, rp, pixel, sample);
+    } else {
+        return camera_ray_of(sc.cam, rp, pixel, sample);
+    }
 }
 
 // ------------------------------------------------------------------ materials ----

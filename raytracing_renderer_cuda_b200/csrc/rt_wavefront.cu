@@ -196,8 +196,10 @@ struct WfLane {
 // scatter.  Returns true when a new ray (ln.r) has to be extended.  Otherwise the entry is finished here —
 // emitter, absorbed ray, depth limit, or no path left — and `out_q` says where the slot goes (Q_NEW / Q_NONE).
 // NEE = RT_RENDER_EMITTER_SAMPLING (a separate instantiation: the reference estimator's kernels do not change).
-// ADAPT = adaptive sampling: new paths take their pixel from rp.adapt_pixels, values go to the plane of the sample's parity.
-template <bool NEE, int STREAM, bool ADAPT = false>
+// RM = RM_ADAPT: adaptive sampling, new paths take their pixel from rp.adapt_pixels, values go to the plane of the sample's
+// parity.  RM = RM_FRAMES: a frame sequence, new paths look through the camera of their sample's frame and values go to
+// that frame's accumulator.  Neither changes the path record: pixel and sample determine both.
+template <bool NEE, int STREAM, int RM = RM_PLAIN>
 RT_DEV bool wf_begin(const DScene& sc, const DRenderParams& rp, const WfBuffers& wb, const PerlinTab& pt, int kind, bool valid,
                      uint32_t slot, uint32_t idx, const PathMap& pm, float4* __restrict__ accum, WfLane& ln, int& out_q) {
     const V3 bloom = mk(rp.bloom, rp.bloom, rp.bloom);
@@ -218,11 +220,11 @@ RT_DEV bool wf_begin(const DScene& sc, const DRenderParams& rp, const WfBuffers&
             if (idx < pm.n_valid) {
                 const uint32_t x = pm.pix_base + idx, q = fastdiv(x, rp.div_npix);
                 pixel = x - q * rp.div_npix.d;
-                if (ADAPT) pixel = __ldg(rp.adapt_pixels + pixel);
+                if (RM == RM_ADAPT) pixel = __ldg(rp.adapt_pixels + pixel);
                 sample = pm.smp_base + q + uint32_t(rp.sample_offset);
                 A = mk(rp.world_r, rp.world_g, rp.world_b);
                 if (rp.max_depth > 0) {
-                    r = camera_ray(sc, rp, pixel, sample);
+                    r = camera_ray<RM>(sc, rp, pixel, sample);
                     has_ray = true;
                 } else { // exceeded recursion before the first hit test (main.cu:42,70)
                     A = mk(0.f, 0.f, 0.f);
@@ -273,7 +275,7 @@ RT_DEV bool wf_begin(const DScene& sc, const DRenderParams& rp, const WfBuffers&
                     scatter_lambertian(q, p, n, rn, r);
                     if (NEE && int(bounce) < rp.max_depth) { // the hit's shadow/emission ray (rt_shade.cuh), traced right here
                         const V3 c = emitter_sample(sc, rp, pt, p, n, q.time, pixel, sample, bounce, shadow_rays);
-                        if (c.x != 0.f || c.y != 0.f || c.z != 0.f) atomicAdd(&accum_plane<ADAPT>(accum, rp, sample)[pixel], make_float4(c.x, c.y, c.z, 0.f));
+                        if (c.x != 0.f || c.y != 0.f || c.z != 0.f) atomicAdd(&accum_plane<RM>(accum, rp, sample)[pixel], make_float4(c.x, c.y, c.z, 0.f));
                         nee_vertex = true;
                     }
                 }
@@ -294,7 +296,7 @@ RT_DEV bool wf_begin(const DScene& sc, const DRenderParams& rp, const WfBuffers&
             }
         }
     }
-    if (finished) atomicAdd(&accum_plane<ADAPT>(accum, rp, sample)[pixel], make_float4(A.x, A.y, A.z, 1.f));
+    if (finished) atomicAdd(&accum_plane<RM>(accum, rp, sample)[pixel], make_float4(A.x, A.y, A.z, 1.f));
     out_q = slot_free ? int(Q_NEW) : Q_NONE;
     ln.nee_vertex = nee_vertex;
     ln.shadow_rays = shadow_rays;
@@ -309,7 +311,7 @@ RT_DEV bool wf_begin(const DScene& sc, const DRenderParams& rp, const WfBuffers&
 
 // Second half: the closest hit `h` of ln.r is known.  Miss / constant emitter: the path ends (accumulate, slot to
 // Q_NEW); otherwise the record is stored and the slot goes to the shading queue of the hit.  Returns that queue.
-template <bool NEE, int STREAM, bool ADAPT = false>
+template <bool NEE, int STREAM, int RM = RM_PLAIN>
 RT_DEV int wf_finish(const DScene& sc, const DRenderParams& rp, const WfBuffers& wb, float4* __restrict__ accum, WfLane& ln,
                      const RayQ& q, Hit h) {
     WfRecord* rec = wb.rec + ln.slot;
@@ -337,7 +339,7 @@ RT_DEV int wf_finish(const DScene& sc, const DRenderParams& rp, const WfBuffers&
         }
     }
     if (finished) {
-        atomicAdd(&accum_plane<ADAPT>(accum, rp, ln.sample)[ln.pixel], make_float4(A.x, A.y, A.z, 1.f));
+        atomicAdd(&accum_plane<RM>(accum, rp, ln.sample)[ln.pixel], make_float4(A.x, A.y, A.z, 1.f));
         out_q = Q_NEW;
     }
     return out_q;
@@ -345,13 +347,13 @@ RT_DEV int wf_finish(const DScene& sc, const DRenderParams& rp, const WfBuffers&
 
 // One whole queue entry (the CTA-chunk and warp-chunk kernels): begin, closest hit, finish.  Called by all 32 lanes of
 // the warp (the BVH traversal is warp-cooperative); `valid` = false for lanes past the end of the queue.
-template <bool USE_BVH, bool NEE, int ACC = WF_STREAM, int LIST = 0, bool ADAPT = false>
+template <bool USE_BVH, bool NEE, int ACC = WF_STREAM, int LIST = 0, int RM = RM_PLAIN>
 RT_DEV int wf_process_entry(const DScene& sc, const DRenderParams& rp, const WfBuffers& wb, const PerlinTab& pt, int kind,
                             bool valid, uint32_t slot, uint32_t idx, const PathMap& pm, float4* __restrict__ accum,
                             unsigned long long& nrays) {
     WfLane ln;
     int out_q;
-    const bool has_ray = wf_begin<NEE, ACC, ADAPT>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, ln, out_q);
+    const bool has_ray = wf_begin<NEE, ACC, RM>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, ln, out_q);
     if (NEE) nrays += ln.shadow_rays;
     if (USE_BVH) {
         const RayQ q = make_rayq(ln.r);
@@ -363,13 +365,13 @@ RT_DEV int wf_process_entry(const DScene& sc, const DRenderParams& rp, const WfB
 #endif
         if (has_ray) {
             ++nrays;
-            out_q = wf_finish<NEE, ACC, ADAPT>(sc, rp, wb, accum, ln, q, h);
+            out_q = wf_finish<NEE, ACC, RM>(sc, rp, wb, accum, ln, q, h);
         }
     } else if (has_ray) {
         const RayQ q = make_rayq(ln.r);
         const Hit h = closest_hit_list<LIST>(sc, q, rp.tmin);
         ++nrays;
-        out_q = wf_finish<NEE, ACC, ADAPT>(sc, rp, wb, accum, ln, q, h);
+        out_q = wf_finish<NEE, ACC, RM>(sc, rp, wb, accum, ln, q, h);
     }
     return out_q;
 }
@@ -396,7 +398,7 @@ RT_DEV bool wf_frame_done(const WfBuffers& wb, const uint32_t* cnt_cur, int it, 
 // block-wide barriers per chunk.  Best when all rays of a chunk cost the same (brute-force scenes): C1 runs 11 % faster
 // this way than with warp chunks, whose atomic traffic (~1 atomic per 3.5 ns and queue counter) saturates the L2
 // atomic units.
-template <bool USE_BVH, bool NEE, int LIST = 0, bool ADAPT = false>
+template <bool USE_BVH, bool NEE, int LIST = 0, int RM = RM_PLAIN>
 __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
     k_wf_step_cta(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp, const __grid_constant__ WfBuffers wb,
               int it, float4* __restrict__ accum, unsigned long long* __restrict__ ray_counter) {
@@ -440,7 +442,7 @@ __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
     // Tail iterations hold a few hundred live paths: CTAs without a chunk leave before staging anything, and
     // the Perlin table is staged only by CTAs that will run a noise shader (their first chunk is the
     // lowest-numbered one they get, and the noise queues come first; textured emitters may need it too).
-    const unsigned long long npix = ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
+    const unsigned long long npix = RM == RM_ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     if (blockIdx.x == 0 && threadIdx.x == 0) wf_advance_paths(wb, it, path_base, n_q[Q_NEW], npix);
     if (blockIdx.x >= total_chunks) return;
@@ -484,7 +486,7 @@ __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
         const uint32_t idx = ck.first + threadIdx.x;
         const bool valid = idx < ck.n_kind;
 
-        const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, LIST, ADAPT>(sc, rp, wb, pt, ck.kind, valid, slot, idx, pm, accum, nrays);
+        const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, LIST, RM>(sc, rp, wb, pt, ck.kind, valid, slot, idx, pm, accum, nrays);
 
         // ---- queue push: warp ballot -> shared counters -> one global atomic per queue ----
         uint32_t local = 0;
@@ -540,7 +542,7 @@ __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
 #endif
 #define WF_TAIL_MINBLOCKS (1024 / WF_TAIL_THREADS)
 #define WF_TAIL_DEAD 0xffffffffu
-template <bool USE_BVH, bool NEE, int LIST = 0, bool ADAPT = false>
+template <bool USE_BVH, bool NEE, int LIST = 0, int RM = RM_PLAIN>
 __global__ void __launch_bounds__(WF_TAIL_THREADS, WF_TAIL_MINBLOCKS)
     k_wf_tail(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp, const __grid_constant__ WfBuffers wb,
               float4* __restrict__ accum, unsigned long long* __restrict__ ray_counter) {
@@ -608,7 +610,7 @@ __global__ void __launch_bounds__(WF_TAIL_THREADS, WF_TAIL_MINBLOCKS)
             for (int k = 1; k < NQ; ++k) kind += (i >= s_off[k]) ? 1 : 0; // (an empty class has s_off[k] == s_off[k + 1]: skipped)
             const bool valid = i - s_off[kind] < s_cin[kind];
             const uint32_t slot = valid ? s_in[i] : 0u;
-            const int out_q = wf_process_entry<USE_BVH, NEE, WF_ACC_PLAIN, LIST, ADAPT>(sc, rp, wb, pt, kind, valid, slot, 0u, pm, accum, nrays);
+            const int out_q = wf_process_entry<USE_BVH, NEE, WF_ACC_PLAIN, LIST, RM>(sc, rp, wb, pt, kind, valid, slot, 0u, pm, accum, nrays);
             const bool live = valid && out_q != Q_NONE && out_q != Q_NEW;
             s_out[i] = live ? (slot | uint32_t(out_q) << 28) : WF_TAIL_DEAD;
             if (live) atomicAdd(&s_cnt[out_q], 1u);
@@ -661,7 +663,7 @@ __global__ void __launch_bounds__(WF_TAIL_THREADS, WF_TAIL_MINBLOCKS)
 #define RT_PT_REFILL_DEFAULT 16
 #endif
 
-template <bool USE_BVH, bool NEE, bool ADAPT = false>
+template <bool USE_BVH, bool NEE, int RM = RM_PLAIN>
 __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
     k_wf_step_warp(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp, const __grid_constant__ WfBuffers wb,
               int it, float4* __restrict__ accum, unsigned long long* __restrict__ ray_counter) {
@@ -696,7 +698,7 @@ __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
     // Tail iterations hold a few hundred live paths: CTAs without a chunk leave before staging anything, and
     // the Perlin table is staged only by CTAs that will run a noise shader (their first chunk is the
     // lowest-numbered one they get, and the noise queues come first; textured emitters may need it too).
-    const unsigned long long npix = ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
+    const unsigned long long npix = RM == RM_ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     if (blockIdx.x == 0 && threadIdx.x == 0) wf_advance_paths(wb, it, path_base, n_q[Q_NEW], npix);
     const uint32_t warps_per_cta = WF_THREADS / 32;
@@ -735,7 +737,7 @@ __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
             const uint32_t idx = first + uint32_t(e) * 32u + lane;
             const bool valid = idx < n_kind;
             const uint32_t slot = valid ? wf_qload<WF_STREAM>(q_in + idx) : 0u;
-            const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, 0, ADAPT>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, nrays);
+            const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, 0, RM>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, nrays);
                 outq_pack |= uint32_t(out_q + 1) << (4 * e);
         }
 
@@ -784,7 +786,7 @@ __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
 // 775-820 (11 of 32), this kernel 880-940.  On C2/C3 (a few hundred spheres, shading a third of the work) the
 // partial-width shading of refilled lanes costs more than the traversal gains (C2: 10.3 -> 7.1 Grays/s), so the
 // kernel is used from RT_PT_MIN_SPHERES primitives on.
-template <bool NEE, bool QUANT, bool ADAPT = false>
+template <bool NEE, bool QUANT, int RM = RM_PLAIN>
 __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
     k_wf_step_pt(const __grid_constant__ DScene sc, const __grid_constant__ DRenderParams rp, const __grid_constant__ WfBuffers wb,
                  int it, float4* __restrict__ accum, unsigned long long* __restrict__ ray_counter, int refill, int leaf_lanes) {
@@ -819,7 +821,7 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
         if (order[k] == Q_EMIT) n_emit = n;
         if (order[k] == Q_NEW) n_new = n;
     }
-    const unsigned long long npix = ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
+    const unsigned long long npix = RM == RM_ADAPT ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     if (blockIdx.x == 0 && threadIdx.x == 0) wf_advance_paths(wb, it, path_base, n_new, npix);
     if (blockIdx.x * (WF_PT_THREADS / 32) >= total_chunks) return;
@@ -874,7 +876,7 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
             int out_q = Q_NONE;
             if (tracing && t.node == RT_TRAV_DONE && t.leaf >= 0) { // (t.leaf < 0: a postponed leaf, -DRT_PT_POSTPONE only)
                 ++nrays;
-                out_q = wf_finish<NEE, WF_PT_STREAM, ADAPT>(sc, rp, wb, accum, ln, q, t.best);
+                out_q = wf_finish<NEE, WF_PT_STREAM, RM>(sc, rp, wb, accum, ln, q, t.best);
                 tracing = false;
             }
             push(out_q, ln.slot);
@@ -903,7 +905,7 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
             if (!tracing && rank < navail) {
                 const uint32_t idx = pos + rank;
                 const uint32_t slot = wf_qload<WF_PT_STREAM>(q_in + idx);
-                if (wf_begin<NEE, WF_PT_STREAM, ADAPT>(sc, rp, wb, pt, kind, true, slot, idx, pm, accum, ln, out_q)) {
+                if (wf_begin<NEE, WF_PT_STREAM, RM>(sc, rp, wb, pt, kind, true, slot, idx, pm, accum, ln, out_q)) {
                     q = make_rayq(ln.r);
                     trav_begin(sc, q, t);
 #ifndef RT_PT_BINARY
@@ -1042,8 +1044,10 @@ size_t wavefront_pool(const WavefrontState* ws) { return ws ? ws->b.pool : 0; }
 bool wavefront_render(WavefrontState* ws, const DScene& sc, const DRenderParams& rp, bool use_bvh, float4* accum,
                       unsigned long long* ray_counter, int sm_count, cudaStream_t st, uint32_t* launches,
                       uint32_t* iterations) {
-    // adaptive sampling: the pass covers the div_npix.d pixels of rp.adapt_pixels (the ADAPT instantiations)
+    // adaptive sampling: the pass covers the div_npix.d pixels of rp.adapt_pixels (the ADAPT instantiations); a frame
+    // sequence covers every pixel, rp.spp samples each over all its frames (the FRAMES instantiations)
     const bool adapt = rp.adapt_pixels != nullptr;
+    const int rm = adapt ? RM_ADAPT : (rp.frame_cams ? RM_FRAMES : RM_PLAIN);
     const unsigned long long npix = adapt ? (unsigned long long)rp.div_npix.d : (unsigned long long)rp.width * rp.height;
     const unsigned long long npaths = npix * (unsigned long long)rp.spp;
     *launches = 0;
@@ -1163,60 +1167,62 @@ bool wavefront_render(WavefrontState* ws, const DScene& sc, const DRenderParams&
     };
     auto launch = [&](auto kernel, auto... args) { launch_dims(grid, grain == G_PT ? WF_PT_THREADS : (warp_grain ? WF_THREADS : WF_CTA_THREADS), kernel, args...); };
     uint32_t it = 0;
-    auto step = [&](auto adapt_tag) {
-        constexpr bool AD = decltype(adapt_tag)::value;
+    auto step = [&](auto rm_tag) {
+        constexpr int RM = decltype(rm_tag)::value;
         if (grain == G_PT) {
             if (quant) {
-                if (nee) launch(k_wf_step_pt<true, true, AD>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
-                else launch(k_wf_step_pt<false, true, AD>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
+                if (nee) launch(k_wf_step_pt<true, true, RM>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
+                else launch(k_wf_step_pt<false, true, RM>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
             } else {
-                if (nee) launch(k_wf_step_pt<true, false, AD>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
-                else launch(k_wf_step_pt<false, false, AD>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
+                if (nee) launch(k_wf_step_pt<true, false, RM>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
+                else launch(k_wf_step_pt<false, false, RM>, sc, rp, wb, int(it), accum, ray_counter, refill, leaf_lanes);
             }
         } else if (warp_grain) {
             if (nee) {
-                if (use_bvh) launch(k_wf_step_warp<true, true, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else launch(k_wf_step_warp<false, true, AD>, sc, rp, wb, int(it), accum, ray_counter);
+                if (use_bvh) launch(k_wf_step_warp<true, true, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else launch(k_wf_step_warp<false, true, RM>, sc, rp, wb, int(it), accum, ray_counter);
             } else {
-                if (use_bvh) launch(k_wf_step_warp<true, false, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else launch(k_wf_step_warp<false, false, AD>, sc, rp, wb, int(it), accum, ray_counter);
+                if (use_bvh) launch(k_wf_step_warp<true, false, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else launch(k_wf_step_warp<false, false, RM>, sc, rp, wb, int(it), accum, ray_counter);
             }
         } else {
             if (nee) {
-                if (use_bvh) launch(k_wf_step_cta<true, true, 0, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else if (sc.n_list) launch(k_wf_step_cta<false, true, 1, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else launch(k_wf_step_cta<false, true, 2, AD>, sc, rp, wb, int(it), accum, ray_counter);
+                if (use_bvh) launch(k_wf_step_cta<true, true, 0, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else if (sc.n_list) launch(k_wf_step_cta<false, true, 1, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else launch(k_wf_step_cta<false, true, 2, RM>, sc, rp, wb, int(it), accum, ray_counter);
             } else {
-                if (use_bvh) launch(k_wf_step_cta<true, false, 0, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else if (sc.n_list) launch(k_wf_step_cta<false, false, 1, AD>, sc, rp, wb, int(it), accum, ray_counter);
-                else launch(k_wf_step_cta<false, false, 2, AD>, sc, rp, wb, int(it), accum, ray_counter);
+                if (use_bvh) launch(k_wf_step_cta<true, false, 0, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else if (sc.n_list) launch(k_wf_step_cta<false, false, 1, RM>, sc, rp, wb, int(it), accum, ray_counter);
+                else launch(k_wf_step_cta<false, false, 2, RM>, sc, rp, wb, int(it), accum, ray_counter);
             }
         }
     };
     auto enqueue = [&](uint32_t count) {
         for (uint32_t k = 0; k < count; ++k, ++it) {
-            if (adapt) step(std::true_type{});
-            else step(std::false_type{});
+            if (rm == RM_ADAPT) step(std::integral_constant<int, RM_ADAPT>{});
+            else if (rm == RM_FRAMES) step(std::integral_constant<int, RM_FRAMES>{});
+            else step(std::integral_constant<int, RM_PLAIN>{});
             ++*launches;
         }
     };
-    auto tail = [&](auto adapt_tag) {
-        constexpr bool AD = decltype(adapt_tag)::value;
+    auto tail = [&](auto rm_tag) {
+        constexpr int RM = decltype(rm_tag)::value;
         const unsigned nb = tail_grid, nt = WF_TAIL_THREADS;
         if (nee) {
-            if (use_bvh) launch_dims(nb, nt, k_wf_tail<true, true, 0, AD>, sc, rp, wb, accum, ray_counter);
-            else if (sc.n_list) launch_dims(nb, nt, k_wf_tail<false, true, 1, AD>, sc, rp, wb, accum, ray_counter);
-            else launch_dims(nb, nt, k_wf_tail<false, true, 2, AD>, sc, rp, wb, accum, ray_counter);
+            if (use_bvh) launch_dims(nb, nt, k_wf_tail<true, true, 0, RM>, sc, rp, wb, accum, ray_counter);
+            else if (sc.n_list) launch_dims(nb, nt, k_wf_tail<false, true, 1, RM>, sc, rp, wb, accum, ray_counter);
+            else launch_dims(nb, nt, k_wf_tail<false, true, 2, RM>, sc, rp, wb, accum, ray_counter);
         } else {
-            if (use_bvh) launch_dims(nb, nt, k_wf_tail<true, false, 0, AD>, sc, rp, wb, accum, ray_counter);
-            else if (sc.n_list) launch_dims(nb, nt, k_wf_tail<false, false, 1, AD>, sc, rp, wb, accum, ray_counter);
-            else launch_dims(nb, nt, k_wf_tail<false, false, 2, AD>, sc, rp, wb, accum, ray_counter);
+            if (use_bvh) launch_dims(nb, nt, k_wf_tail<true, false, 0, RM>, sc, rp, wb, accum, ray_counter);
+            else if (sc.n_list) launch_dims(nb, nt, k_wf_tail<false, false, 1, RM>, sc, rp, wb, accum, ray_counter);
+            else launch_dims(nb, nt, k_wf_tail<false, false, 2, RM>, sc, rp, wb, accum, ray_counter);
         }
     };
     auto enqueue_tail = [&]() {
         if (!tail_paths) return;
-        if (adapt) tail(std::true_type{});
-        else tail(std::false_type{});
+        if (rm == RM_ADAPT) tail(std::integral_constant<int, RM_ADAPT>{});
+        else if (rm == RM_FRAMES) tail(std::integral_constant<int, RM_FRAMES>{});
+        else tail(std::integral_constant<int, RM_PLAIN>{});
         ++*launches;
     };
     // Iterations are enqueued in batches.  After each batch the queue sizes and the path counter are copied to
