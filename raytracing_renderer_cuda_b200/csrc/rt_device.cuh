@@ -135,7 +135,9 @@ struct BvhNode4Q {
 
 #define RT_MAX_IMAGES 8
 #define RT_LIST_MAX 12 // scenes of up to this many spheres travel inside the kernel parameters (constant bank), see DScene::lst_*
-#define RT_BVH_STACK_DEPTH 64 // per-thread traversal stack entries (rt_intersect.cuh)
+// Deepest binary tree a scene may have (rt_scene_create rejects deeper ones).  The binary walks push at most one entry per
+// inner ancestor, so this is also their stack size; the 4-wide walks need RT_BVH4_STACK entries (rt_intersect.cuh).
+#define RT_BVH_STACK_DEPTH 64
 
 struct DScene {
     // primitives, static spheres first: [0, n_static) static, [n_static, n) moving

@@ -178,6 +178,11 @@ RT_DEV bool slab_ch(float4 c, float4 h, const V3& inv, const V3& noi, float e, f
 }
 
 #define RT_BVH_STACK RT_BVH_STACK_DEPTH
+// A 4-wide node is a binary node with its inner children replaced by their children, so a path from the root through a
+// tree of binary depth d meets at most ceil(d / 2) 4-wide nodes, and each pushes at most 3 of its 4 children.  A push
+// the stack has no room for would drop a subtree (and possibly the closest hit) without any error.
+#define RT_BVH4_STACK (3 * ((RT_BVH_STACK_DEPTH + 1) / 2))
+static_assert(RT_BVH_STACK_DEPTH != 64 || RT_BVH4_STACK == 96, "depth <= 64: at most 32 4-wide nodes on a path, each pushing at most 3 entries");
 
 // Flattened-BVH closest hit: short per-thread stack, both child boxes fetched with four
 // float4 read-only loads per visited node, near child first, culled by the closest t so far.
@@ -260,9 +265,9 @@ RT_DEV void trav_inner(const DScene& sc, const RayQ& q, float tmin, Trav& t, int
     }
     RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3) RT_CSWAP(1, 2)
 #undef RT_CSWAP
-    if (nhit > 3 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[3];
-    if (nhit > 2 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[2];
-    if (nhit > 1 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[1];
+    if (nhit > 3 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
+    if (nhit > 2 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
+    if (nhit > 1 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
     t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
   } else {
 #ifdef RT_BVH_MINMAX // A/B: the min/max nodes
@@ -388,7 +393,7 @@ RT_DEV void trav_inner_q(const DScene& sc, const RayQ& q, float tmin, Trav& t, i
 #pragma unroll
         for (int s = 3; s >= 0; --s)
             if (key[s] < inf) {
-                if (nxt != RT_TRAV_DONE && t.sp < RT_BVH_STACK) stack[t.sp++] = nxt;
+                if (nxt != RT_TRAV_DONE && t.sp < RT_BVH4_STACK) stack[t.sp++] = nxt;
                 nxt = ref[s];
             }
         t.node = nxt != RT_TRAV_DONE ? nxt : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
@@ -399,9 +404,9 @@ RT_DEV void trav_inner_q(const DScene& sc, const RayQ& q, float tmin, Trav& t, i
 #undef RT_CSWAP
     {
         const float inf = __int_as_float(0x7f800000);
-        if (key[3] < inf && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[3];
-        if (key[2] < inf && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[2];
-        if (key[1] < inf && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[1];
+        if (key[3] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
+        if (key[2] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
+        if (key[1] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
         t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
         return;
     }
@@ -409,9 +414,9 @@ RT_DEV void trav_inner_q(const DScene& sc, const RayQ& q, float tmin, Trav& t, i
     RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3) RT_CSWAP(1, 2)
 #undef RT_CSWAP
 #endif
-    if (nhit > 3 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[3];
-    if (nhit > 2 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[2];
-    if (nhit > 1 && t.sp < RT_BVH_STACK) stack[t.sp++] = ref[1];
+    if (nhit > 3 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
+    if (nhit > 2 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
+    if (nhit > 1 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
     // (requesting the second-nearest child into L1 with prefetch.global.L1 while the nearest is walked: C4 1 487 -> 1 420 Mrays/s,
     // profiles/r02_c4_ab_travq.log — the kernel is short of load slots, not of hits)
     t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
@@ -442,7 +447,7 @@ RT_DEV Hit closest_hit_bvh(const DScene& sc, const RayQ& q, float tmin) {
 // with the reference kernel ray by ray.
 template <bool QUANT = false>
 RT_DEV Hit closest_hit_bvh4(const DScene& sc, const RayQ& q, float tmin) {
-    int stack[RT_BVH_STACK];
+    int stack[RT_BVH4_STACK];
     Trav t;
     trav_begin(sc, q, t);
     t.node = int(sc.root4);

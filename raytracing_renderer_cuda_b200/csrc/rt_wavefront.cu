@@ -848,7 +848,7 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
         }
     };
 
-    int stack[RT_BVH_STACK];
+    int stack[RT_BVH4_STACK];
     Trav t;
     t.node = RT_TRAV_DONE;
     t.leaf = 0;
