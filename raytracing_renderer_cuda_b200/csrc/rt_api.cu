@@ -749,7 +749,6 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     s->d.mats = dmats;
     s->d.texs = dtexs;
     s->d.n_list = 0;
-#ifndef RT_NO_LIST_CONST // (A/B switch: the global-memory list loop)
     if (mode == RT_BVH_NONE && n != 0 && n <= RT_LIST_MAX) { // the list in the constant bank (DScene::lst_*)
         s->d.n_list = n;
         for (uint32_t k = 0; k < n; ++k) {
@@ -758,7 +757,6 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
             memcpy(&s->d.lst_dt[k], &hc[k].x, 4);
         }
     }
-#endif
     s->d.has_noise = 0;
     for (const auto& t : ht)
         if (t.kind == RT_TEX_NOISE_PERLIN || t.kind == RT_TEX_NOISE_TURBULANCE || t.kind == RT_TEX_NOISE_MARBLE || t.kind == RT_TEX_WOOD) s->d.has_noise = 1;

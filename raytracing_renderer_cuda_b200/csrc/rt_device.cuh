@@ -148,7 +148,7 @@ struct DScene {
     uint32_t n_static;
     const BvhNode* nodes; // nullptr => brute force
     const BvhNode4* nodes4; // 4-wide form of the same tree (densely renumbered), nullptr if not built
-    const BvhNodeCH* nodes_ch; // the binary nodes in centre / half-extent form (same numbering): what trav_inner<false> reads
+    const BvhNodeCH* nodes_ch; // the binary nodes in centre / half-extent form (same numbering): what trav_inner reads
     const BvhNode4Q* nodes4q; // ... and its 64-byte quantised form (same numbering), nullptr if not built / not representable
     uint32_t n_nodes4;
     uint32_t root4;

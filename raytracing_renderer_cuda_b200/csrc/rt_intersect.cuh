@@ -120,18 +120,19 @@ RT_DEV Hit closest_hit_list(const DScene& sc, const RayQ& q, float tmin) {
         }
         return best;
     }
-    if (FORM == 1) return best; // (not reached)
-    // two spheres per trip: the second sphere's load is in flight while the first is tested
+    if constexpr (FORM != 1) {
+        // two spheres per trip: the second sphere's load is in flight while the first is tested
 #pragma unroll 2
-    for (uint32_t i = 0; i < sc.n_static; ++i) {
-        float4 a = __ldg(&sc.sph_a[i]);
-        if (sphere_root_static(q, a, tmin, t)) consider(sc, i, t, best);
-    }
-    for (uint32_t i = sc.n_static; i < sc.n_spheres; ++i) {
-        float4 a = __ldg(&sc.sph_a[i]);
-        float4 b = __ldg(&sc.sph_b[i]);
-        float dt = __uint_as_float(__ldg(&sc.sph_c[i]).x);
-        if (sphere_root_moving(q, a, b, dt, tmin, t)) consider(sc, i, t, best);
+        for (uint32_t i = 0; i < sc.n_static; ++i) {
+            float4 a = __ldg(&sc.sph_a[i]);
+            if (sphere_root_static(q, a, tmin, t)) consider(sc, i, t, best);
+        }
+        for (uint32_t i = sc.n_static; i < sc.n_spheres; ++i) {
+            float4 a = __ldg(&sc.sph_a[i]);
+            float4 b = __ldg(&sc.sph_b[i]);
+            float dt = __uint_as_float(__ldg(&sc.sph_c[i]).x);
+            if (sphere_root_moving(q, a, b, dt, tmin, t)) consider(sc, i, t, best);
+        }
     }
     return best;
 }
@@ -149,15 +150,9 @@ RT_DEV Hit closest_hit_list(const DScene& sc, const RayQ& q, float tmin) {
 // leaves are visited (per-lane loop, speculative rounds, refilled lanes: same image), at 0.4 % more box overlap.
 #define RT_SLAB_FAR_WIDEN 1.00390625f
 RT_DEV bool slab(float4 lo, float4 hi, const V3& inv, const V3& noi, float e, float tmin, float tmax, float& tnear) {
-#ifdef RT_SLAB_SUBMUL // A/B: subtract-then-multiply (noi holds -o here)
-    float tx0 = (lo.x + noi.x) * inv.x, tx1 = (hi.x + noi.x) * inv.x;
-    float ty0 = (lo.y + noi.y) * inv.y, ty1 = (hi.y + noi.y) * inv.y;
-    float tz0 = (lo.z + noi.z) * inv.z, tz1 = (hi.z + noi.z) * inv.z;
-#else
     float tx0 = __fmaf_rn(lo.x, inv.x, noi.x), tx1 = __fmaf_rn(hi.x, inv.x, noi.x);
     float ty0 = __fmaf_rn(lo.y, inv.y, noi.y), ty1 = __fmaf_rn(hi.y, inv.y, noi.y);
     float tz0 = __fmaf_rn(lo.z, inv.z, noi.z), tz1 = __fmaf_rn(hi.z, inv.z, noi.z);
-#endif
     float tn = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), tmin));
     float tf = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), tmax));
     tnear = tn;
@@ -224,18 +219,52 @@ RT_DEV void trav_begin(const DScene& sc, const RayQ& q, Trav& t) {
     t.inv = V3{iv[0], iv[1], iv[2]};
     t.noi = V3{no[0], no[1], no[2]};
     t.e = m * 2.3841858e-7f; // 2^-22
-#ifdef RT_SLAB_SUBMUL
-    t.inv = V3{1.0f / q.d.x, 1.0f / q.d.y, 1.0f / q.d.z};
-    t.noi = V3{-q.o.x, -q.o.y, -q.o.z};
-    t.e = 0.f;
-#endif
 }
-// one inner-node visit (precondition: t.node >= 0 && t.node != RT_TRAV_DONE)
-template <bool WIDE = false>
+// One visit of a binary node (BvhNodeCH; precondition: t.node >= 0 && t.node != RT_TRAV_DONE).
+// (lmin / lmax / rmin / rmax: centre and half-extent of the left, then of the right child)
 RT_DEV void trav_inner(const DScene& sc, const RayQ& q, float tmin, Trav& t, int* stack) {
-  if (WIDE) {
-    // 4-wide node (BvhNode4): seven vector loads, four slab tests in SoA form, the hit children ordered by entry
-    // distance with a 5-comparator network; the nearest is walked next, the others are pushed farthest first.
+    const float4* np = reinterpret_cast<const float4*>(sc.nodes_ch + t.node);
+    float4 lmin = __ldg(np + 0), lmax = __ldg(np + 1), rmin = __ldg(np + 2), rmax = __ldg(np + 3);
+    float tl, tr;
+    const bool hl = slab_ch(lmin, lmax, t.inv, t.noi, t.e, tmin, t.best.t, tl);
+    const bool hr = slab_ch(rmin, rmax, t.inv, t.noi, t.e, tmin, t.best.t, tr);
+    const int cl = __float_as_int(lmin.w), cr = __float_as_int(lmax.w);
+    if (hl && hr) {
+        const bool left_first = tl <= tr;
+        if (t.sp < RT_BVH_STACK) stack[t.sp++] = left_first ? cr : cl;
+        t.node = left_first ? cl : cr;
+    } else if (hl) {
+        t.node = cl;
+    } else if (hr) {
+        t.node = cr;
+    } else {
+        t.node = t.sp ? stack[--t.sp] : RT_TRAV_DONE;
+    }
+}
+// The end of every 4-wide node visit: the `nhit` hit children (key = entry distance, +inf for a miss) ordered with a
+// 5-comparator network; the nearest is walked next, the others are pushed farthest first.
+RT_DEV void trav_next4(Trav& t, int* stack, float (&key)[4], int (&ref)[4], int nhit) {
+#define RT_CSWAP(a, b)                       \
+    {                                        \
+        const bool sw = key[b] < key[a];     \
+        const float ka = key[a], kb = key[b]; \
+        const int ra = ref[a], rb = ref[b];  \
+        key[a] = sw ? kb : ka;               \
+        key[b] = sw ? ka : kb;               \
+        ref[a] = sw ? rb : ra;               \
+        ref[b] = sw ? ra : rb;               \
+    }
+    RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3) RT_CSWAP(1, 2)
+#undef RT_CSWAP
+    if (nhit > 3 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
+    if (nhit > 2 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
+    if (nhit > 1 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
+    // (requesting the second-nearest child into L1 with prefetch.global.L1 while the nearest is walked: C4 1 487 -> 1 420 Mrays/s,
+    // profiles/r02_c4_ab_travq.log — the kernel is short of load slots, not of hits)
+    t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
+}
+// One visit of a 128-byte 4-wide node (BvhNode4): seven vector loads, four slab tests in SoA form, then trav_next4.
+RT_DEV void trav_inner4(const DScene& sc, const RayQ& q, float tmin, Trav& t, int* stack) {
     const float4* np = reinterpret_cast<const float4*>(sc.nodes4 + t.node);
     const float4 mnx = __ldg(np + 0), mny = __ldg(np + 1), mnz = __ldg(np + 2);
     const float4 mxx = __ldg(np + 3), mxy = __ldg(np + 4), mxz = __ldg(np + 5);
@@ -253,59 +282,13 @@ RT_DEV void trav_inner(const DScene& sc, const RayQ& q, float tmin, Trav& t, int
         key[s] = hit ? tn : __int_as_float(0x7f800000); // +inf: misses sort to the end
         nhit += hit ? 1 : 0;
     }
-#define RT_CSWAP(a, b)                       \
-    {                                        \
-        const bool sw = key[b] < key[a];     \
-        const float ka = key[a], kb = key[b]; \
-        const int ra = ref[a], rb = ref[b];  \
-        key[a] = sw ? kb : ka;               \
-        key[b] = sw ? ka : kb;               \
-        ref[a] = sw ? rb : ra;               \
-        ref[b] = sw ? ra : rb;               \
-    }
-    RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3) RT_CSWAP(1, 2)
-#undef RT_CSWAP
-    if (nhit > 3 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
-    if (nhit > 2 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
-    if (nhit > 1 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
-    t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
-  } else {
-#ifdef RT_BVH_MINMAX // A/B: the min/max nodes
-    const float4* np = reinterpret_cast<const float4*>(sc.nodes + t.node);
-    float4 lmin = __ldg(np + 0), lmax = __ldg(np + 1), rmin = __ldg(np + 2), rmax = __ldg(np + 3);
-    float tl, tr;
-    const bool hl = slab(lmin, lmax, t.inv, t.noi, t.e, tmin, t.best.t, tl);
-    const bool hr = slab(rmin, rmax, t.inv, t.noi, t.e, tmin, t.best.t, tr);
-#else // (lmin / lmax / rmin / rmax: centre and half-extent of the left, then of the right child)
-    const float4* np = reinterpret_cast<const float4*>(sc.nodes_ch + t.node);
-    float4 lmin = __ldg(np + 0), lmax = __ldg(np + 1), rmin = __ldg(np + 2), rmax = __ldg(np + 3);
-    float tl, tr;
-    const bool hl = slab_ch(lmin, lmax, t.inv, t.noi, t.e, tmin, t.best.t, tl);
-    const bool hr = slab_ch(rmin, rmax, t.inv, t.noi, t.e, tmin, t.best.t, tr);
-#endif
-    const int cl = __float_as_int(lmin.w), cr = __float_as_int(lmax.w);
-    if (hl && hr) {
-        const bool left_first = tl <= tr;
-        if (t.sp < RT_BVH_STACK) stack[t.sp++] = left_first ? cr : cl;
-        t.node = left_first ? cl : cr;
-    } else if (hl) {
-        t.node = cl;
-    } else if (hr) {
-        t.node = cr;
-    } else {
-        t.node = t.sp ? stack[--t.sp] : RT_TRAV_DONE;
-    }
-  }
+    trav_next4(t, stack, key, ref, nhit);
 }
 // One visit of a QUANTISED 4-wide node (BvhNode4Q): four 16-byte loads instead of seven.  The ray is moved into the
 // node's grid once per axis — s = unit * (1/d), o = p * (1/d) - origin * (1/d), the same FFMA form as slab() — and every
 // bound is then ONE FFMA on a byte: t = q * s + o.  The decoded boxes contain the float boxes with a whole unit to
 // spare (k_quantize4), so the test can only add visits; acceptance test, far-bound margin, ordering network and stack
 // discipline are those of the 128-byte form.
-#ifdef RT_TRAVQ_I2F // A/B: the first form — bytes converted with I2F.U8 (XU pipe), both bounds of every axis computed and ordered
-RT_DEV float byte_f(uint32_t w, int k) { return float((w >> (8 * k)) & 255u); }
-#else
-// byte K of `w` as the float 1 + byte * 2^-15: ONE byte permute (ALU pipe) drops it into the mantissa of 1.0f
 // three-input minimum / maximum (FMNMX3, sm_100)
 RT_DEV float fmax3(float a, float b, float c) {
     float d;
@@ -317,40 +300,22 @@ RT_DEV float fmin3(float a, float b, float c) {
     asm("min.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
     return d;
 }
+// byte K of `w` as the float 1 + byte * 2^-15: ONE byte permute (ALU pipe) drops it into the mantissa of 1.0f
 template <int K>
 RT_DEV float byte_m(uint32_t w) { return __uint_as_float(__byte_perm(w, 0x3F800000u, 0x7604u | (uint32_t(K) << 4))); }
-#endif
 RT_DEV void trav_inner_q(const DScene& sc, const RayQ& q, float tmin, Trav& t, int* stack) {
     const uint4* np = reinterpret_cast<const uint4*>(sc.nodes4q + t.node);
     const uint4 q0 = __ldg(np + 0), q1 = __ldg(np + 1), q2 = __ldg(np + 2), q3 = __ldg(np + 3);
-#ifdef RT_TRAVQ_I2F
-    const float sx = __uint_as_float((q0.w & 0xffu) << 23) * t.inv.x;
-    const float sy = __uint_as_float((q0.w & 0xff00u) << 15) * t.inv.y;
-    const float sz = __uint_as_float((q0.w & 0xff0000u) << 7) * t.inv.z;
-#else // 2^15 units per axis (the exponent bytes are at most 20 + 127)
+    // 2^15 units per axis (the exponent bytes are at most 20 + 127)
     const float Sx = __uint_as_float(((q0.w & 0xffu) << 23) + (15u << 23)) * t.inv.x;
     const float Sy = __uint_as_float(((q0.w & 0xff00u) << 15) + (15u << 23)) * t.inv.y;
     const float Sz = __uint_as_float(((q0.w & 0xff0000u) << 7) + (15u << 23)) * t.inv.z;
-#endif
     const float ox = __fmaf_rn(__uint_as_float(q0.x), t.inv.x, t.noi.x);
     const float oy = __fmaf_rn(__uint_as_float(q0.y), t.inv.y, t.noi.y);
     const float oz = __fmaf_rn(__uint_as_float(q0.z), t.inv.z, t.noi.z);
     float key[4];
     int ref[4] = {int(q1.x), int(q1.y), int(q1.z), int(q1.w)};
     int nhit = 0;
-#ifdef RT_TRAVQ_I2F
-#pragma unroll
-    for (int s = 0; s < 4; ++s) {
-        const float tx0 = __fmaf_rn(byte_f(q2.x, s), sx, ox), tx1 = __fmaf_rn(byte_f(q2.w, s), sx, ox);
-        const float ty0 = __fmaf_rn(byte_f(q2.y, s), sy, oy), ty1 = __fmaf_rn(byte_f(q3.x, s), sy, oy);
-        const float tz0 = __fmaf_rn(byte_f(q2.z, s), sz, oz), tz1 = __fmaf_rn(byte_f(q3.y, s), sz, oz);
-        const float tn = fmaxf(fmaxf(fminf(tx0, tx1), fminf(ty0, ty1)), fmaxf(fminf(tz0, tz1), tmin));
-        const float tf = fminf(fminf(fmaxf(tx0, tx1), fmaxf(ty0, ty1)), fminf(fmaxf(tz0, tz1), t.best.t));
-        const bool hit = tn <= __fmaf_rn(tf, RT_SLAB_FAR_WIDEN, t.e) && ref[s] != RT_BVH4_EMPTY;
-        key[s] = hit ? tn : __int_as_float(0x7f800000); // +inf: misses sort to the end
-        nhit += hit ? 1 : 0;
-    }
-#else
     // The sign of 1/d says which face of a box the ray enters through, for all four children at once: the word of entry
     // bytes and the word of exit bytes are selected per axis (6 selects per node) instead of ordering two bounds per axis
     // and child (24 min/max).  With the byte in the mantissa — 1 + b * 2^-15 — the bound is t = f * S + O with
@@ -374,52 +339,7 @@ RT_DEV void trav_inner_q(const DScene& sc, const RayQ& q, float tmin, Trav& t, i
     }
     RT_CHILD(0) RT_CHILD(1) RT_CHILD(2) RT_CHILD(3)
 #undef RT_CHILD
-#endif
-#define RT_CSWAP(a, b)                       \
-    {                                        \
-        const bool sw = key[b] < key[a];     \
-        const float ka = key[a], kb = key[b]; \
-        const int ra = ref[a], rb = ref[b];  \
-        key[a] = sw ? kb : ka;               \
-        key[b] = sw ? ka : kb;               \
-        ref[a] = sw ? rb : ra;               \
-        ref[b] = sw ? ra : rb;               \
-    }
-#if defined(RT_TRAVQ_NOSORT) // A/B: no ordering at all — hit children in slot order
-#undef RT_CSWAP
-    {
-        const float inf = __int_as_float(0x7f800000);
-        int nxt = RT_TRAV_DONE;
-#pragma unroll
-        for (int s = 3; s >= 0; --s)
-            if (key[s] < inf) {
-                if (nxt != RT_TRAV_DONE && t.sp < RT_BVH4_STACK) stack[t.sp++] = nxt;
-                nxt = ref[s];
-            }
-        t.node = nxt != RT_TRAV_DONE ? nxt : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
-        return;
-    }
-#elif defined(RT_TRAVQ_NEAR1) // A/B: the nearest child first, the others in any order
-    RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3)
-#undef RT_CSWAP
-    {
-        const float inf = __int_as_float(0x7f800000);
-        if (key[3] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
-        if (key[2] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
-        if (key[1] < inf && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
-        t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
-        return;
-    }
-#else
-    RT_CSWAP(0, 1) RT_CSWAP(2, 3) RT_CSWAP(0, 2) RT_CSWAP(1, 3) RT_CSWAP(1, 2)
-#undef RT_CSWAP
-#endif
-    if (nhit > 3 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[3];
-    if (nhit > 2 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[2];
-    if (nhit > 1 && t.sp < RT_BVH4_STACK) stack[t.sp++] = ref[1];
-    // (requesting the second-nearest child into L1 with prefetch.global.L1 while the nearest is walked: C4 1 487 -> 1 420 Mrays/s,
-    // profiles/r02_c4_ab_travq.log — the kernel is short of load slots, not of hits)
-    t.node = nhit ? ref[0] : (t.sp ? stack[--t.sp] : RT_TRAV_DONE);
+    trav_next4(t, stack, key, ref, nhit);
 }
 // one leaf test (precondition: t.node < 0)
 RT_DEV void trav_leaf(const DScene& sc, const RayQ& q, float tmin, Trav& t, int* stack) {
@@ -454,7 +374,7 @@ RT_DEV Hit closest_hit_bvh4(const DScene& sc, const RayQ& q, float tmin) {
     while (true) {
         while (t.node >= 0 && t.node != RT_TRAV_DONE) {
             if (QUANT) trav_inner_q(sc, q, tmin, t, stack);
-            else trav_inner<true>(sc, q, tmin, t, stack);
+            else trav_inner4(sc, q, tmin, t, stack);
         }
         if (t.node == RT_TRAV_DONE) break;
         trav_leaf(sc, q, tmin, t, stack);
@@ -498,14 +418,7 @@ RT_DEV Hit closest_hit_bvh_warp(const DScene& sc, const RayQ& q, float tmin, boo
     Trav t;
     trav_begin(sc, q, t);
     if (!has_ray) t.node = RT_TRAV_DONE;
-#ifdef RT_WARP_IFIF // A/B: one step per lane and iteration (inner node, then the leaf it may have reached), no postponing
-    while (__any_sync(0xffffffffu, t.node != RT_TRAV_DONE)) {
-        if (t.node >= 0 && t.node != RT_TRAV_DONE) trav_inner(sc, q, tmin, t, stack);
-        if (t.node < 0) trav_leaf(sc, q, tmin, t, stack);
-    }
-#else
     while (__any_sync(0xffffffffu, t.node != RT_TRAV_DONE)) trav_round_warp(sc, q, tmin, t, stack);
-#endif
     return t.best;
 }
 

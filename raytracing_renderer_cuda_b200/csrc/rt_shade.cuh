@@ -24,13 +24,6 @@ namespace rtd {
 //    perlin_noise.h:173-181).  A gradient is then R2P + 5 FSEL + FADD = 7 instructions instead of 13-14.
 //  * per octave: 10 LDS + 7 address adds instead of 7 LDS + 33 shifts/masks/adds; 124 instead of 194 instructions.
 // The arithmetic (operands, order, roundings) is unchanged: every value is bit-identical to the round-1 code.
-#ifndef RT_PERLIN_INLINE
-#define RT_PERLIN_FN static __device__ __noinline__
-#define RT_PERLIN_UNROLL _Pragma("unroll 1")
-#else
-#define RT_PERLIN_FN RT_DEV
-#define RT_PERLIN_UNROLL _Pragma("unroll")
-#endif
 // Ken Perlin's 2002 permutation (perlin_noise.h:24-37).  p[512] of the reference is
 // this table twice (perlin_noise.h:43), so p[i] == perm[i & 255] for every index used.
 __device__ const uint8_t k_perlin_perm[256] = {
@@ -111,15 +104,15 @@ RT_DEV float perlin_noise_body(const char* base, V3 p) {
                     perlin_lerp(u, perlin_grad<3>(gab, xf, y1, z1), perlin_grad<3>(gbb, x1, y1, z1))));
     return (res + 1.0f) / 2.0f;
 }
-RT_PERLIN_FN float perlin_noise(const PerlinTab& pt, V3 p) { return perlin_noise_body(perlin_base(pt), p); }
+static __device__ __noinline__ float perlin_noise(const PerlinTab& pt, V3 p) { return perlin_noise_body(perlin_base(pt), p); }
 
 // perlin_noise::turbulance_noise, implementation 3 (perlin_noise.h:142-153), defaults
 // lacunacity 2, gain .5, 6 octaves (perlin_noise.h:13-17).  ONE out-of-line call per 6-octave evaluation with the
 // noise body inlined in its loop.
-RT_PERLIN_FN float perlin_turbulence(const PerlinTab& pt, V3 p) {
+static __device__ __noinline__ float perlin_turbulence(const PerlinTab& pt, V3 p) {
     const char* base = perlin_base(pt);
     float frequency = 1.f, sum = 0.f, amplitude = 1.f;
-    RT_PERLIN_UNROLL
+#pragma unroll 1
     for (int i = 0; i < 6; ++i) {
         float r = perlin_noise_body(base, p * frequency);
         sum += fabsf(r * 2.f - 1.f) * amplitude;

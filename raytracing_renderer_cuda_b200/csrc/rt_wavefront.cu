@@ -40,14 +40,10 @@ enum : int { Q_NEW = 0, Q_LAMB_CONST, Q_LAMB_NOISE1, Q_LAMB_NOISE6, Q_LAMB_IMAGE
 #endif
 // Programmatic dependent launch: iteration i+1 is launched while iteration i drains, so its CTAs are resident and
 // waiting (griddepcontrol.wait returns once the previous grid has completed and its writes are visible) instead
-// of paying the launch latency between two of the ~70 dependent launches of a frame.  WF_NO_PDL disables it.
-#ifndef WF_NO_PDL
+// of paying the launch latency between two of the ~70 dependent launches of a frame.
 #define WF_PDL_PROLOGUE()                                      \
     asm volatile("griddepcontrol.launch_dependents;");          \
     asm volatile("griddepcontrol.wait;" ::: "memory")
-#else
-#define WF_PDL_PROLOGUE()
-#endif
 #ifndef WF_CTA_THREADS
 // CTA size of the CTA-chunk kernel (= its chunk size).  128 threads x 8 CTAs per SM instead of 256 x 4: the two block
 // barriers of a chunk span 4 warps instead of 8 (C1 -1.1 % at equal table size (round-1 A/B, log not kept); 64 x 16: +2 %)
@@ -115,37 +111,26 @@ struct WavefrontState {
 // Streaming accesses to data that is read once and written once per iteration (path records, queue entries): L1
 // evict-first loads and stores (ld/st.global.cs), so they do not displace the stack frames and the sphere data
 // (C1 -1.5 %, C2 -1.9 % on the probes, C2 bench -11 % (round-1 A/Bs, logs not kept); L2-only .cg accesses were
-// 3.7 % SLOWER than .cs on C1 in round 1).  Used by the CTA-chunk and warp-chunk kernels.  The persistent-lane
-// kernel keeps plain accesses: with streaming ones its million-sphere frame differed from the megakernel's in 0.04 %
-// of the rays, identically for .cs and .cg (so not a matter of cache coherence; the kernel sits at its register
-// limit and has shown such a codegen-dependent difference once before, DESIGN.md section 3) — unexplained, so not shipped.
-// MODE: 0 plain, 1 streaming (.cs), 2 L2-only (.cg) — the ring kernel below re-reads records other SMs wrote during the
-// SAME launch, so nothing it touches may be served from a stale L1 line.
-enum : int { WF_ACC_PLAIN = 0, WF_ACC_STREAM = 1, WF_ACC_L2 = 2 };
+// 3.7 % SLOWER than .cs on C1 in round 1).  Used by the CTA-chunk and warp-chunk kernels.
+// The persistent-lane kernel uses plain accesses because they keep its image right: with streaming ones its
+// million-sphere frame differed from the megakernel's in 0.04 % of the rays, identically for .cs and .cg (so not a
+// matter of cache coherence; the kernel sits at its register limit and has shown such a codegen-dependent difference
+// once before, DESIGN.md section 3).  The cause is not known, so that kernel keeps the accesses it was verified with.
+// k_wf_tail uses plain accesses as well.
+enum : int { WF_ACC_PLAIN = 0, WF_ACC_STREAM = 1 };
 template <int MODE, typename T>
 RT_DEV T wf_ld(const T* p) {
-    return MODE == WF_ACC_L2 ? __ldcg(p) : (MODE == WF_ACC_STREAM ? __ldcs(p) : *p);
+    return MODE == WF_ACC_STREAM ? __ldcs(p) : *p;
 }
 template <int MODE, typename T>
 RT_DEV void wf_st(T* p, T v) {
-    if (MODE == WF_ACC_L2) __stcg(p, v);
-    else if (MODE == WF_ACC_STREAM) __stcs(p, v);
+    if (MODE == WF_ACC_STREAM) __stcs(p, v);
     else *p = v;
 }
 template <int MODE>
 RT_DEV uint32_t wf_qload(const uint32_t* p) {
-    return MODE == WF_ACC_L2 ? __ldcg(p) : (MODE == WF_ACC_STREAM ? __ldcs(p) : __ldg(p));
+    return MODE == WF_ACC_STREAM ? __ldcs(p) : __ldg(p);
 }
-#ifdef WF_PT_STREAM_ON // debugging aid: streaming accesses in the persistent-lane kernel too (see above)
-#define WF_PT_STREAM WF_ACC_STREAM
-#else
-#define WF_PT_STREAM WF_ACC_PLAIN
-#endif
-#ifdef WF_NO_STREAM // A/B: plain accesses everywhere
-#define WF_STREAM WF_ACC_PLAIN
-#else
-#define WF_STREAM WF_ACC_STREAM
-#endif
 RT_DEV uint32_t* wf_queue(const WfBuffers& b, int parity, int q) { return b.queue + (size_t(parity) * NQ + size_t(q)) * b.pool; }
 
 // Shading class of a hit: material kind x cost class of its (checker-resolved) leaf texture.
@@ -347,7 +332,7 @@ RT_DEV int wf_finish(const DScene& sc, const DRenderParams& rp, const WfBuffers&
 
 // One whole queue entry (the CTA-chunk and warp-chunk kernels): begin, closest hit, finish.  Called by all 32 lanes of
 // the warp (the BVH traversal is warp-cooperative); `valid` = false for lanes past the end of the queue.
-template <bool USE_BVH, bool NEE, int ACC = WF_STREAM, int LIST = 0, int RM = RM_PLAIN>
+template <bool USE_BVH, bool NEE, int ACC = WF_ACC_STREAM, int LIST = 0, int RM = RM_PLAIN>
 RT_DEV int wf_process_entry(const DScene& sc, const DRenderParams& rp, const WfBuffers& wb, const PerlinTab& pt, int kind,
                             bool valid, uint32_t slot, uint32_t idx, const PathMap& pm, float4* __restrict__ accum,
                             unsigned long long& nrays) {
@@ -357,12 +342,7 @@ RT_DEV int wf_process_entry(const DScene& sc, const DRenderParams& rp, const WfB
     if (NEE) nrays += ln.shadow_rays;
     if (USE_BVH) {
         const RayQ q = make_rayq(ln.r);
-#ifdef WF_NO_SPEC // A/B: the per-lane loop
-        Hit h{FLT_MAX, RT_INVALID_ID};
-        if (has_ray) h = closest_hit_bvh(sc, q, rp.tmin);
-#else
         const Hit h = closest_hit_bvh_warp(sc, q, rp.tmin, has_ray);
-#endif
         if (has_ray) {
             ++nrays;
             out_q = wf_finish<NEE, ACC, RM>(sc, rp, wb, accum, ln, q, h);
@@ -479,14 +459,14 @@ __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
     // the two barriers of the trip publish the record.
     uint32_t* ticket = wb.tickets + (it % 3);
     Chunk ck = s_chunk[0];
-    uint32_t slot = (ck.first + threadIdx.x < ck.n_kind) ? wf_qload<WF_STREAM>(ck.q_in + ck.first + threadIdx.x) : 0u;
+    uint32_t slot = (ck.first + threadIdx.x < ck.n_kind) ? wf_qload<WF_ACC_STREAM>(ck.q_in + ck.first + threadIdx.x) : 0u;
     while (ck.kind >= 0) {
         uint32_t drawn = 0u;
         if (threadIdx.x == 0) drawn = atomicAdd(ticket, 1u);
         const uint32_t idx = ck.first + threadIdx.x;
         const bool valid = idx < ck.n_kind;
 
-        const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, LIST, RM>(sc, rp, wb, pt, ck.kind, valid, slot, idx, pm, accum, nrays);
+        const int out_q = wf_process_entry<USE_BVH, NEE, WF_ACC_STREAM, LIST, RM>(sc, rp, wb, pt, ck.kind, valid, slot, idx, pm, accum, nrays);
 
         // ---- queue push: warp ballot -> shared counters -> one global atomic per queue ----
         uint32_t local = 0;
@@ -508,12 +488,12 @@ __global__ void __launch_bounds__(WF_CTA_THREADS, WF_CTA_MINBLOCKS)
             s_count[cpar ^ 1u][threadIdx.x] = 0u; // the other buffer was last read before the barrier above
         }
         __syncthreads();
-        if (out_q != Q_NONE) wf_st<WF_STREAM>(wf_queue(wb, par_next, out_q) + s_base[cpar][out_q] + local, slot);
+        if (out_q != Q_NONE) wf_st<WF_ACC_STREAM>(wf_queue(wb, par_next, out_q) + s_base[cpar][out_q] + local, slot);
         cpar ^= 1u;
         // (requesting the next chunk's slot indices a chunk ahead, and prefetching their records, was measured in
         // round 1: 2.6 % and 1.2 % slower with 16 Mi slots)
         ck = s_chunk[cpar]; // written before the two barriers of this trip; rewritten after the first barrier of the next
-        if (ck.kind >= 0) slot = ck.first + threadIdx.x < ck.n_kind ? wf_qload<WF_STREAM>(ck.q_in + ck.first + threadIdx.x) : 0u;
+        if (ck.kind >= 0) slot = ck.first + threadIdx.x < ck.n_kind ? wf_qload<WF_ACC_STREAM>(ck.q_in + ck.first + threadIdx.x) : 0u;
     }
 
     for (int off = 16; off > 0; off >>= 1) nrays += __shfl_down_sync(0xffffffffu, nrays, off);
@@ -631,6 +611,8 @@ __global__ void __launch_bounds__(WF_TAIL_THREADS, WF_TAIL_MINBLOCKS)
 // ticket counter and pushes its results with one global atomic per target queue.  No block-wide barrier inside the
 // loop: a warp whose rays finish early moves on instead of waiting for the slowest BVH traversal of the CTA
 // (ncu, C2: 21 % of all stall samples sat on that barrier; C2 runs 14 % faster this way, C3 4 %).
+// (The shipped build runs one round.  The rounds loop below stays anyway: written without it, nvcc 12.9 sign-extends
+// the target queue of the push instead of zero-extending it, and the kernel's SASS changes.)
 #ifndef WF_ROUNDS
 #define WF_ROUNDS 1
 #endif
@@ -736,8 +718,8 @@ __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
         for (int e = 0; e < WF_ROUNDS; ++e) {
             const uint32_t idx = first + uint32_t(e) * 32u + lane;
             const bool valid = idx < n_kind;
-            const uint32_t slot = valid ? wf_qload<WF_STREAM>(q_in + idx) : 0u;
-            const int out_q = wf_process_entry<USE_BVH, NEE, WF_STREAM, 0, RM>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, nrays);
+            const uint32_t slot = valid ? wf_qload<WF_ACC_STREAM>(q_in + idx) : 0u;
+            const int out_q = wf_process_entry<USE_BVH, NEE, WF_ACC_STREAM, 0, RM>(sc, rp, wb, pt, kind, valid, slot, idx, pm, accum, nrays);
                 outq_pack |= uint32_t(out_q + 1) << (4 * e);
         }
 
@@ -766,8 +748,8 @@ __global__ void __launch_bounds__(WF_THREADS, WF_MINBLOCKS)
             const uint32_t oq1 = (outq_pack >> (4 * e)) & 15u; // queue + 1
             const uint32_t base = __shfl_sync(0xffffffffu, my_base, int(oq1 + 31u) & 31);
             if (oq1) { // the slot index is re-read from the input queue (an L1 hit) instead of living in a register
-                const uint32_t slot = wf_qload<WF_STREAM>(q_in + first + uint32_t(e) * 32u + lane);
-                wf_st<WF_STREAM>(wf_queue(wb, par_next, int(oq1) - 1) + base + rank_r[e], slot);
+                const uint32_t slot = wf_qload<WF_ACC_STREAM>(q_in + first + uint32_t(e) * 32u + lane);
+                wf_st<WF_ACC_STREAM>(wf_queue(wb, par_next, int(oq1) - 1) + base + rank_r[e], slot);
             }
         }
     }
@@ -844,7 +826,7 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
             uint32_t base = 0u;
             if (int(lane) == leader) base = atomicAdd(cnt_next + out_q, uint32_t(__popc(peers)));
             base = __shfl_sync(peers, base, leader);
-            wf_st<WF_PT_STREAM>(wf_queue(wb, par_next, out_q) + base + uint32_t(__popc(peers & lt_mask)), slot);
+            wf_st<WF_ACC_PLAIN>(wf_queue(wb, par_next, out_q) + base + uint32_t(__popc(peers & lt_mask)), slot);
         }
     };
 
@@ -874,9 +856,9 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
         // ---- 1. second half of the entries whose ray is done ----
         {
             int out_q = Q_NONE;
-            if (tracing && t.node == RT_TRAV_DONE && t.leaf >= 0) { // (t.leaf < 0: a postponed leaf, -DRT_PT_POSTPONE only)
+            if (tracing && t.node == RT_TRAV_DONE) {
                 ++nrays;
-                out_q = wf_finish<NEE, WF_PT_STREAM, RM>(sc, rp, wb, accum, ln, q, t.best);
+                out_q = wf_finish<NEE, WF_ACC_PLAIN, RM>(sc, rp, wb, accum, ln, q, t.best);
                 tracing = false;
             }
             push(out_q, ln.slot);
@@ -904,13 +886,11 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
             int out_q = Q_NONE;
             if (!tracing && rank < navail) {
                 const uint32_t idx = pos + rank;
-                const uint32_t slot = wf_qload<WF_PT_STREAM>(q_in + idx);
-                if (wf_begin<NEE, WF_PT_STREAM, RM>(sc, rp, wb, pt, kind, true, slot, idx, pm, accum, ln, out_q)) {
+                const uint32_t slot = wf_qload<WF_ACC_PLAIN>(q_in + idx);
+                if (wf_begin<NEE, WF_ACC_PLAIN, RM>(sc, rp, wb, pt, kind, true, slot, idx, pm, accum, ln, out_q)) {
                     q = make_rayq(ln.r);
                     trav_begin(sc, q, t);
-#ifndef RT_PT_BINARY
                     t.node = int(sc.root4); // this kernel walks the 4-wide nodes
-#endif
                     tracing = true;
                 }
                 if (NEE) nrays += ln.shadow_rays;
@@ -925,48 +905,18 @@ __global__ void __launch_bounds__(WF_PT_THREADS, WF_PT_MINBLOCKS)
         const int keep = more ? max(__popc(live) - refill, 0) : 0;
         int nlive;
         do {
-#ifdef RT_PT_POSTPONE // A/B: a lane that reaches a leaf postpones it and keeps walking (as the warp-chunk kernel does); the postponed
-                      // leaves are tested when RT_PT_POSTPONE lanes hold one, when a lane stands at a second leaf, or when nobody can walk
-            if (t.node >= 0 && t.node != RT_TRAV_DONE) {
-                if (QUANT) trav_inner_q(sc, q, rp.tmin, t, stack);
-                else trav_inner<true>(sc, q, rp.tmin, t, stack);
-                if (t.node < 0 && t.leaf >= 0) {
-                    t.leaf = t.node;
-                    t.node = t.sp ? stack[--t.sp] : RT_TRAV_DONE;
-                }
-            }
-            const unsigned pend = __ballot_sync(0xffffffffu, t.leaf < 0);
-            const unsigned blocked = __ballot_sync(0xffffffffu, t.node < 0);
-            const unsigned can_go = __ballot_sync(0xffffffffu, t.node >= 0 && t.node != RT_TRAV_DONE);
-            if (__popc(pend) >= RT_PT_POSTPONE || blocked != 0u || can_go == 0u) {
-                if (t.leaf < 0) {
-                    test_prim(sc, q, uint32_t(~t.leaf), rp.tmin, t.best);
-                    t.leaf = 0;
-                }
-                if (t.node < 0) { // the node after the postponed leaf is a leaf too: it waits in its place
-                    t.leaf = t.node;
-                    t.node = t.sp ? stack[--t.sp] : RT_TRAV_DONE;
-                }
-            }
-            nlive = __popc(__ballot_sync(0xffffffffu, t.node != RT_TRAV_DONE || t.leaf < 0));
-#else
             // One inner-node step for every lane that stands at an inner node; lanes that stand at a leaf (or just
             // arrived at one) test it once `leaf_lanes` of them wait, or when no lane can take an inner step.
-#ifdef RT_PT_BINARY // A/B: the binary tree
-            if (t.node >= 0 && t.node != RT_TRAV_DONE) trav_inner<false>(sc, q, rp.tmin, t, stack);
-#else
             if (t.node >= 0 && t.node != RT_TRAV_DONE) { // 4-wide nodes, 64-byte (quantised) or 128-byte form
                 if (QUANT) trav_inner_q(sc, q, rp.tmin, t, stack);
-                else trav_inner<true>(sc, q, rp.tmin, t, stack);
+                else trav_inner4(sc, q, rp.tmin, t, stack);
             }
-#endif
             const unsigned at_leaf = __ballot_sync(0xffffffffu, t.node < 0);
             const unsigned can_go = __ballot_sync(0xffffffffu, t.node >= 0 && t.node != RT_TRAV_DONE);
             if (__popc(at_leaf) >= leaf_lanes || can_go == 0u) {
                 if (t.node < 0) trav_leaf(sc, q, rp.tmin, t, stack);
             }
             nlive = __popc(__ballot_sync(0xffffffffu, t.node != RT_TRAV_DONE));
-#endif
         } while (nlive > keep);
     }
 
@@ -1156,11 +1106,7 @@ bool wavefront_render(WavefrontState* ws, const DScene& sc, const DRenderParams&
         cfg.stream = st;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-#ifndef WF_NO_PDL
         attr[0].val.programmaticStreamSerializationAllowed = 1;
-#else
-        attr[0].val.programmaticStreamSerializationAllowed = 0;
-#endif
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         cudaLaunchKernelEx(&cfg, kernel, args...);
