@@ -9,7 +9,7 @@ CSRC      := $(PKG)/csrc
 OBJDIR    := build
 LIB       := $(PKG)/librt_b200.so
 
-CU_SRCS   := $(CSRC)/rt_api.cu $(CSRC)/rt_kernels.cu $(CSRC)/rt_wavefront.cu $(CSRC)/rt_lbvh.cu $(CSRC)/rt_jpeg.cu $(CSRC)/rt_jpeg_decode.cu $(CSRC)/rt_multi.cu $(CSRC)/rt_denoise.cu $(CSRC)/rt_adaptive.cu
+CU_SRCS   := $(CSRC)/rt_api.cu $(CSRC)/rt_kernels.cu $(CSRC)/rt_wavefront.cu $(CSRC)/rt_lbvh.cu $(CSRC)/rt_jpeg.cu $(CSRC)/rt_jpeg_decode.cu $(CSRC)/rt_multi.cu $(CSRC)/rt_denoise.cu $(CSRC)/rt_adaptive.cu $(CSRC)/rt_selftest.cu
 CPP_SRCS  := $(CSRC)/rt_host.cpp $(CSRC)/rt_bvh_host.cpp $(CSRC)/rt_jpeg_decode_host.cpp
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(CU_SRCS))
 CPP_OBJS  := $(patsubst $(CSRC)/%.cpp,$(OBJDIR)/%.o,$(CPP_SRCS))

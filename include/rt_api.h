@@ -277,6 +277,22 @@ rt_status rt_trace_primary(rt_context* ctx, const rt_scene* scene, const rt_ray*
  * __fsqrt_rz(x) } for n caller-supplied operand pairs (HOST arrays), so a test can require bit equality. */
 rt_status rt_selftest_rz(rt_context* ctx, const float* x, const float* y, size_t n, float* out);
 
+/* Self-tests of the device-wide primitives the LBVH build, the 4-wide compaction, the adaptive pixel list and the JPEG
+ * writer are built on (csrc/rt_prims.cuh), with HOST arrays in and out.  Each call allocates its device buffers and the
+ * primitive's scratch from the context's pool with the sizes the library's own callers use, puts 256 bytes of 0xA5
+ * before and after every buffer the primitive may write, and sets *overrun to 1 if any of those bytes changed, else 0.
+ * Arguments are checked before any device work; n = 0 is valid, launches nothing and writes no output array.
+ * Exclusive prefix sum of n unsigned integers of elem_bytes (4 or 8) bytes, wrapping like the integer type:
+ * out[i] = in[0] + ... + in[i-1].  in_place != 0 scans one device buffer in place, else from an input buffer into an
+ * output buffer. */
+rt_status rt_selftest_exclusive_sum(rt_context* ctx, const void* in, void* out, size_t n, int32_t elem_bytes, int32_t in_place,
+                                    int32_t* overrun);
+/* Stable LSD radix sort of n (64-bit key, 32-bit value) pairs by the key bits [0, 8*passes), passes in [1, 8], n < 2^32:
+ * keys_out / vals_out receive the sorted pairs with their full keys; *in_alt = 1 when the result came out of the
+ * ping-pong buffers (an odd number of passes). */
+rt_status rt_selftest_sort_pairs(rt_context* ctx, const uint64_t* keys, const uint32_t* vals, size_t n, int32_t passes,
+                                 uint64_t* keys_out, uint32_t* vals_out, int32_t* in_alt, int32_t* overrun);
+
 /* Second parity hook: closest hit + one shading step per ray (see rt_shade_sample). */
 rt_status rt_shade_probe(rt_context* ctx, const rt_scene* scene, const rt_ray* rays, size_t n,
                          const rt_render_params* p, int use_bvh, rt_shade_sample* out);

@@ -146,6 +146,9 @@ _SIGNATURES = {
     "rt_scene_get_info": (C.c_int, [_VP, C.POINTER(rt_scene_info)]),
     "rt_trace_primary": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_float, C.c_int, _VP]),
     "rt_selftest_rz": (C.c_int, [_VP, _VP, _VP, C.c_size_t, _VP]),
+    "rt_selftest_exclusive_sum": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
+    "rt_selftest_sort_pairs": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_int32, _VP, _VP, C.POINTER(C.c_int32),
+                                         C.POINTER(C.c_int32)]),
     "rt_shade_probe": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.POINTER(rt_render_params), C.c_int, _VP]),
     "rt_render": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), _VP, C.POINTER(rt_stats)]),
     "rt_render_accum": (C.c_int, [_VP, _VP, C.POINTER(rt_render_params), _VP, C.POINTER(rt_stats)]),
@@ -573,6 +576,32 @@ def selftest_rz(ctx: "Context", x: np.ndarray, y: np.ndarray) -> np.ndarray:
     out = np.empty((x.size, 4), np.float32)
     _check(ctx.lib, ctx.lib.rt_selftest_rz(ctx._h, x.ctypes.data, y.ctypes.data, x.size, out.ctypes.data))
     return out
+
+
+def selftest_exclusive_sum(ctx: "Context", values: np.ndarray, in_place: bool = False, out: np.ndarray | None = None):
+    """rt_selftest_exclusive_sum on a uint32 or uint64 array -> (exclusive prefix sums, overrun).  `out` (same dtype and
+    size) receives the sums when given."""
+    values = np.ascontiguousarray(values)
+    assert values.dtype in (np.uint32, np.uint64), values.dtype
+    if out is None:
+        out = np.empty_like(values)
+    assert out.dtype == values.dtype and out.size == values.size and out.flags.c_contiguous
+    overrun = C.c_int32(-1)
+    _check(ctx.lib, ctx.lib.rt_selftest_exclusive_sum(ctx._h, values.ctypes.data, out.ctypes.data, values.size, values.itemsize,
+                                                      int(in_place), C.byref(overrun)))
+    return out, bool(overrun.value)
+
+
+def selftest_sort_pairs(ctx: "Context", keys: np.ndarray, vals: np.ndarray, passes: int):
+    """rt_selftest_sort_pairs -> (sorted uint64 keys, uint32 values, in_alt, overrun): stable by the key bits
+    [0, 8 * passes)."""
+    keys, vals = np.ascontiguousarray(keys, np.uint64), np.ascontiguousarray(vals, np.uint32)
+    assert keys.size == vals.size
+    k_out, v_out = np.empty_like(keys), np.empty_like(vals)
+    in_alt, overrun = C.c_int32(-1), C.c_int32(-1)
+    _check(ctx.lib, ctx.lib.rt_selftest_sort_pairs(ctx._h, keys.ctypes.data, vals.ctypes.data, keys.size, passes, k_out.ctypes.data,
+                                                   v_out.ctypes.data, C.byref(in_alt), C.byref(overrun)))
+    return k_out, v_out, bool(in_alt.value), bool(overrun.value)
 
 
 def shard_samples(spp_total: int, rank: int, world: int):
