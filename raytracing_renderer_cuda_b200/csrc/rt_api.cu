@@ -12,18 +12,20 @@
 #include <exception>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rt_bvh_host.hpp"
-#include "rt_jpeg.cuh"
+#include "rt_internal.hpp"
 #include "rt_jpeg_decode.cuh"
-#include "rt_kernels.cuh"
 #include "rt_lbvh.cuh"
 
 namespace {
-
 thread_local std::string g_last_error;
+thread_local cudaMemPool_t g_thread_pool = nullptr;
+} // namespace
 
+namespace rtd {
 void set_error(const char* fmt, ...) {
     char buf[1024];
     va_list ap;
@@ -32,60 +34,17 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
     g_last_error = buf;
 }
-
-} // namespace
-namespace rtd {
-namespace {
-thread_local cudaMemPool_t g_thread_pool = nullptr;
-}
+void set_error_message(const char* msg) { g_last_error = msg ? msg : ""; }
 void set_thread_mempool(cudaMemPool_t pool) { g_thread_pool = pool; }
 cudaError_t malloc_async_bytes(void** p, size_t bytes, cudaStream_t st) {
     return g_thread_pool ? cudaMallocFromPoolAsync(p, bytes, g_thread_pool, st) : cudaMallocAsync(p, bytes, st);
 }
-// message hook for the host-only translation unit (rt_host.cpp), which has no CUDA error paths of its own
-void set_error_message(const char* msg) { g_last_error = msg ? msg : ""; }
 } // namespace rtd
-namespace {
 
-#define CUDA_TRY(expr)                                                                          \
-    do {                                                                                        \
-        cudaError_t e__ = (expr);                                                               \
-        if (e__ != cudaSuccess) {                                                               \
-            set_error("%s:%d: %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(e__));   \
-            return e__ == cudaErrorMemoryAllocation ? RT_ERR_OOM : RT_ERR_CUDA;                 \
-        }                                                                                       \
-    } while (0)
-
-// Every rt_status entry point is a function-try-block closed by this: nothing propagates through the C ABI
-// (SURVEY.md 8b "no exceptions across the boundary"); host containers that cannot grow are RT_ERR_OOM.
-#define RT_API_CATCH                                   \
-    catch (const std::bad_alloc&) {                    \
-        set_error("out of host memory");               \
-        return RT_ERR_OOM;                             \
-    }                                                  \
-    catch (const std::exception& e) {                  \
-        set_error("unexpected exception: %s", e.what()); \
-        return RT_ERR_INVALID_ARG;                     \
-    }
-#define ARG_CHECK(cond, msg)                  \
-    do {                                      \
-        if (!(cond)) {                        \
-            set_error("invalid argument: %s", msg); \
-            return RT_ERR_INVALID_ARG;        \
-        }                                     \
-    } while (0)
-
-} // namespace
-
-#include "rt_internal.hpp"
+using rtd::make_current;
+using rtd::set_error;
 
 namespace {
-
-rt_status make_current(const rt_context* ctx) {
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    rtd::set_thread_mempool(ctx->pool);
-    return RT_OK;
-}
 
 template <class T>
 rt_status dev_alloc(rt_scene* s, T** out, size_t count) {
@@ -217,35 +176,15 @@ rtd::DRenderParams to_device_params(const rt_render_params& p) {
     return d;
 }
 
-rt_status ensure_accum(rt_context* ctx, size_t npix) {
-    if (ctx->accum_px < npix) {
-        if (ctx->accum) cudaFree(ctx->accum);
-        ctx->accum = nullptr;
-        ctx->accum_px = 0;
-        CUDA_TRY(cudaMalloc(&ctx->accum, npix * sizeof(float4)));
-        ctx->accum_px = npix;
-    }
-    return RT_OK;
-}
-
-rt_status ensure_out(rt_context* ctx, size_t npix) {
-    if (ctx->out_px < npix) {
-        if (ctx->out_rgb) cudaFree(ctx->out_rgb);
-        ctx->out_rgb = nullptr;
-        ctx->out_px = 0;
-        CUDA_TRY(cudaMalloc(&ctx->out_rgb, npix * 3 * sizeof(float)));
-        ctx->out_px = npix;
-    }
-    return RT_OK;
-}
-
-rt_status ensure_rgb8(rt_context* ctx, size_t npix) {
-    if (ctx->rgb8_px < npix) {
-        if (ctx->rgb8) cudaFree(ctx->rgb8);
-        ctx->rgb8 = nullptr;
-        ctx->rgb8_px = 0;
-        CUDA_TRY(cudaMalloc(&ctx->rgb8, npix * 3));
-        ctx->rgb8_px = npix;
+// a context buffer of at least n elements (it grows, never shrinks)
+template <class T>
+rt_status grow(T*& p, size_t& cap, size_t n) {
+    if (cap < n) {
+        if (p) cudaFree(p);
+        p = nullptr;
+        cap = 0;
+        CUDA_TRY(cudaMalloc(&p, n * sizeof(T)));
+        cap = n;
     }
     return RT_OK;
 }
@@ -325,34 +264,78 @@ rt_status render_pass(rt_context* ctx, const rt_scene* scene, const rtd::DRender
     return RT_OK;
 }
 
+// The timed window of a render when stats are wanted: stats_begin zeroes the ray counter and records ev[0]; stats_end
+// records ev[1], reads the counter back (synchronising) and fills the render's part of *stats.
+rt_status stats_begin(rt_context* ctx, const rt_stats* stats) {
+    if (!stats) return RT_OK;
+    CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[0], ctx->stream));
+    return RT_OK;
+}
+
+rt_status stats_end(rt_context* ctx, rt_stats* stats, uint64_t paths, uint32_t launches, uint32_t iterations) {
+    if (!stats) return RT_OK;
+    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
+    unsigned long long rays = 0;
+    CUDA_TRY(cudaMemcpyAsync(&rays, ctx->d_ray_counter, sizeof rays, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    memset(stats, 0, sizeof *stats);
+    CUDA_TRY(cudaEventElapsedTime(&stats->ms_total, ctx->ev[0], ctx->ev[1]));
+    stats->paths = paths;
+    stats->rays = rays;
+    stats->launches = launches;
+    stats->iterations = iterations;
+    return RT_OK;
+}
+
 // Core: adds rp.spp samples per pixel into accum (device).  Fills stats if requested
 // (which synchronises the stream).
 rt_status render_rp(rt_context* ctx, const rt_scene* scene, const rtd::DRenderParams& rp, uint32_t pipeline, float4* accum,
                     rt_stats* stats) {
     uint32_t launches = 0, iterations = 0;
-    if (stats) {
-        CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), ctx->stream));
-        CUDA_TRY(cudaEventRecord(ctx->ev[0], ctx->stream));
-    }
-    rt_status st = render_pass(ctx, scene, rp, pipeline, accum, &launches, &iterations);
+    rt_status st = stats_begin(ctx, stats);
     if (st != RT_OK) return st;
-    if (stats) {
-        CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
-        unsigned long long rays = 0;
-        CUDA_TRY(cudaMemcpyAsync(&rays, ctx->d_ray_counter, sizeof rays, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        memset(stats, 0, sizeof *stats);
-        CUDA_TRY(cudaEventElapsedTime(&stats->ms_total, ctx->ev[0], ctx->ev[1]));
-        stats->paths = uint64_t(rp.width) * uint64_t(rp.height) * uint64_t(rp.spp);
-        stats->rays = rays;
-        stats->launches = launches;
-        stats->iterations = iterations;
-    }
+    if ((st = render_pass(ctx, scene, rp, pipeline, accum, &launches, &iterations)) != RT_OK) return st;
+    return stats_end(ctx, stats, uint64_t(rp.width) * uint64_t(rp.height) * uint64_t(rp.spp), launches, iterations);
+}
+
+// the pixel finalisation of the n_frames frames of ctx->accum into ctx->out_rgb
+rt_status tonemap_frames(rt_context* ctx, const rt_render_params* p, int32_t n_frames) {
+    const size_t npix = size_t(p->width) * size_t(p->height);
+    for (int32_t f = 0; f < n_frames; ++f)
+        rtd::launch_tonemap(ctx->accum + size_t(f) * npix, p->width, p->height, ctx->out_rgb + size_t(f) * npix * 3, nullptr,
+                            ctx->sm_count, ctx->stream);
+    CUDA_TRY(cudaGetLastError());
     return RT_OK;
 }
 
-rt_status render_into(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float4* accum, rt_stats* stats) {
-    return render_rp(ctx, scene, to_device_params(*p), p->pipeline, accum, stats);
+struct HostCopy {
+    const void* src = nullptr;
+    void* dst = nullptr;
+    size_t bytes = 0;
+};
+
+// The end of a host render entry, after the render into ctx->accum: `finalise` (the kernels that make the device image;
+// nullptr: none) between ev[1] and ev[2], the copy of `image` to the host between ev[2] and ev[3], then `also` (untimed),
+// one synchronisation, and the two windows in stats->ms_tonemap / ms_d2h.  *out_stats = stats on success.
+template <class Finalise>
+rt_status finish_to_host(rt_context* ctx, Finalise&& finalise, const HostCopy& image, rt_stats& stats, rt_stats* out_stats,
+                         const HostCopy& also = {}) {
+    constexpr bool kFinalise = !std::is_null_pointer<std::decay_t<Finalise>>::value;
+    if constexpr (kFinalise) {
+        CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
+        const rt_status st = finalise();
+        if (st != RT_OK) return st;
+    }
+    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(image.dst, image.src, image.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
+    if (also.bytes) CUDA_TRY(cudaMemcpyAsync(also.dst, also.src, also.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if constexpr (kFinalise) CUDA_TRY(cudaEventElapsedTime(&stats.ms_tonemap, ctx->ev[1], ctx->ev[2]));
+    CUDA_TRY(cudaEventElapsedTime(&stats.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    if (out_stats) *out_stats = stats;
+    return RT_OK;
 }
 
 } // namespace
@@ -574,14 +557,13 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
             }
         }
         const uint32_t m = big.empty() ? n : uint32_t(normal.size());
-        uint32_t* d_ids = nullptr;
+        rtd::PoolBuffer<uint32_t> d_ids;
         if (!big.empty()) {
-            CUDA_TRY(rtd::malloc_async(&d_ids, m * sizeof(uint32_t), stream));
-            CUDA_TRY(cudaMemcpyAsync(d_ids, normal.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+            CUDA_TRY(d_ids.alloc(m, stream));
+            CUDA_TRY(cudaMemcpyAsync(d_ids.get(), normal.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
         }
         float rb[6];
-        cudaError_t e = rtd::lbvh_build(da, db, n_static, d_ids, m, dnodes, stream, &lbvh_ms, &bstats.depth, rb);
-        if (d_ids) cudaFreeAsync(d_ids, stream);
+        cudaError_t e = rtd::lbvh_build(da, db, n_static, d_ids.get(), m, dnodes, stream, &lbvh_ms, &bstats.depth, rb);
         if (e != cudaSuccess) {
             set_error("GPU LBVH build failed: %s", cudaGetErrorString(e));
             return RT_ERR_CUDA;
@@ -628,17 +610,15 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     uint32_t n_nodes4 = 0, root4 = 0;
     if (dnodes && n_nodes) { // the 4-wide form the persistent-lane kernel walks (half the dependent node fetches per ray)
         if ((st = dev_alloc(s, &dnodes4, n_nodes / 2 + 64)) != RT_OK) return st;
-        rtd::BvhNode4* scratch = nullptr; // worst case (a degenerate chain) every binary node survives
-        CUDA_TRY(rtd::malloc_async(&scratch, size_t(n_nodes) * sizeof(rtd::BvhNode4), stream));
-        cudaError_t e = rtd::bvh_collapse4(dnodes, n_nodes, bvh_root, bstats.depth, scratch, &n_nodes4, &root4, stream);
+        rtd::PoolBuffer<rtd::BvhNode4> scratch; // worst case (a degenerate chain) every binary node survives
+        CUDA_TRY(scratch.alloc(n_nodes, stream));
+        cudaError_t e = rtd::bvh_collapse4(dnodes, n_nodes, bvh_root, bstats.depth, scratch.get(), &n_nodes4, &root4, stream);
         if (e == cudaSuccess && n_nodes4 <= n_nodes / 2 + 64) {
-            e = cudaMemcpyAsync(dnodes4, scratch, size_t(n_nodes4) * sizeof(rtd::BvhNode4), cudaMemcpyDeviceToDevice, stream);
+            e = cudaMemcpyAsync(dnodes4, scratch.get(), size_t(n_nodes4) * sizeof(rtd::BvhNode4), cudaMemcpyDeviceToDevice, stream);
         } else if (e == cudaSuccess) { // unusually deep tree: keep the big array itself
-            s->allocs.push_back(scratch);
-            dnodes4 = scratch;
-            scratch = nullptr;
+            s->allocs.push_back(scratch.get());
+            dnodes4 = scratch.release();
         }
-        if (scratch) cudaFreeAsync(scratch, stream);
         if (e != cudaSuccess) {
             set_error("4-wide BVH collapse failed: %s", cudaGetErrorString(e));
             return RT_ERR_CUDA;
@@ -680,12 +660,11 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     for (uint32_t i = 0; i < desc->n_images; ++i) {
         const rt_image& im = desc->images[i];
         const size_t texels = size_t(im.width) * size_t(im.height);
-        float* d_rgb = nullptr;
-        float4* d_rgba = nullptr;
-        CUDA_TRY(rtd::malloc_async(&d_rgb, texels * 3 * sizeof(float), stream));
-        cudaError_t e = rtd::malloc_async(&d_rgba, texels * sizeof(float4), stream);
+        rtd::PoolBuffer<float> d_rgb;
+        rtd::PoolBuffer<float4> d_rgba;
+        CUDA_TRY(d_rgb.alloc(texels * 3, stream));
+        cudaError_t e = d_rgba.alloc(texels, stream);
         if (e != cudaSuccess) {
-            cudaFreeAsync(d_rgb, stream);
             set_error("cudaMallocAsync(image staging) failed: %s", cudaGetErrorString(e));
             return RT_ERR_OOM;
         }
@@ -700,18 +679,16 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
                 }
         }
         cudaChannelFormatDesc cd = cudaCreateChannelDesc<float4>();
-        e = cudaMemcpyAsync(d_rgb, im.rgb, texels * 3 * sizeof(float), cudaMemcpyHostToDevice, stream);
+        e = cudaMemcpyAsync(d_rgb.get(), im.rgb, texels * 3 * sizeof(float), cudaMemcpyHostToDevice, stream);
         if (e == cudaSuccess) {
-            rtd::launch_rgb_to_rgba(d_rgb, d_rgba, texels, ctx->sm_count, stream);
+            rtd::launch_rgb_to_rgba(d_rgb.get(), d_rgba.get(), texels, ctx->sm_count, stream);
             if (!arr) e = cudaMallocArray(&arr, &cd, size_t(im.width), size_t(im.height));
         }
         if (e == cudaSuccess) {
             s->arrays.push_back(rt_context::CachedArray{im.width, im.height, arr});
-            e = cudaMemcpy2DToArrayAsync(arr, 0, 0, d_rgba, size_t(im.width) * sizeof(float4), size_t(im.width) * sizeof(float4),
+            e = cudaMemcpy2DToArrayAsync(arr, 0, 0, d_rgba.get(), size_t(im.width) * sizeof(float4), size_t(im.width) * sizeof(float4),
                                          size_t(im.height), cudaMemcpyDeviceToDevice, stream);
         }
-        cudaFreeAsync(d_rgb, stream);
-        cudaFreeAsync(d_rgba, stream);
         if (e != cudaSuccess) {
             set_error("image texture upload failed: %s", cudaGetErrorString(e));
             return RT_ERR_CUDA;
@@ -825,19 +802,17 @@ rt_status rt_trace_primary(rt_context* ctx, const rt_scene* scene, const rt_ray*
     if (n == 0) return RT_OK;
     rt_status st = make_current(ctx);
     if (st != RT_OK) return st;
-    rt_ray* d_rays = nullptr;
-    rt_hit* d_hits = nullptr;
-    CUDA_TRY(rtd::malloc_async(&d_rays, n * sizeof(rt_ray), ctx->stream));
-    cudaError_t e = rtd::malloc_async(&d_hits, n * sizeof(rt_hit), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, ctx->stream);
+    rtd::PoolBuffer<rt_ray> d_rays;
+    rtd::PoolBuffer<rt_hit> d_hits;
+    CUDA_TRY(d_rays.alloc(n, ctx->stream));
+    cudaError_t e = d_hits.alloc(n, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays.get(), rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) {
-        rtd::launch_trace_primary(scene->d, d_rays, n, tmin, use_bvh, d_hits, ctx->stream);
+        rtd::launch_trace_primary(scene->d, d_rays.get(), n, tmin, use_bvh, d_hits.get(), ctx->stream);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(hits, d_hits, n * sizeof(rt_hit), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(hits, d_hits.get(), n * sizeof(rt_hit), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFreeAsync(d_rays, ctx->stream);
-    if (d_hits) cudaFreeAsync(d_hits, ctx->stream);
     if (e != cudaSuccess) {
         set_error("rt_trace_primary: %s", cudaGetErrorString(e));
         return RT_ERR_CUDA;
@@ -853,21 +828,19 @@ rt_status rt_shade_probe(rt_context* ctx, const rt_scene* scene, const rt_ray* r
     if (n == 0) return RT_OK;
     rt_status st = make_current(ctx);
     if (st != RT_OK) return st;
-    rt_ray* d_rays = nullptr;
-    rt_shade_sample* d_out = nullptr;
-    CUDA_TRY(rtd::malloc_async(&d_rays, n * sizeof(rt_ray), ctx->stream));
-    cudaError_t e = rtd::malloc_async(&d_out, n * sizeof(rt_shade_sample), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, ctx->stream);
+    rtd::PoolBuffer<rt_ray> d_rays;
+    rtd::PoolBuffer<rt_shade_sample> d_out;
+    CUDA_TRY(d_rays.alloc(n, ctx->stream));
+    cudaError_t e = d_out.alloc(n, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_rays.get(), rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) {
         rtd::DRenderParams rp = to_device_params(*p);
         rp.flags = 0; // the probe reports the reference estimator's terms (rt_shade_sample carries no path weight)
-        rtd::launch_shade_probe(scene->d, rp, d_rays, n, use_bvh != 0, d_out, ctx->stream);
+        rtd::launch_shade_probe(scene->d, rp, d_rays.get(), n, use_bvh != 0, d_out.get(), ctx->stream);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, n * sizeof(rt_shade_sample), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out.get(), n * sizeof(rt_shade_sample), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFreeAsync(d_rays, ctx->stream);
-    if (d_out) cudaFreeAsync(d_out, ctx->stream);
     if (e != cudaSuccess) {
         set_error("rt_shade_probe: %s", cudaGetErrorString(e));
         return RT_ERR_CUDA;
@@ -881,7 +854,7 @@ rt_status rt_render_accum_device(rt_context* ctx, const rt_scene* scene, const r
     rt_status st = check_params(p);
     if (st != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
-    return render_into(ctx, scene, p, static_cast<float4*>(accum_dev), stats);
+    return render_rp(ctx, scene, to_device_params(*p), p->pipeline, static_cast<float4*>(accum_dev), stats);
 } RT_API_CATCH
 
 rt_status rt_render_accum(rt_context* ctx, const rt_scene* scene, const rt_render_params* p, float* out_accum, rt_stats* stats) try {
@@ -890,17 +863,11 @@ rt_status rt_render_accum(rt_context* ctx, const rt_scene* scene, const rt_rende
     if (st != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
     rt_stats local;
-    if ((st = render_into(ctx, scene, p, ctx->accum, &local)) != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_accum, ctx->accum, npix * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
-    if (stats) *stats = local;
-    return RT_OK;
+    if ((st = render_rp(ctx, scene, to_device_params(*p), p->pipeline, ctx->accum, &local)) != RT_OK) return st;
+    return finish_to_host(ctx, nullptr, {ctx->accum, out_accum, npix * sizeof(float4)}, local, stats);
 } RT_API_CATCH
 
 rt_status rt_tonemap_device(rt_context* ctx, const void* accum_dev, int32_t width, int32_t height, void* out_rgb_dev,
@@ -921,21 +888,18 @@ rt_status rt_selftest_rz(rt_context* ctx, const float* x, const float* y, size_t
     if (n == 0) return RT_OK;
     rt_status st = make_current(ctx);
     if (st != RT_OK) return st;
-    float *dx = nullptr, *dy = nullptr, *dout = nullptr;
-    CUDA_TRY(rtd::malloc_async(&dx, n * sizeof(float), ctx->stream));
-    cudaError_t e = rtd::malloc_async(&dy, n * sizeof(float), ctx->stream);
-    if (e == cudaSuccess) e = rtd::malloc_async(&dout, 4 * n * sizeof(float), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dx, x, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dy, y, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    rtd::PoolBuffer<float> dx, dy, dout;
+    CUDA_TRY(dx.alloc(n, ctx->stream));
+    cudaError_t e = dy.alloc(n, ctx->stream);
+    if (e == cudaSuccess) e = dout.alloc(4 * n, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dx.get(), x, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dy.get(), y, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) {
-        rtd::launch_selftest_rz(dx, dy, n, dout, ctx->stream);
+        rtd::launch_selftest_rz(dx.get(), dy.get(), n, dout.get(), ctx->stream);
         e = cudaGetLastError();
     }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, 4 * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout.get(), 4 * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (dx) cudaFreeAsync(dx, ctx->stream);
-    if (dy) cudaFreeAsync(dy, ctx->stream);
-    if (dout) cudaFreeAsync(dout, ctx->stream);
     if (e != cudaSuccess) {
         set_error("rt_selftest_rz: %s", cudaGetErrorString(e));
         return RT_ERR_CUDA;
@@ -969,23 +933,14 @@ rt_status rt_render(rt_context* ctx, const rt_scene* scene, const rt_render_para
     if (st != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
-    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->out_rgb, ctx->out_rgb_n, npix * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
     rt_stats local;
-    if ((st = render_into(ctx, scene, p, ctx->accum, &local)) != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
-    rtd::launch_tonemap(ctx->accum, p->width, p->height, ctx->out_rgb, nullptr, ctx->sm_count, ctx->stream);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    if ((st = render_rp(ctx, scene, to_device_params(*p), p->pipeline, ctx->accum, &local)) != RT_OK) return st;
     local.launches += 1;
-    if (stats) *stats = local;
-    return RT_OK;
+    return finish_to_host(ctx, [&] { return tonemap_frames(ctx, p, 1); }, {ctx->out_rgb, out_rgb, npix * 3 * sizeof(float)}, local,
+                          stats);
 } RT_API_CATCH
 
 size_t rt_jpeg_max_bytes(int32_t width, int32_t height) {
@@ -1009,7 +964,7 @@ rt_status rt_jpeg_encode(rt_context* ctx, const uint8_t* rgb8, int32_t width, in
     rt_status st = make_current(ctx);
     if (st != RT_OK) return st;
     const size_t npix = size_t(width) * size_t(height);
-    if ((st = ensure_rgb8(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->rgb8, ctx->rgb8_n, npix * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemcpyAsync(ctx->rgb8, rgb8, npix * 3, cudaMemcpyHostToDevice, ctx->stream));
     return jpeg_from_device(ctx, ctx->rgb8, width, height, quality, out_jpg, cap, n_bytes, nullptr);
 } RT_API_CATCH
@@ -1043,11 +998,11 @@ rt_status rt_render_jpeg(rt_context* ctx, const rt_scene* scene, const rt_render
     ARG_CHECK(p->width < 65536 && p->height < 65536, "JPEG dimensions must be in [1, 65535]");
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
-    if ((st = ensure_rgb8(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->rgb8, ctx->rgb8_n, npix * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
     rt_stats local;
-    if ((st = render_into(ctx, scene, p, ctx->accum, &local)) != RT_OK) return st;
+    if ((st = render_rp(ctx, scene, to_device_params(*p), p->pipeline, ctx->accum, &local)) != RT_OK) return st;
     CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
     rtd::launch_tonemap(ctx->accum, p->width, p->height, nullptr, ctx->rgb8, ctx->sm_count, ctx->stream);
     CUDA_TRY(cudaGetLastError());
@@ -1069,8 +1024,8 @@ rt_status rt_render_progressive(rt_context* ctx, const rt_scene* scene, const rt
     if (st != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
-    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->out_rgb, ctx->out_rgb_n, npix * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
     rt_stats total;
     memset(&total, 0, sizeof total);
@@ -1078,10 +1033,9 @@ rt_status rt_render_progressive(rt_context* ctx, const rt_scene* scene, const rt
         rt_render_params pk = *p;
         pk.sample_offset = p->sample_offset + k * p->spp; // Philox keys use the global sample index: no sample repeats
         rt_stats local;
-        if ((st = render_into(ctx, scene, &pk, ctx->accum, &local)) != RT_OK) return st;
+        if ((st = render_rp(ctx, scene, to_device_params(pk), pk.pipeline, ctx->accum, &local)) != RT_OK) return st;
         // the accumulator carries the sample count per pixel, so the same finalisation works after every pass
-        rtd::launch_tonemap(ctx->accum, p->width, p->height, ctx->out_rgb, nullptr, ctx->sm_count, ctx->stream);
-        CUDA_TRY(cudaGetLastError());
+        if ((st = tonemap_frames(ctx, p, 1)) != RT_OK) return st;
         CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         total.paths += local.paths;
@@ -1136,19 +1090,18 @@ rt_status denoise_into(rt_context* ctx, const float4* accum, const float4* featu
         return RT_OK;
     }
     const size_t npix = size_t(width) * size_t(height);
-    float4* scratch = nullptr;
-    CUDA_TRY(rtd::malloc_async(&scratch, 2 * npix * sizeof(float4), ctx->stream));
+    rtd::PoolBuffer<float4> scratch;
+    CUDA_TRY(scratch.alloc(2 * npix, ctx->stream));
     const float4* in = accum;
-    float4* out = scratch;
+    float4* out = scratch.get();
     for (int32_t level = 0; level < d->iterations; ++level) {
         rtd::launch_atrous(in, level == 0, features, width, height, level, d->sigma_color, d->sigma_normal, d->sigma_depth,
                            d->sigma_albedo, out, ctx->stream);
         in = out;
-        out = out == scratch ? scratch + npix : scratch;
+        out = out == scratch.get() ? scratch.get() + npix : scratch.get();
     }
     rtd::launch_tonemap(in, width, height, out_rgb, out_rgb8, ctx->sm_count, ctx->stream);
     const cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(scratch, ctx->stream);
     if (e != cudaSuccess) {
         set_error("denoise: %s", cudaGetErrorString(e));
         return RT_ERR_CUDA;
@@ -1193,27 +1146,19 @@ rt_status rt_render_denoised(rt_context* ctx, const rt_scene* scene, const rt_re
     ARG_CHECK(int64_t(p->sample_offset) + d->feature_spp <= INT32_MAX, "sample indices exceed 2^31");
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
-    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->out_rgb, ctx->out_rgb_n, npix * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, npix * sizeof(float4), ctx->stream));
     rt_stats local;
-    if ((st = render_into(ctx, scene, p, ctx->accum, &local)) != RT_OK) return st;
-    float4* features = nullptr;
-    CUDA_TRY(rtd::malloc_async(&features, 2 * npix * sizeof(float4), ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
-    st = features_into(ctx, scene, p, d->feature_spp, features);
-    if (st == RT_OK) st = denoise_into(ctx, ctx->accum, features, p->width, p->height, d, ctx->out_rgb, nullptr);
-    cudaFreeAsync(features, ctx->stream);
-    if (st != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
+    if ((st = render_rp(ctx, scene, to_device_params(*p), p->pipeline, ctx->accum, &local)) != RT_OK) return st;
+    rtd::PoolBuffer<float4> features;
+    CUDA_TRY(features.alloc(2 * npix, ctx->stream));
+    auto finalise = [&] {
+        const rt_status s = features_into(ctx, scene, p, d->feature_spp, features.get());
+        return s != RT_OK ? s : denoise_into(ctx, ctx->accum, features.get(), p->width, p->height, d, ctx->out_rgb, nullptr);
+    };
     local.launches += 2 + uint32_t(d->iterations); // features, the levels, the finalisation
-    if (stats) *stats = local;
-    return RT_OK;
+    return finish_to_host(ctx, finalise, {ctx->out_rgb, out_rgb, npix * 3 * sizeof(float)}, local, stats);
 } RT_API_CATCH
 
 void rt_default_adaptive_params(rt_adaptive_params* a) {
@@ -1250,71 +1195,55 @@ rt_status adaptive_into(rt_context* ctx, const rt_scene* scene, const rt_render_
     auto align = [](size_t b) { return (b + 255) & ~size_t(255); };
     const size_t b_planes = align(2 * size_t(npix) * sizeof(float4)), b_px = align(size_t(npix) * sizeof(uint32_t));
     const size_t b_words = align(rtd::adapt_select_scratch_words(npix) * sizeof(uint32_t));
-    char* base = nullptr; // planes A and B, the error map, two pixel lists, the selection's words, the list length
-    CUDA_TRY(rtd::malloc_async(&base, b_planes + 3 * b_px + b_words + 256, stream));
+    rtd::PoolBuffer<char> mem; // planes A and B, the error map, two pixel lists, the selection's words, the list length
+    CUDA_TRY(mem.alloc(b_planes + 3 * b_px + b_words + 256, stream));
+    char* base = mem.get();
     float4* planes = reinterpret_cast<float4*>(base);
     float* e = reinterpret_cast<float*>(base + b_planes);
     uint32_t* list[2] = {reinterpret_cast<uint32_t*>(base + b_planes + b_px), reinterpret_cast<uint32_t*>(base + b_planes + 2 * b_px)};
     uint32_t* words = reinterpret_cast<uint32_t*>(base + b_planes + 3 * b_px);
     uint32_t* n_dev = reinterpret_cast<uint32_t*>(base + b_planes + 3 * b_px + b_words);
-    const rt_status st = [&]() -> rt_status {
-        CUDA_TRY(cudaMemsetAsync(planes, 0, 2 * size_t(npix) * sizeof(float4), stream));
-        CUDA_TRY(cudaMemsetAsync(ctx->d_ray_counter, 0, sizeof(unsigned long long), stream));
-        CUDA_TRY(cudaEventRecord(ctx->ev[0], stream));
-        rtd::launch_adapt_iota(list[0], npix, stream);
-        rtd::DRenderParams rp = to_device_params(*p);
-        rp.adapt_first = uint32_t(p->sample_offset);
-        rp.adapt_plane = npix;
-        uint32_t n = npix, launches = 2, iterations = 0; // (iota and merge)
-        int32_t done = 0, passes = 0, cur = 0;          // samples of every listed pixel so far, passes run, current list
-        uint64_t paths = 0;
-        for (;;) {
-            rp.spp = passes == 0 ? a->min_spp : a->step_spp;
-            rp.sample_offset = p->sample_offset + done;
-            rp.adapt_pixels = list[cur];
-            rp.div_npix = rtd::make_fastdiv(n);
-            uint32_t l = 0, it = 0;
-            const rt_status s = render_pass(ctx, scene, rp, p->pipeline, planes, &l, &it);
-            if (s != RT_OK) return s;
-            launches += l;
-            iterations += it;
-            paths += uint64_t(n) * uint64_t(rp.spp);
-            done += rp.spp;
-            ++passes;
-            if (done >= a->max_spp) break;
-            CUDA_TRY(rtd::launch_adapt_select(planes, p->width, p->height, list[cur], n, a->threshold, a->max_spp, e, words, list[cur ^ 1],
-                                              n_dev, &l, stream));
-            launches += l;
-            uint32_t n_next = 0;
-            CUDA_TRY(cudaMemcpyAsync(&n_next, n_dev, sizeof n_next, cudaMemcpyDeviceToHost, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            if (n_next == 0) break;
-            n = n_next;
-            cur ^= 1;
-        }
-        rtd::launch_adapt_merge(planes, npix, accum, stream);
-        if (error_dev) {
-            rtd::launch_adapt_error_map(planes, p->width, p->height, e, error_dev, stream);
-            launches += 2;
-        }
-        CUDA_TRY(cudaGetLastError());
-        if (passes_out) *passes_out = passes;
-        if (stats) {
-            CUDA_TRY(cudaEventRecord(ctx->ev[1], stream));
-            unsigned long long rays = 0;
-            CUDA_TRY(cudaMemcpyAsync(&rays, ctx->d_ray_counter, sizeof rays, cudaMemcpyDeviceToHost, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream));
-            memset(stats, 0, sizeof *stats);
-            CUDA_TRY(cudaEventElapsedTime(&stats->ms_total, ctx->ev[0], ctx->ev[1]));
-            stats->paths = paths;
-            stats->rays = rays;
-            stats->launches = launches;
-            stats->iterations = iterations;
-        }
-        return RT_OK;
-    }();
-    cudaFreeAsync(base, stream);
-    return st;
+    CUDA_TRY(cudaMemsetAsync(planes, 0, 2 * size_t(npix) * sizeof(float4), stream));
+    rt_status st = stats_begin(ctx, stats);
+    if (st != RT_OK) return st;
+    rtd::launch_adapt_iota(list[0], npix, stream);
+    rtd::DRenderParams rp = to_device_params(*p);
+    rp.adapt_first = uint32_t(p->sample_offset);
+    rp.adapt_plane = npix;
+    uint32_t n = npix, launches = 2, iterations = 0; // (iota and merge)
+    int32_t done = 0, passes = 0, cur = 0;          // samples of every listed pixel so far, passes run, current list
+    uint64_t paths = 0;
+    for (;;) {
+        rp.spp = passes == 0 ? a->min_spp : a->step_spp;
+        rp.sample_offset = p->sample_offset + done;
+        rp.adapt_pixels = list[cur];
+        rp.div_npix = rtd::make_fastdiv(n);
+        uint32_t l = 0, it = 0;
+        if ((st = render_pass(ctx, scene, rp, p->pipeline, planes, &l, &it)) != RT_OK) return st;
+        launches += l;
+        iterations += it;
+        paths += uint64_t(n) * uint64_t(rp.spp);
+        done += rp.spp;
+        ++passes;
+        if (done >= a->max_spp) break;
+        CUDA_TRY(rtd::launch_adapt_select(planes, p->width, p->height, list[cur], n, a->threshold, a->max_spp, e, words, list[cur ^ 1],
+                                          n_dev, &l, stream));
+        launches += l;
+        uint32_t n_next = 0;
+        CUDA_TRY(cudaMemcpyAsync(&n_next, n_dev, sizeof n_next, cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaStreamSynchronize(stream));
+        if (n_next == 0) break;
+        n = n_next;
+        cur ^= 1;
+    }
+    rtd::launch_adapt_merge(planes, npix, accum, stream);
+    if (error_dev) {
+        rtd::launch_adapt_error_map(planes, p->width, p->height, e, error_dev, stream);
+        launches += 2;
+    }
+    CUDA_TRY(cudaGetLastError());
+    if (passes_out) *passes_out = passes;
+    return stats_end(ctx, stats, paths, launches, iterations);
 }
 
 } // namespace
@@ -1327,11 +1256,10 @@ rt_status rt_adaptive_error_device(rt_context* ctx, const void* planes_dev, int3
     ARG_CHECK(uint64_t(width) * uint64_t(height) < (1ull << 31), "frame has more than 2^31 pixels");
     rt_status st = make_current(ctx);
     if (st != RT_OK) return st;
-    float* e = nullptr;
-    CUDA_TRY(rtd::malloc_async(&e, size_t(width) * size_t(height) * sizeof(float), ctx->stream));
-    rtd::launch_adapt_error_map(static_cast<const float4*>(planes_dev), width, height, e, static_cast<float*>(error_dev), ctx->stream);
+    rtd::PoolBuffer<float> e;
+    CUDA_TRY(e.alloc(size_t(width) * size_t(height), ctx->stream));
+    rtd::launch_adapt_error_map(static_cast<const float4*>(planes_dev), width, height, e.get(), static_cast<float*>(error_dev), ctx->stream);
     const cudaError_t err = cudaGetLastError();
-    cudaFreeAsync(e, ctx->stream);
     if (err != cudaSuccess) {
         set_error("adaptive error map: %s", cudaGetErrorString(err));
         return RT_ERR_CUDA;
@@ -1357,25 +1285,16 @@ rt_status rt_render_adaptive(rt_context* ctx, const rt_scene* scene, const rt_re
     if ((st = check_adaptive(p, a)) != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height);
-    if ((st = ensure_accum(ctx, npix)) != RT_OK) return st;
-    if ((st = ensure_out(ctx, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, npix)) != RT_OK) return st;
+    if ((st = grow(ctx->out_rgb, ctx->out_rgb_n, npix * 3)) != RT_OK) return st;
     rt_stats local;
     if ((st = adaptive_into(ctx, scene, p, a, ctx->accum, nullptr, nullptr, &local)) != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
-    rtd::launch_tonemap(ctx->accum, p->width, p->height, ctx->out_rgb, nullptr, ctx->sm_count, ctx->stream);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
-    std::vector<float4> acc(out_spp ? npix : 0);
-    if (out_spp) CUDA_TRY(cudaMemcpyAsync(acc.data(), ctx->accum, npix * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    for (size_t i = 0; i < acc.size(); ++i) out_spp[i] = int32_t(acc[i].w); // (exact: counts stay below 2^24)
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
     local.launches += 1;
-    if (stats) *stats = local;
-    return RT_OK;
+    std::vector<float4> acc(out_spp ? npix : 0); // read back with the image, for the per-pixel sample counts
+    st = finish_to_host(ctx, [&] { return tonemap_frames(ctx, p, 1); }, {ctx->out_rgb, out_rgb, npix * 3 * sizeof(float)}, local,
+                        stats, {ctx->accum, acc.data(), acc.size() * sizeof(float4)});
+    for (size_t i = 0; st == RT_OK && i < acc.size(); ++i) out_spp[i] = int32_t(acc[i].w); // (exact: counts stay below 2^24)
+    return st;
 } RT_API_CATCH
 
 } // extern "C"
@@ -1398,18 +1317,14 @@ rt_status frames_into(rt_context* ctx, const rt_scene* scene, const rt_render_pa
                       float4* accum, rt_stats* stats) {
     std::vector<rtd::DCamera> cams(static_cast<size_t>(n_frames));
     for (int32_t f = 0; f < n_frames; ++f) make_camera(cameras[f], cams[f]);
-    rtd::DCamera* d_cams = nullptr;
-    CUDA_TRY(rtd::malloc_async(&d_cams, cams.size() * sizeof(rtd::DCamera), ctx->stream));
-    const rt_status st = [&]() -> rt_status {
-        CUDA_TRY(cudaMemcpyAsync(d_cams, cams.data(), cams.size() * sizeof(rtd::DCamera), cudaMemcpyHostToDevice, ctx->stream));
-        rtd::DRenderParams rp = to_device_params(*p);
-        rp.spp = p->spp * n_frames; // <= 2^31 - 1: check_frames
-        rp.frame_cams = d_cams;
-        rp.div_spp = rtd::make_fastdiv(uint32_t(p->spp));
-        return render_rp(ctx, scene, rp, p->pipeline, accum, stats);
-    }();
-    cudaFreeAsync(d_cams, ctx->stream);
-    return st;
+    rtd::PoolBuffer<rtd::DCamera> d_cams;
+    CUDA_TRY(d_cams.alloc(cams.size(), ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(d_cams.get(), cams.data(), cams.size() * sizeof(rtd::DCamera), cudaMemcpyHostToDevice, ctx->stream));
+    rtd::DRenderParams rp = to_device_params(*p);
+    rp.spp = p->spp * n_frames; // <= 2^31 - 1: check_frames
+    rp.frame_cams = d_cams.get();
+    rp.div_spp = rtd::make_fastdiv(uint32_t(p->spp));
+    return render_rp(ctx, scene, rp, p->pipeline, accum, stats);
 }
 
 } // namespace
@@ -1432,25 +1347,14 @@ rt_status rt_render_frames(rt_context* ctx, const rt_scene* scene, const rt_rend
     if (st != RT_OK) return st;
     if ((st = make_current(ctx)) != RT_OK) return st;
     const size_t npix = size_t(p->width) * size_t(p->height), total = npix * size_t(n_frames);
-    if ((st = ensure_accum(ctx, total)) != RT_OK) return st;
-    if ((st = ensure_out(ctx, total)) != RT_OK) return st;
+    if ((st = grow(ctx->accum, ctx->accum_n, total)) != RT_OK) return st;
+    if ((st = grow(ctx->out_rgb, ctx->out_rgb_n, total * 3)) != RT_OK) return st;
     CUDA_TRY(cudaMemsetAsync(ctx->accum, 0, total * sizeof(float4), ctx->stream));
     rt_stats local;
     if ((st = frames_into(ctx, scene, p, cameras, n_frames, ctx->accum, &local)) != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(ctx->ev[1], ctx->stream));
-    for (int32_t f = 0; f < n_frames; ++f)
-        rtd::launch_tonemap(ctx->accum + size_t(f) * npix, p->width, p->height, ctx->out_rgb + size_t(f) * npix * 3, nullptr,
-                            ctx->sm_count, ctx->stream);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(ctx->ev[2], ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_rgb, ctx->out_rgb, total * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev[3], ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_tonemap, ctx->ev[1], ctx->ev[2]));
-    CUDA_TRY(cudaEventElapsedTime(&local.ms_d2h, ctx->ev[2], ctx->ev[3]));
     local.launches += uint32_t(n_frames);
-    if (stats) *stats = local;
-    return RT_OK;
+    return finish_to_host(ctx, [&] { return tonemap_frames(ctx, p, n_frames); }, {ctx->out_rgb, out_rgb, total * 3 * sizeof(float)},
+                          local, stats);
 } RT_API_CATCH
 
 namespace {
@@ -1505,15 +1409,14 @@ rt_status rt_jpeg_decode(rt_context* ctx, const uint8_t* file, size_t n_bytes, f
     }
     const int ch = img.n_comp == 1 ? 1 : 3;
     const size_t n = size_t(img.width) * size_t(img.height) * size_t(ch);
-    float* d_out = nullptr;
-    CUDA_TRY(rtd::malloc_async(&d_out, n * sizeof(float), ctx->stream));
-    cudaError_t e = rtd::jpeg_pixels_device(img, d_out, ctx->stream, ms_device);
+    rtd::PoolBuffer<float> d_out;
+    CUDA_TRY(d_out.alloc(n, ctx->stream));
+    cudaError_t e = rtd::jpeg_pixels_device(img, d_out.get(), ctx->stream, ms_device);
     float* host = e == cudaSuccess ? static_cast<float*>(malloc(n * sizeof(float))) : nullptr;
     if (e == cudaSuccess && host) {
-        e = cudaMemcpyAsync(host, d_out, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+        e = cudaMemcpyAsync(host, d_out.get(), n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     }
-    cudaFreeAsync(d_out, ctx->stream);
     if (e != cudaSuccess) {
         free(host);
         set_error("jpeg_decode: %s", cudaGetErrorString(e));

@@ -11,11 +11,7 @@
 #include "../../include/rt/scene_json.hpp"
 #include "../../include/rt/scenes.hpp"
 #include "../../include/rt_api.h"
-
-namespace rtd {
-void set_error_message(const char* msg); // rt_api.cu
-bool camera_finite(const rt_camera& c); // rt_api.cu
-}
+#include "rt_error.hpp"
 
 namespace {
 
@@ -46,15 +42,11 @@ size_t rt_abi_sizeof(const char* name) {
 }
 
 rt_status rt_orbit_cameras(const rt_camera* base, int32_t n_frames, float degrees, rt_camera* out) {
-    auto fail = [](const char* msg) {
-        rtd::set_error_message((std::string("invalid argument: ") + msg).c_str());
-        return RT_ERR_INVALID_ARG;
-    };
-    if (!base || !out) return fail("base/out is NULL");
-    if (n_frames < 1) return fail("n_frames must be >= 1");
-    if (!std::isfinite(degrees) || !rtd::camera_finite(*base)) return fail("degrees / camera parameter is not finite");
+    ARG_CHECK(base && out, "base/out is NULL");
+    ARG_CHECK(n_frames >= 1, "n_frames must be >= 1");
+    ARG_CHECK(std::isfinite(degrees) && rtd::camera_finite(*base), "degrees / camera parameter is not finite");
     const double ux = base->up[0], uy = base->up[1], uz = base->up[2], ul = std::sqrt(ux * ux + uy * uy + uz * uz);
-    if (!(ul > 0.0)) return fail("camera up is zero");
+    ARG_CHECK(ul > 0.0, "camera up is zero");
     // Rodrigues' rotation of v = lookfrom - lookat about the unit axis a = up / |up|:
     //   v' = v cos(th) + (a x v) sin(th) + a (a . v) (1 - cos(th))
     const double ax = ux / ul, ay = uy / ul, az = uz / ul;

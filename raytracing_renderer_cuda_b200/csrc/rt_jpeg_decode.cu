@@ -219,63 +219,47 @@ int jpeg_resample_kind(int hs, int vs) {
     return RS_GENERIC;
 }
 
-#define JD_TRY(x)                     \
-    do {                              \
-        cudaError_t e_ = (x);         \
-        if (e_ != cudaSuccess) {      \
-            cleanup();                \
-            return e_;                \
-        }                             \
-    } while (0)
-
 cudaError_t jpeg_pixels_device(const rtj::CoefficientImage& img, float* out_dev, cudaStream_t st, float* ms_device) {
-    std::vector<void*> owned;
-    cudaEvent_t ev[2] = {nullptr, nullptr};
-    auto cleanup = [&]() {
-        for (void* p : owned) cudaFreeAsync(p, st);
-        for (auto& e : ev)
-            if (e) cudaEventDestroy(e);
-    };
-    JD_TRY(cudaEventCreate(&ev[0]));
-    JD_TRY(cudaEventCreate(&ev[1]));
+    TimingEvent ev[2];
+    RTD_TRY(ev[0].create());
+    RTD_TRY(ev[1].create());
     RgbParams P{};
     P.width = img.width;
     P.height = img.height;
     P.n_comp = img.n_comp;
     P.is_rgb = img.is_rgb ? 1 : 0;
     std::vector<std::vector<int>> rows(2 * img.n_comp);
-    JD_TRY(cudaEventRecord(ev[0], st));
+    struct Planes {
+        PoolBuffer<int16_t> coeff;
+        PoolBuffer<uint8_t> plane;
+        PoolBuffer<int> near_rows, far_rows;
+    };
+    std::vector<Planes> owned(img.n_comp); // the device copies of each component
+    RTD_TRY(cudaEventRecord(ev[0].ev, st));
     for (int k = 0; k < img.n_comp; ++k) {
         const rtj::Component& c = img.comp[k];
-        int16_t* d_coeff = nullptr;
-        uint8_t* d_plane = nullptr;
-        int *d_near = nullptr, *d_far = nullptr;
-        JD_TRY(rtd::malloc_async(&d_coeff, c.coeff.size() * sizeof(int16_t), st));
-        owned.push_back(d_coeff);
-        JD_TRY(rtd::malloc_async(&d_plane, size_t(c.w2) * c.h2, st));
-        owned.push_back(d_plane);
-        JD_TRY(rtd::malloc_async(&d_near, size_t(img.height) * sizeof(int), st));
-        owned.push_back(d_near);
-        JD_TRY(rtd::malloc_async(&d_far, size_t(img.height) * sizeof(int), st));
-        owned.push_back(d_far);
-        JD_TRY(cudaMemcpyAsync(d_coeff, c.coeff.data(), c.coeff.size() * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+        Planes& o = owned[k];
+        RTD_TRY(o.coeff.alloc(c.coeff.size(), st));
+        RTD_TRY(o.plane.alloc(size_t(c.w2) * c.h2, st));
+        RTD_TRY(o.near_rows.alloc(size_t(img.height), st));
+        RTD_TRY(o.far_rows.alloc(size_t(img.height), st));
+        RTD_TRY(cudaMemcpyAsync(o.coeff.get(), c.coeff.data(), c.coeff.size() * sizeof(int16_t), cudaMemcpyHostToDevice, st));
         jpeg_row_tables(img, k, rows[2 * k], rows[2 * k + 1]);
-        JD_TRY(cudaMemcpyAsync(d_near, rows[2 * k].data(), size_t(img.height) * sizeof(int), cudaMemcpyHostToDevice, st));
-        JD_TRY(cudaMemcpyAsync(d_far, rows[2 * k + 1].data(), size_t(img.height) * sizeof(int), cudaMemcpyHostToDevice, st));
+        RTD_TRY(cudaMemcpyAsync(o.near_rows.get(), rows[2 * k].data(), size_t(img.height) * sizeof(int), cudaMemcpyHostToDevice, st));
+        RTD_TRY(cudaMemcpyAsync(o.far_rows.get(), rows[2 * k + 1].data(), size_t(img.height) * sizeof(int), cudaMemcpyHostToDevice, st));
         DequantTab dq;
         for (int i = 0; i < 64; ++i) dq.q[i] = img.dequant[c.tq][i];
         const int used_w = (c.x + 7) >> 3, used_h = (c.y + 7) >> 3; // the blocks stb transforms (stb:3012-3019)
-        k_jpegd_idct<<<(used_w * used_h + 127) / 128, 128, 0, st>>>(d_coeff, dq, c.blocks_w, used_w, used_h, c.w2, d_plane);
+        k_jpegd_idct<<<(used_w * used_h + 127) / 128, 128, 0, st>>>(o.coeff.get(), dq, c.blocks_w, used_w, used_h, c.w2, o.plane.get());
         const int hs = img.h_max / c.h, vs = img.v_max / c.v;
-        P.c[k] = PlaneView{d_plane, d_near, d_far, c.w2, (img.width + hs - 1) / hs, hs, jpeg_resample_kind(hs, vs)};
+        P.c[k] = PlaneView{o.plane.get(), o.near_rows.get(), o.far_rows.get(), c.w2, (img.width + hs - 1) / hs, hs, jpeg_resample_kind(hs, vs)};
     }
     const size_t npix = size_t(img.width) * img.height;
     k_jpegd_rgb<<<unsigned((npix + 255) / 256), 256, 0, st>>>(P, out_dev);
-    JD_TRY(cudaGetLastError());
-    JD_TRY(cudaEventRecord(ev[1], st));
-    JD_TRY(cudaStreamSynchronize(st)); // the host vectors above are pageable staging buffers
-    if (ms_device) JD_TRY(cudaEventElapsedTime(ms_device, ev[0], ev[1]));
-    cleanup();
+    RTD_TRY(cudaGetLastError());
+    RTD_TRY(cudaEventRecord(ev[1].ev, st));
+    RTD_TRY(cudaStreamSynchronize(st)); // the host vectors above are pageable staging buffers
+    if (ms_device) RTD_TRY(cudaEventElapsedTime(ms_device, ev[0].ev, ev[1].ev));
     return cudaSuccess;
 }
 

@@ -18,6 +18,53 @@ inline cudaError_t malloc_async(T** p, size_t bytes, cudaStream_t st) {
     return malloc_async_bytes(reinterpret_cast<void**>(p), bytes, st);
 }
 
+// Scratch of `count` T from malloc_async, freed on the same stream when the buffer goes out of scope (stream order makes
+// the free wait for the work queued before it, so no exit path needs a synchronisation or a hand-written free).
+template <class T>
+class PoolBuffer {
+  public:
+    PoolBuffer() = default;
+    PoolBuffer(PoolBuffer&& o) noexcept : p_(o.p_), st_(o.st_) { o.p_ = nullptr; }
+    ~PoolBuffer() {
+        if (p_) cudaFreeAsync(p_, st_);
+    }
+    cudaError_t alloc(size_t count, cudaStream_t st) { // on an empty buffer
+        st_ = st;
+        const cudaError_t e = malloc_async(&p_, count * sizeof(T), st);
+        if (e != cudaSuccess) p_ = nullptr;
+        return e;
+    }
+    T* get() const { return p_; }
+    T* release() { // the caller frees the memory from now on
+        T* p = p_;
+        p_ = nullptr;
+        return p;
+    }
+
+  private:
+    T* p_ = nullptr;
+    cudaStream_t st_ = nullptr;
+};
+
+// A timing event destroyed when it goes out of scope
+struct TimingEvent {
+    cudaEvent_t ev = nullptr;
+    TimingEvent() = default;
+    TimingEvent(const TimingEvent&) = delete;
+    TimingEvent& operator=(const TimingEvent&) = delete;
+    ~TimingEvent() {
+        if (ev) cudaEventDestroy(ev);
+    }
+    cudaError_t create() { return cudaEventCreate(&ev); }
+};
+
+// returns a failing cudaError_t from a function that returns one (its PoolBuffers and TimingEvents release themselves)
+#define RTD_TRY(expr)                          \
+    do {                                       \
+        const cudaError_t e__ = (expr);        \
+        if (e__ != cudaSuccess) return e__;    \
+    } while (0)
+
 // parity hook: closest hit for caller-supplied rays
 void launch_trace_primary(const DScene& sc, const rt_ray* rays_dev, size_t n, float tmin, int use_bvh, // 0 list, 1 BVH, 2 4-wide BVH
                           rt_hit* hits_dev, cudaStream_t st);

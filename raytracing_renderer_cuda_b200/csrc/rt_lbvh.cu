@@ -378,18 +378,17 @@ cudaError_t bvh_nodes_ch(const BvhNode* nodes, uint32_t n, BvhNodeCH* out, cudaS
 cudaError_t bvh_quantize4(const BvhNode4* nodes4, uint32_t n4, BvhNode4Q* out_q, bool* quant_ok, cudaStream_t st) {
     *quant_ok = false;
     if (n4 == 0 || !out_q) return cudaSuccess;
-    uint32_t* bad = nullptr;
-    cudaError_t e = rtd::malloc_async(&bad, sizeof(uint32_t), st);
+    PoolBuffer<uint32_t> bad;
+    cudaError_t e = bad.alloc(1, st);
     if (e != cudaSuccess) return e;
-    e = cudaMemsetAsync(bad, 0, sizeof(uint32_t), st);
+    e = cudaMemsetAsync(bad.get(), 0, sizeof(uint32_t), st);
     if (e == cudaSuccess) {
-        k_quantize4<<<(n4 + 255) / 256, 256, 0, st>>>(nodes4, n4, out_q, bad);
+        k_quantize4<<<(n4 + 255) / 256, 256, 0, st>>>(nodes4, n4, out_q, bad.get());
         e = cudaGetLastError();
     }
     uint32_t h = 1u;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&h, bad, sizeof h, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&h, bad.get(), sizeof h, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaFreeAsync(bad, st);
     *quant_ok = e == cudaSuccess && h == 0u;
     return e;
 }
@@ -402,125 +401,88 @@ cudaError_t bvh_collapse4(const BvhNode* nodes, uint32_t n_nodes, uint32_t root,
     *n_out = 0;
     *root_out = 0;
     if (n_nodes == 0) return cudaSuccess;
-    BvhNode4* wide = nullptr;
-    uint32_t *level = nullptr, *used = nullptr, *idx = nullptr;
-    void* tmp = nullptr;
-    size_t tmp_bytes = 0;
-    auto cleanup = [&]() {
-        void* all[] = {wide, level, used, idx, tmp};
-        for (void* p : all)
-            if (p) cudaFreeAsync(p, st);
-    };
-#define C4_TRY(x)               \
-    do {                        \
-        cudaError_t e_ = (x);   \
-        if (e_ != cudaSuccess) { \
-            cleanup();          \
-            return e_;          \
-        }                       \
-    } while (0)
-    C4_TRY(rtd::malloc_async(&wide, size_t(n_nodes) * sizeof(BvhNode4), st));
-    C4_TRY(rtd::malloc_async(&level, size_t(n_nodes + 1) * sizeof(uint32_t), st));
-    C4_TRY(rtd::malloc_async(&used, size_t(n_nodes + 1) * sizeof(uint32_t), st));
-    C4_TRY(rtd::malloc_async(&idx, size_t(n_nodes + 1) * sizeof(uint32_t), st));
-    tmp_bytes = prims::scan_scratch_elems(size_t(n_nodes) + 1) * sizeof(uint32_t);
-    C4_TRY(rtd::malloc_async(&tmp, tmp_bytes, st));
+    PoolBuffer<BvhNode4> wide;
+    PoolBuffer<uint32_t> level, used, idx, tmp;
+    RTD_TRY(wide.alloc(n_nodes, st));
+    RTD_TRY(level.alloc(size_t(n_nodes) + 1, st));
+    RTD_TRY(used.alloc(size_t(n_nodes) + 1, st));
+    RTD_TRY(idx.alloc(size_t(n_nodes) + 1, st));
+    RTD_TRY(tmp.alloc(prims::scan_scratch_elems(size_t(n_nodes) + 1), st));
     const unsigned blocks = (n_nodes + 255) / 256;
-    k_collapse4<<<blocks, 256, 0, st>>>(nodes, n_nodes, wide);
-    C4_TRY(cudaMemsetAsync(level, 0, size_t(n_nodes + 1) * sizeof(uint32_t), st));
+    k_collapse4<<<blocks, 256, 0, st>>>(nodes, n_nodes, wide.get());
+    RTD_TRY(cudaMemsetAsync(level.get(), 0, size_t(n_nodes + 1) * sizeof(uint32_t), st));
     const uint32_t one = 1u;
-    C4_TRY(cudaMemcpyAsync(level + root, &one, sizeof one, cudaMemcpyHostToDevice, st));
-    for (uint32_t cur = 1; cur <= depth / 2 + 2; ++cur) k_mark4<<<blocks, 256, 0, st>>>(wide, n_nodes, level, cur);
-    k_used4<<<(n_nodes + 256) / 256, 256, 0, st>>>(level, n_nodes + 1, used); // level[n_nodes] == 0: the scan's total slot
-    C4_TRY(prims::exclusive_sum<uint32_t>(used, idx, size_t(n_nodes) + 1, static_cast<uint32_t*>(tmp), st));
-    k_compact4<<<blocks, 256, 0, st>>>(wide, level, idx, n_nodes, out);
-    C4_TRY(cudaGetLastError());
+    RTD_TRY(cudaMemcpyAsync(level.get() + root, &one, sizeof one, cudaMemcpyHostToDevice, st));
+    for (uint32_t cur = 1; cur <= depth / 2 + 2; ++cur) k_mark4<<<blocks, 256, 0, st>>>(wide.get(), n_nodes, level.get(), cur);
+    k_used4<<<(n_nodes + 256) / 256, 256, 0, st>>>(level.get(), n_nodes + 1, used.get()); // level[n_nodes] == 0: the scan's total slot
+    RTD_TRY(prims::exclusive_sum<uint32_t>(used.get(), idx.get(), size_t(n_nodes) + 1, tmp.get(), st));
+    k_compact4<<<blocks, 256, 0, st>>>(wide.get(), level.get(), idx.get(), n_nodes, out);
+    RTD_TRY(cudaGetLastError());
     uint32_t h[2] = {0, 0};
-    C4_TRY(cudaMemcpyAsync(&h[0], idx + n_nodes, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    C4_TRY(cudaMemcpyAsync(&h[1], idx + root, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    C4_TRY(cudaStreamSynchronize(st));
-#undef C4_TRY
+    RTD_TRY(cudaMemcpyAsync(&h[0], idx.get() + n_nodes, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    RTD_TRY(cudaMemcpyAsync(&h[1], idx.get() + root, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    RTD_TRY(cudaStreamSynchronize(st));
     *n_out = h[0];
     *root_out = h[1];
-    cleanup();
     return cudaSuccess;
 }
 
+// The scratch is stream-ordered pool memory (the context keeps freed blocks): no device-wide synchronisation per scene build.
 cudaError_t lbvh_build(const float4* sph_a, const float4* sph_b, uint32_t n_static, const uint32_t* ids, uint32_t n,
                        BvhNode* nodes, cudaStream_t st, float* ms, uint32_t* depth, float root_box[6]) {
     if (n < 2) return cudaErrorInvalidValue;
-    cudaError_t e;
-    float4 *lo = nullptr, *hi = nullptr;
-    unsigned long long *keys = nullptr, *keys_out = nullptr;
-    uint32_t *vals = nullptr, *vals_out = nullptr;
-    int *parent_inner = nullptr, *parent_leaf = nullptr;
-    unsigned *visits = nullptr, *scal = nullptr; // scal: [0..5] centroid bounds, [6] depth, [8..13] root box
-    void* tmp = nullptr;
-    size_t tmp_bytes = 0;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    auto cleanup = [&]() {
-        // stream-ordered pool (the context keeps freed blocks): no device-wide synchronisation per scene build
-        void* all[] = {lo, hi, keys, keys_out, vals, vals_out, parent_inner, parent_leaf, visits, scal, tmp};
-        for (void* p : all)
-            if (p) cudaFreeAsync(p, st);
-        if (e0) cudaEventDestroy(e0);
-        if (e1) cudaEventDestroy(e1);
-    };
-#define LB_TRY(x)              \
-    do {                       \
-        e = (x);               \
-        if (e != cudaSuccess) { \
-            cleanup();         \
-            return e;          \
-        }                      \
-    } while (0)
-    LB_TRY(rtd::malloc_async(&lo, n * sizeof(float4), st));
-    LB_TRY(rtd::malloc_async(&hi, n * sizeof(float4), st));
-    LB_TRY(rtd::malloc_async(&keys, n * sizeof(unsigned long long), st));
-    LB_TRY(rtd::malloc_async(&keys_out, n * sizeof(unsigned long long), st));
-    LB_TRY(rtd::malloc_async(&vals, n * sizeof(uint32_t), st));
-    LB_TRY(rtd::malloc_async(&vals_out, n * sizeof(uint32_t), st));
-    LB_TRY(rtd::malloc_async(&parent_inner, n * sizeof(int), st));
-    LB_TRY(rtd::malloc_async(&parent_leaf, n * sizeof(int), st));
-    LB_TRY(rtd::malloc_async(&visits, n * sizeof(unsigned), st));
-    LB_TRY(rtd::malloc_async(&scal, 16 * sizeof(unsigned), st));
-    tmp_bytes = prims::sort_scratch_elems(n) * sizeof(uint32_t);
-    LB_TRY(rtd::malloc_async(&tmp, tmp_bytes, st));
-    LB_TRY(cudaEventCreate(&e0));
-    LB_TRY(cudaEventCreate(&e1));
+    PoolBuffer<float4> lo, hi;
+    PoolBuffer<unsigned long long> keys_a, keys_b;
+    PoolBuffer<uint32_t> vals_a, vals_b, tmp;
+    PoolBuffer<int> parent_inner, parent_leaf;
+    PoolBuffer<unsigned> visits, scal; // scal: [0..5] centroid bounds, [6] depth, [8..13] root box
+    TimingEvent e0, e1;
+    RTD_TRY(lo.alloc(n, st));
+    RTD_TRY(hi.alloc(n, st));
+    RTD_TRY(keys_a.alloc(n, st));
+    RTD_TRY(keys_b.alloc(n, st));
+    RTD_TRY(vals_a.alloc(n, st));
+    RTD_TRY(vals_b.alloc(n, st));
+    RTD_TRY(parent_inner.alloc(n, st));
+    RTD_TRY(parent_leaf.alloc(n, st));
+    RTD_TRY(visits.alloc(n, st));
+    RTD_TRY(scal.alloc(16, st));
+    RTD_TRY(tmp.alloc(prims::sort_scratch_elems(n), st));
+    RTD_TRY(e0.create());
+    RTD_TRY(e1.create());
 
     const unsigned init[8] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u, 0u, 0u};
-    LB_TRY(cudaMemcpyAsync(scal, init, sizeof init, cudaMemcpyHostToDevice, st));
-    LB_TRY(cudaEventRecord(e0, st));
-    LB_TRY(cudaMemsetAsync(visits, 0, n * sizeof(unsigned), st));
+    RTD_TRY(cudaMemcpyAsync(scal.get(), init, sizeof init, cudaMemcpyHostToDevice, st));
+    RTD_TRY(cudaEventRecord(e0.ev, st));
+    RTD_TRY(cudaMemsetAsync(visits.get(), 0, n * sizeof(unsigned), st));
     const unsigned blocks = (n + 255) / 256;
-    k_prim_boxes<<<blocks, 256, 0, st>>>(sph_a, sph_b, ids, n, n_static, lo, hi, scal);
-    k_morton<<<blocks, 256, 0, st>>>(lo, hi, n, scal, keys, vals);
+    unsigned long long *keys = keys_a.get(), *keys_out = keys_b.get();
+    uint32_t *vals = vals_a.get(), *vals_out = vals_b.get();
+    k_prim_boxes<<<blocks, 256, 0, st>>>(sph_a, sph_b, ids, n, n_static, lo.get(), hi.get(), scal.get());
+    k_morton<<<blocks, 256, 0, st>>>(lo.get(), hi.get(), n, scal.get(), keys, vals);
     { // stable LSD radix sort of the (63-bit Morton code, primitive) pairs: 8 passes of 8 bits (rt_prims.cuh)
         bool in_alt = false;
-        LB_TRY(prims::sort_pairs_u64_u32(keys, vals, keys_out, vals_out, n, 8, static_cast<uint32_t*>(tmp), &in_alt, st));
+        RTD_TRY(prims::sort_pairs_u64_u32(keys, vals, keys_out, vals_out, n, 8, tmp.get(), &in_alt, st));
         if (!in_alt) { // the sorted pairs are in (keys, vals): the code below reads (keys_out, vals_out)
             std::swap(keys, keys_out);
             std::swap(vals, vals_out);
         }
     }
-    k_topology<<<blocks, 256, 0, st>>>(keys_out, vals_out, ids, int(n), nodes, parent_inner, parent_leaf);
-    k_refit<<<blocks, 256, 0, st>>>(vals_out, ids, int(n), lo, hi, nodes, parent_inner, parent_leaf, visits,
-                                    reinterpret_cast<float*>(scal + 8));
-    k_depth<<<blocks, 256, 0, st>>>(int(n), parent_inner, parent_leaf, scal + 6);
-    LB_TRY(cudaEventRecord(e1, st));
-    LB_TRY(cudaGetLastError());
+    k_topology<<<blocks, 256, 0, st>>>(keys_out, vals_out, ids, int(n), nodes, parent_inner.get(), parent_leaf.get());
+    k_refit<<<blocks, 256, 0, st>>>(vals_out, ids, int(n), lo.get(), hi.get(), nodes, parent_inner.get(), parent_leaf.get(),
+                                    visits.get(), reinterpret_cast<float*>(scal.get() + 8));
+    k_depth<<<blocks, 256, 0, st>>>(int(n), parent_inner.get(), parent_leaf.get(), scal.get() + 6);
+    RTD_TRY(cudaEventRecord(e1.ev, st));
+    RTD_TRY(cudaGetLastError());
     unsigned d = 0;
     float rb[6] = {0, 0, 0, 0, 0, 0};
-    LB_TRY(cudaMemcpyAsync(&d, scal + 6, sizeof d, cudaMemcpyDeviceToHost, st));
-    LB_TRY(cudaMemcpyAsync(rb, scal + 8, sizeof rb, cudaMemcpyDeviceToHost, st));
-    LB_TRY(cudaStreamSynchronize(st));
+    RTD_TRY(cudaMemcpyAsync(&d, scal.get() + 6, sizeof d, cudaMemcpyDeviceToHost, st));
+    RTD_TRY(cudaMemcpyAsync(rb, scal.get() + 8, sizeof rb, cudaMemcpyDeviceToHost, st));
+    RTD_TRY(cudaStreamSynchronize(st));
     if (root_box)
         for (int k = 0; k < 6; ++k) root_box[k] = rb[k];
-    if (ms) LB_TRY(cudaEventElapsedTime(ms, e0, e1));
+    if (ms) RTD_TRY(cudaEventElapsedTime(ms, e0.ev, e1.ev));
     if (depth) *depth = d;
-#undef LB_TRY
-    cleanup();
     return cudaSuccess;
 }
 

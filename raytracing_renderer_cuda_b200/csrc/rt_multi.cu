@@ -14,8 +14,6 @@
 //                cudaDeviceEnablePeerAccess, one host thread per device for the render, CUDA events for the cross-device ordering.
 #include <atomic>
 #include <chrono>
-#include <cstdarg>
-#include <cstdio>
 #include <cstring>
 #include <string>
 #include <thread>
@@ -24,39 +22,6 @@
 #include "rt_internal.hpp"
 
 namespace {
-
-void fail(const char* fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    rtd::set_error_message(buf);
-}
-#define M_TRY(expr)                                                                      \
-    do {                                                                                 \
-        cudaError_t e__ = (expr);                                                        \
-        if (e__ != cudaSuccess) {                                                        \
-            fail("%s:%d: %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(e__)); \
-            return e__ == cudaErrorMemoryAllocation ? RT_ERR_OOM : RT_ERR_CUDA;          \
-        }                                                                                \
-    } while (0)
-#define M_ARG(cond, msg)                            \
-    do {                                            \
-        if (!(cond)) {                              \
-            fail("invalid argument: %s", msg);      \
-            return RT_ERR_INVALID_ARG;              \
-        }                                           \
-    } while (0)
-#define M_CATCH                                         \
-    catch (const std::bad_alloc&) {                     \
-        fail("out of host memory");                     \
-        return RT_ERR_OOM;                              \
-    }                                                   \
-    catch (const std::exception& e) {                   \
-        fail("unexpected exception: %s", e.what());     \
-        return RT_ERR_INVALID_ARG;                      \
-    }
 
 constexpr int kMaxRanks = 16;     // PeerPtrs of k_reduce_tonemap
 constexpr size_t kFlagBytes = 256; // kMaxRanks epoch words + the time-out flag, in their own 256-byte tail of the accumulator
@@ -92,8 +57,8 @@ __global__ void k_group_barrier(const __grid_constant__ PeerFlags peers, int ran
 
 // ------------------------------------------------------------------------------------------------ sharding ----
 extern "C" rt_status rt_shard_samples(int32_t spp_total, int32_t rank, int32_t world, int32_t* first, int32_t* count) {
-    M_ARG(world >= 1 && rank >= 0 && rank < world && spp_total >= 0, "bad rank / world / spp_total");
-    M_ARG(first && count, "first/count is NULL");
+    ARG_CHECK(world >= 1 && rank >= 0 && rank < world && spp_total >= 0, "bad rank / world / spp_total");
+    ARG_CHECK(first && count, "first/count is NULL");
     const int32_t base = spp_total / world, rem = spp_total % world;
     *count = base + (rank < rem ? 1 : 0);
     *first = rank * base + (rank < rem ? rank : rem);
@@ -101,8 +66,8 @@ extern "C" rt_status rt_shard_samples(int32_t spp_total, int32_t rank, int32_t w
 }
 
 extern "C" rt_status rt_shard_rows(int32_t height, int32_t rank, int32_t world, int32_t* row_begin, int32_t* row_end) {
-    M_ARG(world >= 1 && rank >= 0 && rank < world && height >= 0, "bad rank / world / height");
-    M_ARG(row_begin && row_end, "row_begin/row_end is NULL");
+    ARG_CHECK(world >= 1 && rank >= 0 && rank < world && height >= 0, "bad rank / world / height");
+    ARG_CHECK(row_begin && row_end, "row_begin/row_end is NULL");
     *row_begin = int32_t(int64_t(rank) * height / world);
     *row_end = int32_t(int64_t(rank + 1) * height / world);
     return RT_OK;
@@ -142,17 +107,17 @@ rt_status group_barrier(rt_group* g) {
     ++g->epoch;
     // ~64 ns per poll: 2^27 polls are several seconds, far beyond any frame's skew between ranks
     k_group_barrier<<<1, 32, 0, g->ctx->stream>>>(pf, g->rank, g->world, g->epoch, 1ull << 27);
-    M_TRY(cudaGetLastError());
+    CUDA_TRY(cudaGetLastError());
     return RT_OK;
 }
 } // namespace
 
 extern "C" rt_status rt_group_create(rt_context* ctx, int32_t rank, int32_t world, int32_t width, int32_t height, rt_group** out) try {
-    M_ARG(ctx && out, "ctx/out is NULL");
+    ARG_CHECK(ctx && out, "ctx/out is NULL");
     *out = nullptr;
-    M_ARG(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world, "rank/world out of range (at most 16 ranks)");
-    M_ARG(width > 0 && height > 0 && uint64_t(width) * uint64_t(height) < (1ull << 31), "bad frame size");
-    M_TRY(cudaSetDevice(ctx->device));
+    ARG_CHECK(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world, "rank/world out of range (at most 16 ranks)");
+    ARG_CHECK(width > 0 && height > 0 && uint64_t(width) * uint64_t(height) < (1ull << 31), "bad frame size");
+    CUDA_TRY(cudaSetDevice(ctx->device));
     rt_group* g = new rt_group();
     g->ctx = ctx;
     g->rank = rank;
@@ -161,11 +126,11 @@ extern "C" rt_status rt_group_create(rt_context* ctx, int32_t rank, int32_t worl
     g->height = height;
     const rt_status st = [&]() -> rt_status {
         const size_t ab = accum_bytes(width, height);
-        M_TRY(cudaMalloc(&g->accum, ab + kFlagBytes)); // cudaMalloc, not the pool: IPC-exportable
-        M_TRY(cudaMemsetAsync(g->accum, 0, ab + kFlagBytes, ctx->stream));
-        if (rank == 0) M_TRY(cudaMalloc(&g->image, size_t(width) * height * (3 * sizeof(float) + 3)));
-        for (auto& e : g->ev) M_TRY(cudaEventCreate(&e));
-        M_TRY(cudaStreamSynchronize(ctx->stream));
+        CUDA_TRY(cudaMalloc(&g->accum, ab + kFlagBytes)); // cudaMalloc, not the pool: IPC-exportable
+        CUDA_TRY(cudaMemsetAsync(g->accum, 0, ab + kFlagBytes, ctx->stream));
+        if (rank == 0) CUDA_TRY(cudaMalloc(&g->image, size_t(width) * height * (3 * sizeof(float) + 3)));
+        for (auto& e : g->ev) CUDA_TRY(cudaEventCreate(&e));
+        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         g->peer_accum[rank] = g->accum;
         if (rank == 0) g->root_image = g->image;
         if (world == 1) g->connected = true;
@@ -178,11 +143,11 @@ extern "C" rt_status rt_group_create(rt_context* ctx, int32_t rank, int32_t worl
     *out = g;
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_group_export(const rt_group* g, void* handle) try {
-    M_ARG(g && handle, "group/handle is NULL");
-    M_TRY(cudaSetDevice(g->ctx->device));
+    ARG_CHECK(g && handle, "group/handle is NULL");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
     GroupHandle h{};
     h.magic = kMagic;
     h.rank = uint32_t(g->rank);
@@ -191,101 +156,101 @@ extern "C" rt_status rt_group_export(const rt_group* g, void* handle) try {
     h.width = g->width;
     h.height = g->height;
     h.has_image = g->image ? 1u : 0u;
-    M_TRY(cudaIpcGetMemHandle(&h.accum, g->accum));
-    if (g->image) M_TRY(cudaIpcGetMemHandle(&h.image, g->image));
+    CUDA_TRY(cudaIpcGetMemHandle(&h.accum, g->accum));
+    if (g->image) CUDA_TRY(cudaIpcGetMemHandle(&h.image, g->image));
     memset(handle, 0, RT_GROUP_HANDLE_BYTES);
     memcpy(handle, &h, sizeof h);
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_group_connect(rt_group* g, const void* handles) try {
-    M_ARG(g && handles, "group/handles is NULL");
-    M_ARG(!g->connected || g->world == 1, "group is already connected");
-    M_TRY(cudaSetDevice(g->ctx->device));
+    ARG_CHECK(g && handles, "group/handles is NULL");
+    ARG_CHECK(!g->connected || g->world == 1, "group is already connected");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
     const char* base = static_cast<const char*>(handles);
     for (int r = 0; r < g->world; ++r) {
         GroupHandle h;
         memcpy(&h, base + size_t(r) * RT_GROUP_HANDLE_BYTES, sizeof h);
-        M_ARG(h.magic == kMagic && int32_t(h.rank) == r && int32_t(h.world) == g->world, "handle table is not in rank order / from another group");
-        M_ARG(h.width == g->width && h.height == g->height, "ranks disagree about the frame size");
+        ARG_CHECK(h.magic == kMagic && int32_t(h.rank) == r && int32_t(h.world) == g->world, "handle table is not in rank order / from another group");
+        ARG_CHECK(h.width == g->width && h.height == g->height, "ranks disagree about the frame size");
         if (r != g->rank) {
-            M_TRY(cudaIpcOpenMemHandle(&g->peer_accum[r], h.accum, cudaIpcMemLazyEnablePeerAccess));
+            CUDA_TRY(cudaIpcOpenMemHandle(&g->peer_accum[r], h.accum, cudaIpcMemLazyEnablePeerAccess));
             g->opened[r] = true;
         }
         if (r == 0 && g->rank != 0) {
-            M_ARG(h.has_image != 0u, "rank 0 exported no image");
-            M_TRY(cudaIpcOpenMemHandle(&g->root_image, h.image, cudaIpcMemLazyEnablePeerAccess));
+            ARG_CHECK(h.has_image != 0u, "rank 0 exported no image");
+            CUDA_TRY(cudaIpcOpenMemHandle(&g->root_image, h.image, cudaIpcMemLazyEnablePeerAccess));
             g->opened_image = true;
         }
     }
     g->connected = true;
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" void* rt_group_accum(const rt_group* g) { return g ? g->accum : nullptr; }
 
 extern "C" rt_status rt_group_begin_frame(rt_group* g) try {
-    M_ARG(g && g->connected, "group is NULL / not connected");
-    M_TRY(cudaSetDevice(g->ctx->device));
+    ARG_CHECK(g && g->connected, "group is NULL / not connected");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
     // (ordered after the closing barrier of the previous frame: no peer still reads this accumulator)
-    M_TRY(cudaMemsetAsync(g->accum, 0, size_t(g->width) * g->height * sizeof(float4), g->ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(g->accum, 0, size_t(g->width) * g->height * sizeof(float4), g->ctx->stream));
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_group_finish_frame(rt_group* g, int32_t want_rgb8, float* ms_reduce) try {
-    M_ARG(g && g->connected, "group is NULL / not connected");
-    M_TRY(cudaSetDevice(g->ctx->device));
+    ARG_CHECK(g && g->connected, "group is NULL / not connected");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
     cudaStream_t st = g->ctx->stream;
     rt_status s = RT_OK;
-    if (ms_reduce) M_TRY(cudaEventRecord(g->ev[0], st));
+    if (ms_reduce) CUDA_TRY(cudaEventRecord(g->ev[0], st));
     if (g->world > 1 && (s = group_barrier(g)) != RT_OK) return s; // every rank's accumulator is complete
     int32_t r0 = 0, r1 = 0;
     rt_shard_rows(g->height, g->rank, g->world, &r0, &r1);
     rtd::launch_reduce_tonemap(g->peer_accum, g->world, nullptr, g->width, g->height, r0, r1, image_rgb(g->root_image),
                                want_rgb8 ? image_rgb8(g->root_image, g->width, g->height) : nullptr, nullptr, g->ctx->sm_count, st);
-    M_TRY(cudaGetLastError());
+    CUDA_TRY(cudaGetLastError());
     if (g->world > 1 && (s = group_barrier(g)) != RT_OK) return s; // every band is in the root's image; accumulators are free again
     if (ms_reduce) {
-        M_TRY(cudaEventRecord(g->ev[1], st));
-        M_TRY(cudaEventSynchronize(g->ev[1]));
-        M_TRY(cudaEventElapsedTime(ms_reduce, g->ev[0], g->ev[1]));
+        CUDA_TRY(cudaEventRecord(g->ev[1], st));
+        CUDA_TRY(cudaEventSynchronize(g->ev[1]));
+        CUDA_TRY(cudaEventElapsedTime(ms_reduce, g->ev[0], g->ev[1]));
     }
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_group_read_frame(rt_group* g, float* out_rgb, uint8_t* out_rgb8) try {
-    M_ARG(g && g->connected, "group is NULL / not connected");
-    M_TRY(cudaSetDevice(g->ctx->device));
+    ARG_CHECK(g && g->connected, "group is NULL / not connected");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
     cudaStream_t st = g->ctx->stream;
     const size_t npix = size_t(g->width) * g->height;
     if (g->rank == 0) {
-        if (out_rgb) M_TRY(cudaMemcpyAsync(out_rgb, image_rgb(g->image), npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (out_rgb8) M_TRY(cudaMemcpyAsync(out_rgb8, image_rgb8(g->image, g->width, g->height), npix * 3, cudaMemcpyDeviceToHost, st));
+        if (out_rgb) CUDA_TRY(cudaMemcpyAsync(out_rgb, image_rgb(g->image), npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (out_rgb8) CUDA_TRY(cudaMemcpyAsync(out_rgb8, image_rgb8(g->image, g->width, g->height), npix * 3, cudaMemcpyDeviceToHost, st));
     }
     uint32_t timed_out = 0;
-    M_TRY(cudaMemcpyAsync(&timed_out, static_cast<char*>(g->accum) + accum_bytes(g->width, g->height) + kMaxRanks * sizeof(uint32_t),
+    CUDA_TRY(cudaMemcpyAsync(&timed_out, static_cast<char*>(g->accum) + accum_bytes(g->width, g->height) + kMaxRanks * sizeof(uint32_t),
                           sizeof timed_out, cudaMemcpyDeviceToHost, st));
-    M_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     if (timed_out) {
-        fail("rt_group: a peer never reached the barrier (rank %d gave up waiting)", g->rank);
+        rtd::set_error("rt_group: a peer never reached the barrier (rank %d gave up waiting)", g->rank);
         return RT_ERR_CUDA;
     }
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_group_read_accum(rt_group* g, float* out_accum) try {
-    M_ARG(g && out_accum, "group/out is NULL");
-    M_TRY(cudaSetDevice(g->ctx->device));
-    M_TRY(cudaMemcpyAsync(out_accum, g->accum, size_t(g->width) * g->height * sizeof(float4), cudaMemcpyDeviceToHost, g->ctx->stream));
-    M_TRY(cudaStreamSynchronize(g->ctx->stream));
+    ARG_CHECK(g && out_accum, "group/out is NULL");
+    CUDA_TRY(cudaSetDevice(g->ctx->device));
+    CUDA_TRY(cudaMemcpyAsync(out_accum, g->accum, size_t(g->width) * g->height * sizeof(float4), cudaMemcpyDeviceToHost, g->ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(g->ctx->stream));
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" void rt_group_destroy(rt_group* g) {
     if (!g) return;
@@ -315,39 +280,39 @@ struct rt_multi {
 };
 
 extern "C" rt_status rt_multi_create(const int32_t* devices, int32_t n_devices, rt_multi** out) try {
-    M_ARG(out, "out is NULL");
+    ARG_CHECK(out, "out is NULL");
     *out = nullptr;
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
         cudaGetLastError();
-        fail("no CUDA device available; this library has no CPU fallback");
+        rtd::set_error("no CUDA device available; this library has no CPU fallback");
         return RT_ERR_NO_DEVICE;
     }
     if (n_devices <= 0) n_devices = count; // all of them
-    M_ARG(n_devices <= kMaxRanks && n_devices <= count, "more devices requested than present (or than 16)");
+    ARG_CHECK(n_devices <= kMaxRanks && n_devices <= count, "more devices requested than present (or than 16)");
     rt_multi* m = new rt_multi();
     m->n = n_devices;
     const rt_status st = [&]() -> rt_status {
         for (int k = 0; k < n_devices; ++k) {
             const int dev = devices ? devices[k] : k;
-            for (int j = 0; j < k; ++j) M_ARG(m->ctx[j]->device != dev, "device listed twice");
+            for (int j = 0; j < k; ++j) ARG_CHECK(m->ctx[j]->device != dev, "device listed twice");
             rt_context* c = nullptr;
             const rt_status s = rt_context_create(dev, &c);
             if (s != RT_OK) return s;
             m->ctx.push_back(c);
         }
         for (int a = 0; a < n_devices; ++a) { // every device reads every other device's accumulator; all write device 0's image
-            M_TRY(cudaSetDevice(m->ctx[a]->device));
+            CUDA_TRY(cudaSetDevice(m->ctx[a]->device));
             for (int b = 0; b < n_devices; ++b) {
                 if (a == b) continue;
                 int can = 0;
-                M_TRY(cudaDeviceCanAccessPeer(&can, m->ctx[a]->device, m->ctx[b]->device));
+                CUDA_TRY(cudaDeviceCanAccessPeer(&can, m->ctx[a]->device, m->ctx[b]->device));
                 if (!can) {
-                    fail("device %d cannot access device %d's memory (no NVLink / P2P path)", m->ctx[a]->device, m->ctx[b]->device);
+                    rtd::set_error("device %d cannot access device %d's memory (no NVLink / P2P path)", m->ctx[a]->device, m->ctx[b]->device);
                     return RT_ERR_UNSUPPORTED;
                 }
                 const cudaError_t e = cudaDeviceEnablePeerAccess(m->ctx[b]->device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) M_TRY(e);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) CUDA_TRY(e);
                 cudaGetLastError();
             }
         }
@@ -356,12 +321,12 @@ extern "C" rt_status rt_multi_create(const int32_t* devices, int32_t n_devices, 
         m->ev_done.assign(n_devices, nullptr);
         m->ev_red.assign(n_devices, nullptr);
         for (int k = 0; k < n_devices; ++k) {
-            M_TRY(cudaSetDevice(m->ctx[k]->device));
-            M_TRY(cudaEventCreateWithFlags(&m->ev_done[k], cudaEventDisableTiming));
-            M_TRY(cudaEventCreateWithFlags(&m->ev_red[k], cudaEventDisableTiming));
+            CUDA_TRY(cudaSetDevice(m->ctx[k]->device));
+            CUDA_TRY(cudaEventCreateWithFlags(&m->ev_done[k], cudaEventDisableTiming));
+            CUDA_TRY(cudaEventCreateWithFlags(&m->ev_red[k], cudaEventDisableTiming));
         }
-        M_TRY(cudaSetDevice(m->ctx[0]->device));
-        for (auto& e : m->ev_t) M_TRY(cudaEventCreate(&e));
+        CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
+        for (auto& e : m->ev_t) CUDA_TRY(cudaEventCreate(&e));
         return RT_OK;
     }();
     if (st != RT_OK) {
@@ -371,12 +336,12 @@ extern "C" rt_status rt_multi_create(const int32_t* devices, int32_t n_devices, 
     *out = m;
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" int32_t rt_multi_size(const rt_multi* m) { return m ? m->n : 0; }
 
 extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) try {
-    M_ARG(m && desc, "multi/desc is NULL");
+    ARG_CHECK(m && desc, "multi/desc is NULL");
     std::vector<rt_status> st(m->n, RT_OK);
     std::vector<std::string> msg(m->n);
     std::vector<std::thread> th;
@@ -390,34 +355,34 @@ extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) 
     for (auto& t : th) t.join();
     for (int k = 0; k < m->n; ++k)
         if (st[k] != RT_OK) {
-            fail("device %d: %s", m->ctx[k]->device, msg[k].c_str());
+            rtd::set_error("device %d: %s", m->ctx[k]->device, msg[k].c_str());
             return st[k];
         }
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_multi_render(rt_multi* m, const rt_render_params* p, float* out_rgb, uint8_t* out_rgb8, rt_stats* stats,
                                      float* ms_reduce) try {
-    M_ARG(m && p, "multi/params is NULL");
-    M_ARG(out_rgb || out_rgb8, "no output buffer");
-    M_ARG(p->width > 0 && p->height > 0 && uint64_t(p->width) * uint64_t(p->height) < (1ull << 31), "bad frame size");
-    for (int k = 0; k < m->n; ++k) M_ARG(m->scene[k] != nullptr, "no scene: call rt_multi_set_scene first");
+    ARG_CHECK(m && p, "multi/params is NULL");
+    ARG_CHECK(out_rgb || out_rgb8, "no output buffer");
+    ARG_CHECK(p->width > 0 && p->height > 0 && uint64_t(p->width) * uint64_t(p->height) < (1ull << 31), "bad frame size");
+    for (int k = 0; k < m->n; ++k) ARG_CHECK(m->scene[k] != nullptr, "no scene: call rt_multi_set_scene first");
     const size_t npix = size_t(p->width) * p->height;
     if (m->accum_px < npix) {
         for (int k = 0; k < m->n; ++k) {
-            M_TRY(cudaSetDevice(m->ctx[k]->device));
+            CUDA_TRY(cudaSetDevice(m->ctx[k]->device));
             if (m->accum[k]) cudaFree(m->accum[k]);
             m->accum[k] = nullptr;
-            M_TRY(cudaMalloc(&m->accum[k], npix * sizeof(float4)));
+            CUDA_TRY(cudaMalloc(&m->accum[k], npix * sizeof(float4)));
         }
         m->accum_px = npix;
     }
     if (m->image_px < npix) {
-        M_TRY(cudaSetDevice(m->ctx[0]->device));
+        CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
         if (m->image) cudaFree(m->image);
         m->image = nullptr;
-        M_TRY(cudaMalloc(&m->image, npix * (3 * sizeof(float) + 3)));
+        CUDA_TRY(cudaMalloc(&m->image, npix * (3 * sizeof(float) + 3)));
         m->image_px = npix;
     }
     // ---- render: one host thread per device (the wavefront loop polls its queue counters) ----
@@ -443,36 +408,36 @@ extern "C" rt_status rt_multi_render(rt_multi* m, const rt_render_params* p, flo
     for (auto& t : th) t.join();
     for (int k = 0; k < m->n; ++k)
         if (st[k] != RT_OK) {
-            fail("device %d: %s", m->ctx[k]->device, msg[k].c_str());
+            rtd::set_error("device %d: %s", m->ctx[k]->device, msg[k].c_str());
             return st[k];
         }
     // ---- fused reduce + finalisation: device k sums band k of all accumulators over NVLink into device 0's image ----
     void* peers[kMaxRanks] = {};
     for (int k = 0; k < m->n; ++k) peers[k] = m->accum[k];
-    M_TRY(cudaSetDevice(m->ctx[0]->device));
-    M_TRY(cudaEventRecord(m->ev_t[0], m->ctx[0]->stream));
+    CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
+    CUDA_TRY(cudaEventRecord(m->ev_t[0], m->ctx[0]->stream));
     for (int k = 0; k < m->n; ++k) {
-        M_TRY(cudaSetDevice(m->ctx[k]->device));
+        CUDA_TRY(cudaSetDevice(m->ctx[k]->device));
         cudaStream_t s = m->ctx[k]->stream;
-        if (k == 0) M_TRY(cudaStreamWaitEvent(s, m->ev_t[0], 0));
+        if (k == 0) CUDA_TRY(cudaStreamWaitEvent(s, m->ev_t[0], 0));
         for (int j = 0; j < m->n; ++j)
-            if (j != k) M_TRY(cudaStreamWaitEvent(s, m->ev_done[j], 0));
+            if (j != k) CUDA_TRY(cudaStreamWaitEvent(s, m->ev_done[j], 0));
         int32_t r0 = 0, r1 = 0;
         rt_shard_rows(p->height, k, m->n, &r0, &r1);
         rtd::launch_reduce_tonemap(peers, m->n, nullptr, p->width, p->height, r0, r1, image_rgb(m->image),
                                    out_rgb8 ? image_rgb8(m->image, p->width, p->height) : nullptr, nullptr, m->ctx[k]->sm_count, s);
-        M_TRY(cudaGetLastError());
-        M_TRY(cudaEventRecord(m->ev_red[k], s));
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaEventRecord(m->ev_red[k], s));
     }
-    M_TRY(cudaSetDevice(m->ctx[0]->device));
+    CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
     cudaStream_t s0 = m->ctx[0]->stream;
-    for (int k = 1; k < m->n; ++k) M_TRY(cudaStreamWaitEvent(s0, m->ev_red[k], 0));
-    M_TRY(cudaEventRecord(m->ev_t[1], s0));
-    if (out_rgb) M_TRY(cudaMemcpyAsync(out_rgb, image_rgb(m->image), npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, s0));
-    if (out_rgb8) M_TRY(cudaMemcpyAsync(out_rgb8, image_rgb8(m->image, p->width, p->height), npix * 3, cudaMemcpyDeviceToHost, s0));
-    M_TRY(cudaStreamSynchronize(s0));
+    for (int k = 1; k < m->n; ++k) CUDA_TRY(cudaStreamWaitEvent(s0, m->ev_red[k], 0));
+    CUDA_TRY(cudaEventRecord(m->ev_t[1], s0));
+    if (out_rgb) CUDA_TRY(cudaMemcpyAsync(out_rgb, image_rgb(m->image), npix * 3 * sizeof(float), cudaMemcpyDeviceToHost, s0));
+    if (out_rgb8) CUDA_TRY(cudaMemcpyAsync(out_rgb8, image_rgb8(m->image, p->width, p->height), npix * 3, cudaMemcpyDeviceToHost, s0));
+    CUDA_TRY(cudaStreamSynchronize(s0));
     float red = 0.f;
-    M_TRY(cudaEventElapsedTime(&red, m->ev_t[0], m->ev_t[1]));
+    CUDA_TRY(cudaEventElapsedTime(&red, m->ev_t[0], m->ev_t[1]));
     if (ms_reduce) *ms_reduce = red;
     if (stats) {
         memset(stats, 0, sizeof *stats);
@@ -489,16 +454,16 @@ extern "C" rt_status rt_multi_render(rt_multi* m, const rt_render_params* p, flo
     }
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" rt_status rt_multi_read_accum(rt_multi* m, int32_t member, float* out_accum) try {
-    M_ARG(m && out_accum && member >= 0 && member < m->n && m->accum[member], "bad member / no frame rendered yet");
-    M_TRY(cudaSetDevice(m->ctx[member]->device));
-    M_TRY(cudaMemcpyAsync(out_accum, m->accum[member], m->accum_px * sizeof(float4), cudaMemcpyDeviceToHost, m->ctx[member]->stream));
-    M_TRY(cudaStreamSynchronize(m->ctx[member]->stream));
+    ARG_CHECK(m && out_accum && member >= 0 && member < m->n && m->accum[member], "bad member / no frame rendered yet");
+    CUDA_TRY(cudaSetDevice(m->ctx[member]->device));
+    CUDA_TRY(cudaMemcpyAsync(out_accum, m->accum[member], m->accum_px * sizeof(float4), cudaMemcpyDeviceToHost, m->ctx[member]->stream));
+    CUDA_TRY(cudaStreamSynchronize(m->ctx[member]->stream));
     return RT_OK;
 }
-M_CATCH
+RT_API_CATCH
 
 extern "C" void rt_multi_destroy(rt_multi* m) {
     if (!m) return;
