@@ -264,6 +264,33 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
 void rt_scene_destroy(rt_scene* scene); /* replaces free_scene<<<1,1>>> (main.cu:360-366) */
 rt_status rt_scene_get_info(const rt_scene* scene, rt_scene_info* info);
 
+/* An edit of a resident scene.  Indices are positions in the rt_scene_desc the scene was created from. */
+typedef struct rt_scene_edit {
+    const uint32_t* sphere_index;   /* spheres to replace (list ordinals), each at most once per edit */
+    const rt_sphere* spheres;       /* their new values */
+    uint32_t n_spheres;
+    const uint32_t* material_index; /* materials to replace, each at most once per edit */
+    const rt_material* materials;   /* their new values */
+    uint32_t n_materials;
+    const rt_camera* camera;        /* NULL: keep the scene's camera */
+} rt_scene_edit;
+/* Applies an edit to a scene on the device, without a new upload or build.  After RT_OK the scene renders and probes
+ * exactly like rt_scene_create of its creation description with the edit applied (same bvh_mode): rt_trace_primary gives
+ * bit-identical hits for every use_bvh both scenes support, rt_shade_probe identical records, renders equal sample and
+ * ray counts and sums equal up to the order of float additions.  The tree keeps its topology and depth; every node box is
+ * refitted on the device (all node forms), so large motions make the tree slower, never wrong — create the scene again
+ * for a fresh tree.  rt_scene_get_info keeps describing the scene as it was built.
+ * Not editable: the sphere and material counts, textures, images, bvh_mode, and a sphere's RT_SPHERE_MOVING flag (static
+ * spheres are stored first; create a sphere that may start moving as a moving sphere with center1 == center0).
+ * Every argument is checked before any device work; RT_ERR_INVALID_ARG leaves the scene unchanged: NULLs, ctx not the
+ * scene's own context, indices out of range or repeated, a changed RT_SPHERE_MOVING flag, and the sphere, material and
+ * camera rules of rt_scene_create.  An empty edit is a valid no-op.
+ * Ordering: the update runs on ctx's stream after the work queued there before it (a render enqueued before the call
+ * renders the old scene); renders of this scene through other contexts must have completed (as for rt_scene_destroy).
+ * Returns when the update is complete.  ms_device (may be NULL): device time of the update.  A CUDA error during the
+ * update (RT_ERR_CUDA / RT_ERR_OOM) leaves the scene unusable: destroy it. */
+rt_status rt_scene_update(rt_context* ctx, rt_scene* scene, const rt_scene_edit* edit, float* ms_device);
+
 /* Parity hook: closest hit of scene.hit(r, tmin, FLT_MAX) (hitable_list.h:60-79)
  * for n caller-supplied rays.  use_bvh = 0 forces the brute-force list path, 1 walks the binary BVH
  * (bvh_node::dfs, bvh.h:121-155), 2 the 4-wide form of the same tree, 3 its 64-byte quantised form — the nodes the
@@ -454,6 +481,9 @@ rt_status rt_multi_create(const int32_t* devices, int32_t n_devices, rt_multi** 
 int32_t rt_multi_size(const rt_multi* m);
 /* uploads the scene to every device (the uploads and BVH builds run side by side) */
 rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc);
+/* rt_scene_update of every member's scene with the same edit (the updates run side by side); reports the first failing
+ * device */
+rt_status rt_multi_update_scene(rt_multi* m, const rt_scene_edit* edit);
 /* p->spp is the TOTAL sample count of the frame.  out_rgb (HOST, layout of rt_render) and/or out_rgb8 (HOST, Y-flipped
  * bytes as main.cu:476-487).  stats (may be NULL): paths, rays and launches summed over the devices, ms_total = the slowest
  * device's render, ms_tonemap = device time from the root's render end to the last band of the reduce, ms_d2h = wall

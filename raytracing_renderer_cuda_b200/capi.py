@@ -83,6 +83,12 @@ class rt_scene_desc(C.Structure):
                 ("camera", rt_camera), ("bvh_mode", C.c_uint32)]
 
 
+class rt_scene_edit(C.Structure):
+    _fields_ = [("sphere_index", C.POINTER(C.c_uint32)), ("spheres", C.POINTER(rt_sphere)), ("n_spheres", C.c_uint32),
+                ("material_index", C.POINTER(C.c_uint32)), ("materials", C.POINTER(rt_material)), ("n_materials", C.c_uint32),
+                ("camera", C.POINTER(rt_camera))]
+
+
 class rt_render_params(C.Structure):
     _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("spp", C.c_int32), ("sample_offset", C.c_int32),
                 ("max_depth", C.c_int32), ("seed", C.c_uint32), ("tmin", C.c_float), ("world", C.c_float * 3),
@@ -144,6 +150,7 @@ _SIGNATURES = {
     "rt_scene_create": (C.c_int, [_VP, C.POINTER(rt_scene_desc), C.POINTER(_VP)]),
     "rt_scene_destroy": (None, [_VP]),
     "rt_scene_get_info": (C.c_int, [_VP, C.POINTER(rt_scene_info)]),
+    "rt_scene_update": (C.c_int, [_VP, _VP, C.POINTER(rt_scene_edit), C.POINTER(C.c_float)]),
     "rt_trace_primary": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_float, C.c_int, _VP]),
     "rt_selftest_rz": (C.c_int, [_VP, _VP, _VP, C.c_size_t, _VP]),
     "rt_selftest_exclusive_sum": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
@@ -176,6 +183,7 @@ _SIGNATURES = {
     "rt_multi_create": (C.c_int, [C.POINTER(C.c_int32), C.c_int32, C.POINTER(_VP)]),
     "rt_multi_size": (C.c_int32, [_VP]),
     "rt_multi_set_scene": (C.c_int, [_VP, C.POINTER(rt_scene_desc)]),
+    "rt_multi_update_scene": (C.c_int, [_VP, C.POINTER(rt_scene_edit)]),
     "rt_multi_render": (C.c_int, [_VP, C.POINTER(rt_render_params), _VP, _VP, C.POINTER(rt_stats), C.POINTER(C.c_float)]),
     "rt_multi_read_accum": (C.c_int, [_VP, C.c_int32, _VP]),
     "rt_multi_destroy": (None, [_VP]),
@@ -241,7 +249,7 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
 
 def check_layout(lib: C.CDLL) -> None:
     for cls in (rt_jpeg_component, rt_jpeg_coefficients, rt_sphere, rt_material, rt_texture, rt_image, rt_camera, rt_scene_desc, rt_render_params, rt_stats,
-                rt_scene_info, rt_ray, rt_hit, rt_shade_sample, rt_denoise_params, rt_adaptive_params):
+                rt_scene_info, rt_scene_edit, rt_ray, rt_hit, rt_shade_sample, rt_denoise_params, rt_adaptive_params):
         want = lib.rt_abi_sizeof(cls.__name__.encode())
         if want != C.sizeof(cls):
             raise RuntimeError(f"ABI drift: sizeof({cls.__name__}) is {want} in the library, {C.sizeof(cls)} here")
@@ -408,6 +416,15 @@ class Scene:
         _check(self.lib, self.lib.rt_scene_get_info(self._h, C.byref(i)))
         return i
 
+    def update(self, sphere_index=None, spheres=None, material_index=None, materials=None, camera: "rt_camera | None" = None) -> float:
+        """rt_scene_update: replaces spheres (SPHERE_DTYPE records) and materials (rt_material sequence) at the given list
+        positions and, if given, the camera.  Returns the device time of the update in ms."""
+        edit, keep = scene_edit(sphere_index, spheres, material_index, materials, camera)
+        ms = C.c_float()
+        _check(self.lib, self.lib.rt_scene_update(self.ctx._h, self._h, C.byref(edit), C.byref(ms)))
+        del keep
+        return ms.value
+
     def trace_primary(self, rays: np.ndarray, tmin: float = 1e-5, use_bvh: bool | int = True) -> np.ndarray:
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
         hits = np.zeros(rays.shape[0], dtype=HIT_DTYPE)
@@ -535,6 +552,35 @@ class Scene:
             pass
 
 
+def scene_edit(sphere_index=None, spheres=None, material_index=None, materials=None, camera: "rt_camera | None" = None):
+    """(rt_scene_edit, the arrays it points into): the arrays must stay alive while the edit is used."""
+    edit = rt_scene_edit()
+    keep = []
+    if sphere_index is not None and len(sphere_index):
+        idx = np.ascontiguousarray(sphere_index, dtype=np.uint32)
+        sph = np.ascontiguousarray(spheres, dtype=SPHERE_DTYPE)
+        if sph.shape != idx.shape:
+            raise ValueError("sphere_index and spheres differ in length")
+        edit.sphere_index = idx.ctypes.data_as(C.POINTER(C.c_uint32))
+        edit.spheres = sph.ctypes.data_as(C.POINTER(rt_sphere))
+        edit.n_spheres = len(idx)
+        keep += [idx, sph]
+    if material_index is not None and len(material_index):
+        idx = np.ascontiguousarray(material_index, dtype=np.uint32)
+        mats = (rt_material * len(materials))(*materials)
+        if len(mats) != len(idx):
+            raise ValueError("material_index and materials differ in length")
+        edit.material_index = idx.ctypes.data_as(C.POINTER(C.c_uint32))
+        edit.materials = mats
+        edit.n_materials = len(idx)
+        keep += [idx, mats]
+    if camera is not None:
+        cam = rt_camera.from_buffer_copy(camera)
+        edit.camera = C.pointer(cam)
+        keep.append(cam)
+    return edit, keep
+
+
 def _camera_array(cameras):
     cams = list(cameras)
     return (rt_camera * len(cams))(*cams)
@@ -635,6 +681,12 @@ class Multi:
 
     def set_scene(self, desc: "SceneDesc") -> None:
         _check(self.lib, self.lib.rt_multi_set_scene(self._h, desc._ptr))
+
+    def update_scene(self, sphere_index=None, spheres=None, material_index=None, materials=None, camera: "rt_camera | None" = None) -> None:
+        """rt_multi_update_scene: Scene.update's edit on every member's scene."""
+        edit, keep = scene_edit(sphere_index, spheres, material_index, materials, camera)
+        _check(self.lib, self.lib.rt_multi_update_scene(self._h, C.byref(edit)))
+        del keep
 
     def render(self, params: rt_render_params, want_rgb8: bool = False):
         rgb = np.empty((params.height, params.width, 3), np.float32)

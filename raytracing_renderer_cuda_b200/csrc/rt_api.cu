@@ -66,11 +66,9 @@ bool camera_finite(const rt_camera& c) {
     return finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && std::isfinite(c.vfov) && std::isfinite(c.aspect) &&
            std::isfinite(c.aperture) && std::isfinite(c.focus_dist) && std::isfinite(c.time0) && std::isfinite(c.time1);
 }
-} // namespace rtd
-namespace {
 
 // camera ctor (camera.h:7-31) in host float arithmetic
-void make_camera(const rt_camera& c, rtd::DCamera& out) {
+void make_camera(const rt_camera& c, DCamera& out) {
     auto V = [](const float* p) { return rtd::V3{p[0], p[1], p[2]}; };
     auto sub = [](rtd::V3 a, rtd::V3 b) { return rtd::V3{a.x - b.x, a.y - b.y, a.z - b.z}; };
     auto mul = [](rtd::V3 a, float s) { return rtd::V3{a.x * s, a.y * s, a.z * s}; };
@@ -101,6 +99,65 @@ void make_camera(const rt_camera& c, rtd::DCamera& out) {
     out.vertical = mul(v, 2 * half_height * c.focus_dist);
 }
 
+rt_status check_material(const rt_material& m, uint32_t n_textures) {
+    ARG_CHECK(m.kind <= RT_MAT_EMITTER, "bad material kind");
+    if (m.kind == RT_MAT_LAMBERTIAN || m.kind == RT_MAT_EMITTER)
+        ARG_CHECK(m.texture >= 0 && uint32_t(m.texture) < n_textures, "material texture out of range");
+    return RT_OK;
+}
+
+rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials) {
+    // non-finite geometry would reach the builders' bin arithmetic (undefined for NaN / infinity) and the slab tests
+    auto finite3 = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
+    ARG_CHECK(sp.material < n_materials, "sphere material out of range");
+    ARG_CHECK(finite3(sp.center0) && finite3(sp.center1) && std::isfinite(sp.radius) && std::isfinite(sp.time0) &&
+                  std::isfinite(sp.time1),
+              "sphere centre / radius / time is not finite");
+    return RT_OK;
+}
+
+void pack_spheres(const rt_sphere* spheres, const uint32_t* src, const uint32_t* ordinal, size_t count, float4* a, float4* b,
+                  uint4* c) {
+    {
+        // c1 - c0 rounded toward zero (== __fsub_rz, vec3 operator- of moving_sphere::center, sphere.h:51).  The rounding
+        // mode is switched once around this loop, not per operation: at 10^6 spheres a per-call switch
+        // cost 150 ms of every scene upload.
+        const int old_round = std::fegetround();
+        std::fesetround(FE_TOWARDZERO);
+        for (size_t k = 0; k < count; ++k) {
+            const rt_sphere& sp = spheres[src ? src[k] : k];
+            volatile float dx = sp.center1[0], dy = sp.center1[1], dz = sp.center1[2];
+            dx = dx - sp.center0[0];
+            dy = dy - sp.center0[1];
+            dz = dz - sp.center0[2];
+            b[k] = make_float4(dx, dy, dz, sp.time0);
+        }
+        std::fesetround(old_round);
+    }
+    for (size_t k = 0; k < count; ++k) {
+        const rt_sphere& sp = spheres[src ? src[k] : k];
+        a[k] = make_float4(sp.center0[0], sp.center0[1], sp.center0[2], sp.radius);
+        float dt = sp.time1 - sp.time0; // FADD(RN) in the reference's SASS (sphere.h:51)
+        uint32_t dt_bits;
+        memcpy(&dt_bits, &dt, 4);
+        c[k] = make_uint4(dt_bits, sp.material, sp.id, ordinal[k]);
+    }
+}
+
+DMaterial pack_material(const rt_material& m) {
+    return DMaterial{m.kind, m.texture, m.albedo[0], m.albedo[1], m.albedo[2], m.param, 0.f, 0.f};
+}
+
+void find_lights(rt_scene* s) {
+    s->d.n_lights = 0;
+    const size_t n = s->where.size();
+    for (size_t i = 0; i < n && s->d.n_lights < RT_MAX_LIGHTS; ++i)
+        if (s->material_kind[s->sphere_material[i]] == RT_MAT_EMITTER) s->d.lights[s->d.n_lights++] = s->where[i];
+    for (uint32_t k = s->d.n_lights; k < RT_MAX_LIGHTS; ++k) s->d.lights[k] = 0;
+}
+} // namespace rtd
+namespace {
+
 rt_status validate_desc(const rt_scene_desc* d) {
     ARG_CHECK(d != nullptr, "desc is NULL");
     ARG_CHECK(d->n_spheres == 0 || d->spheres, "spheres is NULL");
@@ -119,21 +176,10 @@ rt_status validate_desc(const rt_scene_desc* d) {
                       "checker child out of range");
         if (t.kind == RT_TEX_IMAGE) ARG_CHECK(t.image >= 0 && uint32_t(t.image) < d->n_images, "image index out of range");
     }
-    for (uint32_t i = 0; i < d->n_materials; ++i) {
-        const rt_material& m = d->materials[i];
-        ARG_CHECK(m.kind <= RT_MAT_EMITTER, "bad material kind");
-        if (m.kind == RT_MAT_LAMBERTIAN || m.kind == RT_MAT_EMITTER)
-            ARG_CHECK(m.texture >= 0 && uint32_t(m.texture) < d->n_textures, "material texture out of range");
-    }
-    // non-finite geometry would reach the builders' bin arithmetic (undefined for NaN / infinity) and the slab tests
-    auto finite3 = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
-    for (uint32_t i = 0; i < d->n_spheres; ++i) {
-        const rt_sphere& sp = d->spheres[i];
-        ARG_CHECK(sp.material < d->n_materials, "sphere material out of range");
-        ARG_CHECK(finite3(sp.center0) && finite3(sp.center1) && std::isfinite(sp.radius) && std::isfinite(sp.time0) &&
-                      std::isfinite(sp.time1),
-                  "sphere centre / radius / time is not finite");
-    }
+    rt_status st = RT_OK;
+    for (uint32_t i = 0; i < d->n_materials && st == RT_OK; ++i) st = rtd::check_material(d->materials[i], d->n_textures);
+    for (uint32_t i = 0; i < d->n_spheres && st == RT_OK; ++i) st = rtd::check_sphere(d->spheres[i], d->n_materials);
+    if (st != RT_OK) return st;
     ARG_CHECK(rtd::camera_finite(d->camera), "camera parameter is not finite");
     return RT_OK;
 }
@@ -482,31 +528,11 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     std::vector<float4> ha(n), hb(n);
     std::vector<uint4> hc(n);
     std::vector<rth::Box> boxes(mode == RT_BVH_HOST_SAH ? n : 0);
-    {
-        // c1 - c0 rounded toward zero (== __fsub_rz, vec3 operator- of moving_sphere::center, sphere.h:51).  The rounding
-        // mode is switched once around this loop, not per operation: at 10^6 spheres a per-call switch
-        // cost 150 ms of every scene upload.
-        const int old_round = std::fegetround();
-        std::fesetround(FE_TOWARDZERO);
-        for (uint32_t k = 0; k < n; ++k) {
-            const rt_sphere& sp = desc->spheres[order[k]];
-            volatile float dx = sp.center1[0], dy = sp.center1[1], dz = sp.center1[2];
-            dx = dx - sp.center0[0];
-            dy = dy - sp.center0[1];
-            dz = dz - sp.center0[2];
-            hb[k] = make_float4(dx, dy, dz, sp.time0);
-        }
-        std::fesetround(old_round);
-    }
-    for (uint32_t k = 0; k < n; ++k) {
+    rtd::pack_spheres(desc->spheres, order.data(), order.data(), n, ha.data(), hb.data(), hc.data());
+    for (uint32_t k = 0; k < n && mode == RT_BVH_HOST_SAH; ++k) {
         const rt_sphere& sp = desc->spheres[order[k]];
-        ha[k] = make_float4(sp.center0[0], sp.center0[1], sp.center0[2], sp.radius);
-        float dt = sp.time1 - sp.time0; // FADD(RN) in the reference's SASS (sphere.h:51)
-        uint32_t dt_bits;
-        memcpy(&dt_bits, &dt, 4);
-        hc[k] = make_uint4(dt_bits, sp.material, sp.id, order[k]);
         const bool moving = (sp.flags & RT_SPHERE_MOVING) != 0;
-        if (mode == RT_BVH_HOST_SAH) boxes[k] = rth::sphere_box(sp.center0, moving ? sp.center1 : sp.center0, sp.radius);
+        boxes[k] = rth::sphere_box(sp.center0, moving ? sp.center1 : sp.center0, sp.radius);
     }
 
     std::vector<rth::NodeHost> nodes;
@@ -632,6 +658,7 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
                 set_error("4-wide BVH quantisation failed: %s", cudaGetErrorString(e));
                 return RT_ERR_CUDA;
             }
+            s->nodes4q_mem = dnodes4q;
             if (!quant_ok) dnodes4q = nullptr; // (the memory stays with the scene; the walk uses the 128-byte nodes)
         }
     }
@@ -641,10 +668,7 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     }
 
     std::vector<rtd::DMaterial> hm(desc->n_materials);
-    for (uint32_t i = 0; i < desc->n_materials; ++i) {
-        const rt_material& m = desc->materials[i];
-        hm[i] = rtd::DMaterial{m.kind, m.texture, m.albedo[0], m.albedo[1], m.albedo[2], m.param, 0.f, 0.f};
-    }
+    for (uint32_t i = 0; i < desc->n_materials; ++i) hm[i] = rtd::pack_material(desc->materials[i]);
     std::vector<rtd::DTexture> ht(desc->n_textures);
     for (uint32_t i = 0; i < desc->n_textures; ++i) {
         const rt_texture& t = desc->textures[i];
@@ -737,16 +761,15 @@ rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene**
     s->d.has_noise = 0;
     for (const auto& t : ht)
         if (t.kind == RT_TEX_NOISE_PERLIN || t.kind == RT_TEX_NOISE_TURBULANCE || t.kind == RT_TEX_NOISE_MARBLE || t.kind == RT_TEX_WOOD) s->d.has_noise = 1;
-    make_camera(desc->camera, s->d.cam);
-    // emitter spheres for RT_RENDER_EMITTER_SAMPLING: device primitive indices in the caller's list order
-    s->d.n_lights = 0;
-    {
-        std::vector<uint32_t> where(n); // list ordinal -> device index
-        for (uint32_t k = 0; k < n; ++k) where[order[k]] = k;
-        for (uint32_t i = 0; i < n && s->d.n_lights < RT_MAX_LIGHTS; ++i)
-            if (desc->materials[desc->spheres[i].material].kind == RT_MAT_EMITTER) s->d.lights[s->d.n_lights++] = where[i];
-        for (uint32_t k = s->d.n_lights; k < RT_MAX_LIGHTS; ++k) s->d.lights[k] = 0;
-    }
+    rtd::make_camera(desc->camera, s->d.cam);
+    s->where.resize(n); // list ordinal -> device index
+    for (uint32_t k = 0; k < n; ++k) s->where[order[k]] = k;
+    s->sphere_material.resize(n);
+    for (uint32_t i = 0; i < n; ++i) s->sphere_material[i] = desc->spheres[i].material;
+    s->material_kind.resize(desc->n_materials);
+    for (uint32_t i = 0; i < desc->n_materials; ++i) s->material_kind[i] = desc->materials[i].kind;
+    s->n_textures = desc->n_textures;
+    rtd::find_lights(s);
 
     const auto t_end = std::chrono::steady_clock::now();
     s->info.n_spheres = n;

@@ -23,9 +23,7 @@ __device__ __forceinline__ float unflip_f(unsigned u) {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
-// Primitive bounds (sphere.h:142-146; moving: union of the boxes at both ends of the motion,
-// sphere.h:192-202), padded exactly like the host builder (rt_bvh_host.cpp sphere_box) so the
-// conservative slab test never rejects a ray the rounded sphere test accepts.
+// Primitive bounds (prim_box, rt_lbvh.cuh) and their centroid bounds.
 __global__ void __launch_bounds__(256) k_prim_boxes(const float4* __restrict__ sph_a, const float4* __restrict__ sph_b,
                                                     const uint32_t* __restrict__ ids, uint32_t n, uint32_t n_static,
                                                     float4* __restrict__ lo, float4* __restrict__ hi,
@@ -35,23 +33,10 @@ __global__ void __launch_bounds__(256) k_prim_boxes(const float4* __restrict__ s
     bool valid = i < n;
     if (valid) {
         const uint32_t prim = ids ? ids[i] : i;
-        float4 a = __ldg(&sph_a[prim]);
-        float c0[3] = {a.x, a.y, a.z}, c1[3] = {a.x, a.y, a.z};
-        if (prim >= n_static) {
-            float4 b = __ldg(&sph_b[prim]);
-            c1[0] = __fadd_rz(a.x, b.x); // where moving_center() puts the sphere at the end of its motion
-            c1[1] = __fadd_rz(a.y, b.y);
-            c1[2] = __fadd_rz(a.z, b.z);
-        }
-        float ar = fabsf(a.w), l[3], h[3];
+        float l[3], h[3];
+        prim_box(sph_a, sph_b, prim, n_static, l, h);
 #pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            float lk = fminf(c0[k], c1[k]) - ar, hk = fmaxf(c0[k], c1[k]) + ar;
-            float pad = ar * 6.1035156e-5f + (fabsf(lk) + fabsf(hk)) * 3.8146973e-6f;
-            l[k] = lk - pad;
-            h[k] = hk + pad;
-            c[k] = 0.5f * l[k] + 0.5f * h[k];
-        }
+        for (int k = 0; k < 3; ++k) c[k] = 0.5f * l[k] + 0.5f * h[k];
         lo[i] = make_float4(l[0], l[1], l[2], 0.f);
         hi[i] = make_float4(h[0], h[1], h[2], 0.f);
     }
@@ -168,21 +153,7 @@ __global__ void __launch_bounds__(256) k_refit(const uint32_t* __restrict__ vals
     int me = ~int(ids ? ids[ci] : ci);
     int parent = parent_leaf[k];
     while (parent >= 0) {
-        BvhNode* nd = nodes + parent;
-        volatile float* f = reinterpret_cast<volatile float*>(nd);
-        int left = reinterpret_cast<const int*>(&nd->lmin)[3];
-        if (left == me) {
-            f[0] = bl.x; f[1] = bl.y; f[2] = bl.z;
-            f[4] = bh.x; f[5] = bh.y; f[6] = bh.z;
-        } else {
-            f[8] = bl.x; f[9] = bl.y; f[10] = bl.z; f[11] = 0.f;
-            f[12] = bh.x; f[13] = bh.y; f[14] = bh.z; f[15] = 0.f;
-        }
-        __threadfence();
-        if (atomicAdd(&visits[parent], 1u) == 0u) return; // sibling subtree not finished yet
-        __threadfence();
-        bl = make_float4(fminf(f[0], f[8]), fminf(f[1], f[9]), fminf(f[2], f[10]), 0.f);
-        bh = make_float4(fmaxf(f[4], f[12]), fmaxf(f[5], f[13]), fmaxf(f[6], f[14]), 0.f);
+        if (!refit_step(nodes, parent, me, bl, bh, visits)) return;
         me = parent;
         parent = parent_inner[parent];
     }

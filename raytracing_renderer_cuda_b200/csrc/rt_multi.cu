@@ -362,6 +362,27 @@ extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) 
 }
 RT_API_CATCH
 
+extern "C" rt_status rt_multi_update_scene(rt_multi* m, const rt_scene_edit* edit) try {
+    ARG_CHECK(m && edit, "multi/edit is NULL");
+    for (int k = 0; k < m->n; ++k) ARG_CHECK(m->scene[k] != nullptr, "no scene: call rt_multi_set_scene first");
+    std::vector<rt_status> st(m->n, RT_OK);
+    std::vector<std::string> msg(m->n);
+    std::vector<std::thread> th;
+    for (int k = 0; k < m->n; ++k)
+        th.emplace_back([&, k] { // the updates of the devices run side by side
+            st[k] = rt_scene_update(m->ctx[k], m->scene[k], edit, nullptr);
+            if (st[k] != RT_OK) msg[k] = rt_last_error();
+        });
+    for (auto& t : th) t.join();
+    for (int k = 0; k < m->n; ++k)
+        if (st[k] != RT_OK) {
+            rtd::set_error("device %d: %s", m->ctx[k]->device, msg[k].c_str());
+            return st[k];
+        }
+    return RT_OK;
+}
+RT_API_CATCH
+
 extern "C" rt_status rt_multi_render(rt_multi* m, const rt_render_params* p, float* out_rgb, uint8_t* out_rgb8, rt_stats* stats,
                                      float* ms_reduce) try {
     ARG_CHECK(m && p, "multi/params is NULL");
