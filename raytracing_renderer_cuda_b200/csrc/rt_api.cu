@@ -1,9 +1,5 @@
-// rt_api.cu — C-ABI of librt_b200.so (include/rt_api.h): context, scene upload +
-// acceleration-structure build, render / accumulate / tonemap entry points.
-// Host logic only; the kernels live in rt_kernels.cu / rt_wavefront.cu / rt_lbvh.cu.
-#include <algorithm>
-#include <cfenv>
-#include <chrono>
+// rt_api.cu — C-ABI of librt_b200.so (include/rt_api.h): contexts, render / accumulate / probe / tonemap / JPEG / image
+// entry points (scenes: rt_scene.cu).  Host logic only; the kernels live in rt_kernels.cu / rt_wavefront.cu / rt_lbvh.cu.
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -15,10 +11,8 @@
 #include <type_traits>
 #include <vector>
 
-#include "rt_bvh_host.hpp"
 #include "rt_internal.hpp"
 #include "rt_jpeg_decode.cuh"
-#include "rt_lbvh.cuh"
 
 namespace {
 thread_local std::string g_last_error;
@@ -44,29 +38,7 @@ cudaError_t malloc_async_bytes(void** p, size_t bytes, cudaStream_t st) {
 using rtd::make_current;
 using rtd::set_error;
 
-namespace {
-
-template <class T>
-rt_status dev_alloc(rt_scene* s, T** out, size_t count) {
-    *out = nullptr;
-    if (count == 0) return RT_OK;
-    void* p = nullptr;
-    CUDA_TRY(cudaMallocFromPoolAsync(&p, count * sizeof(T), s->ctx->pool, s->ctx->stream)); // the context's pool: no map/unmap per scene
-    s->allocs.push_back(p);
-    s->info.device_bytes += count * sizeof(T);
-    *out = static_cast<T*>(p);
-    return RT_OK;
-}
-
-} // namespace
 namespace rtd {
-// every parameter of a camera finite (scene descriptions, frame sequences, rt_orbit_cameras)
-bool camera_finite(const rt_camera& c) {
-    auto finite3 = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
-    return finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && std::isfinite(c.vfov) && std::isfinite(c.aspect) &&
-           std::isfinite(c.aperture) && std::isfinite(c.focus_dist) && std::isfinite(c.time0) && std::isfinite(c.time1);
-}
-
 // camera ctor (camera.h:7-31) in host float arithmetic
 void make_camera(const rt_camera& c, DCamera& out) {
     auto V = [](const float* p) { return rtd::V3{p[0], p[1], p[2]}; };
@@ -98,91 +70,8 @@ void make_camera(const rt_camera& c, DCamera& out) {
     out.horizontal = mul(u, 2 * half_width * c.focus_dist);
     out.vertical = mul(v, 2 * half_height * c.focus_dist);
 }
-
-rt_status check_material(const rt_material& m, uint32_t n_textures) {
-    ARG_CHECK(m.kind <= RT_MAT_EMITTER, "bad material kind");
-    if (m.kind == RT_MAT_LAMBERTIAN || m.kind == RT_MAT_EMITTER)
-        ARG_CHECK(m.texture >= 0 && uint32_t(m.texture) < n_textures, "material texture out of range");
-    return RT_OK;
-}
-
-rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials) {
-    // non-finite geometry would reach the builders' bin arithmetic (undefined for NaN / infinity) and the slab tests
-    auto finite3 = [](const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); };
-    ARG_CHECK(sp.material < n_materials, "sphere material out of range");
-    ARG_CHECK(finite3(sp.center0) && finite3(sp.center1) && std::isfinite(sp.radius) && std::isfinite(sp.time0) &&
-                  std::isfinite(sp.time1),
-              "sphere centre / radius / time is not finite");
-    return RT_OK;
-}
-
-void pack_spheres(const rt_sphere* spheres, const uint32_t* src, const uint32_t* ordinal, size_t count, float4* a, float4* b,
-                  uint4* c) {
-    {
-        // c1 - c0 rounded toward zero (== __fsub_rz, vec3 operator- of moving_sphere::center, sphere.h:51).  The rounding
-        // mode is switched once around this loop, not per operation: at 10^6 spheres a per-call switch
-        // cost 150 ms of every scene upload.
-        const int old_round = std::fegetround();
-        std::fesetround(FE_TOWARDZERO);
-        for (size_t k = 0; k < count; ++k) {
-            const rt_sphere& sp = spheres[src ? src[k] : k];
-            volatile float dx = sp.center1[0], dy = sp.center1[1], dz = sp.center1[2];
-            dx = dx - sp.center0[0];
-            dy = dy - sp.center0[1];
-            dz = dz - sp.center0[2];
-            b[k] = make_float4(dx, dy, dz, sp.time0);
-        }
-        std::fesetround(old_round);
-    }
-    for (size_t k = 0; k < count; ++k) {
-        const rt_sphere& sp = spheres[src ? src[k] : k];
-        a[k] = make_float4(sp.center0[0], sp.center0[1], sp.center0[2], sp.radius);
-        float dt = sp.time1 - sp.time0; // FADD(RN) in the reference's SASS (sphere.h:51)
-        uint32_t dt_bits;
-        memcpy(&dt_bits, &dt, 4);
-        c[k] = make_uint4(dt_bits, sp.material, sp.id, ordinal[k]);
-    }
-}
-
-DMaterial pack_material(const rt_material& m) {
-    return DMaterial{m.kind, m.texture, m.albedo[0], m.albedo[1], m.albedo[2], m.param, 0.f, 0.f};
-}
-
-void find_lights(rt_scene* s) {
-    s->d.n_lights = 0;
-    const size_t n = s->where.size();
-    for (size_t i = 0; i < n && s->d.n_lights < RT_MAX_LIGHTS; ++i)
-        if (s->material_kind[s->sphere_material[i]] == RT_MAT_EMITTER) s->d.lights[s->d.n_lights++] = s->where[i];
-    for (uint32_t k = s->d.n_lights; k < RT_MAX_LIGHTS; ++k) s->d.lights[k] = 0;
-}
 } // namespace rtd
 namespace {
-
-rt_status validate_desc(const rt_scene_desc* d) {
-    ARG_CHECK(d != nullptr, "desc is NULL");
-    ARG_CHECK(d->n_spheres == 0 || d->spheres, "spheres is NULL");
-    ARG_CHECK(d->n_materials == 0 || d->materials, "materials is NULL");
-    ARG_CHECK(d->n_textures == 0 || d->textures, "textures is NULL");
-    ARG_CHECK(d->n_images == 0 || d->images, "images is NULL");
-    ARG_CHECK(d->n_images <= RT_MAX_IMAGES, "too many images (max 8)");
-    ARG_CHECK(d->bvh_mode <= RT_BVH_GPU_LBVH, "bad bvh_mode");
-    for (uint32_t i = 0; i < d->n_images; ++i)
-        ARG_CHECK(d->images[i].rgb && d->images[i].width > 0 && d->images[i].height > 0, "empty image");
-    for (uint32_t i = 0; i < d->n_textures; ++i) {
-        const rt_texture& t = d->textures[i];
-        ARG_CHECK(t.kind <= RT_TEX_IMAGE, "bad texture kind");
-        if (t.kind == RT_TEX_CHECKER)
-            ARG_CHECK(t.even >= 0 && uint32_t(t.even) < d->n_textures && t.odd >= 0 && uint32_t(t.odd) < d->n_textures,
-                      "checker child out of range");
-        if (t.kind == RT_TEX_IMAGE) ARG_CHECK(t.image >= 0 && uint32_t(t.image) < d->n_images, "image index out of range");
-    }
-    rt_status st = RT_OK;
-    for (uint32_t i = 0; i < d->n_materials && st == RT_OK; ++i) st = rtd::check_material(d->materials[i], d->n_textures);
-    for (uint32_t i = 0; i < d->n_spheres && st == RT_OK; ++i) st = rtd::check_sphere(d->spheres[i], d->n_materials);
-    if (st != RT_OK) return st;
-    ARG_CHECK(rtd::camera_finite(d->camera), "camera parameter is not finite");
-    return RT_OK;
-}
 
 rt_status check_params(const rt_render_params* p) {
     ARG_CHECK(p != nullptr, "params is NULL");
@@ -487,331 +376,6 @@ rt_status rt_context_set_stream(rt_context* ctx, void* cuda_stream) try {
 rt_status rt_context_synchronize(rt_context* ctx) try {
     ARG_CHECK(ctx != nullptr, "ctx is NULL");
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    return RT_OK;
-} RT_API_CATCH
-
-rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc, rt_scene** out) try {
-    ARG_CHECK(ctx != nullptr && out != nullptr, "ctx/out is NULL");
-    *out = nullptr;
-    rt_status st = validate_desc(desc);
-    if (st != RT_OK) return st;
-    st = make_current(ctx);
-    if (st != RT_OK) return st;
-
-    rt_scene* s = new (std::nothrow) rt_scene();
-    if (!s) return RT_ERR_OOM;
-    s->ctx = ctx;
-    struct Guard {
-        rt_scene* s;
-        ~Guard() {
-            if (s) rt_scene_destroy(s);
-        }
-    } guard{s};
-
-    const auto t_begin = std::chrono::steady_clock::now();
-    const uint32_t n = desc->n_spheres;
-
-    // ---- primitives: static spheres first (stable), SoA float4 arrays ----
-    std::vector<uint32_t> order;
-    order.reserve(n);
-    for (uint32_t i = 0; i < n; ++i)
-        if (!(desc->spheres[i].flags & RT_SPHERE_MOVING)) order.push_back(i);
-    const uint32_t n_static = uint32_t(order.size());
-    for (uint32_t i = 0; i < n; ++i)
-        if (desc->spheres[i].flags & RT_SPHERE_MOVING) order.push_back(i);
-
-    // ---- acceleration structure: which one ----
-    uint32_t mode = desc->bvh_mode;
-    if (mode == RT_BVH_AUTO) mode = n <= 12 ? RT_BVH_NONE : (n <= 200000 ? RT_BVH_HOST_SAH : RT_BVH_GPU_LBVH);
-    if (n < 2) mode = RT_BVH_NONE;
-
-    std::vector<float4> ha(n), hb(n);
-    std::vector<uint4> hc(n);
-    std::vector<rth::Box> boxes(mode == RT_BVH_HOST_SAH ? n : 0);
-    rtd::pack_spheres(desc->spheres, order.data(), order.data(), n, ha.data(), hb.data(), hc.data());
-    for (uint32_t k = 0; k < n && mode == RT_BVH_HOST_SAH; ++k) {
-        const rt_sphere& sp = desc->spheres[order[k]];
-        const bool moving = (sp.flags & RT_SPHERE_MOVING) != 0;
-        boxes[k] = rth::sphere_box(sp.center0, moving ? sp.center1 : sp.center0, sp.radius);
-    }
-
-    std::vector<rth::NodeHost> nodes;
-    rth::BvhStats bstats;
-    const auto t_build0 = std::chrono::steady_clock::now();
-    if (mode == RT_BVH_HOST_SAH) rth::build_bvh_sah(boxes, nodes, &bstats);
-    const auto t_build1 = std::chrono::steady_clock::now();
-
-    // ---- upload ----
-    float4 *da = nullptr, *db = nullptr;
-    uint4* dc = nullptr;
-    rtd::BvhNode* dnodes = nullptr;
-    rtd::DMaterial* dmats = nullptr;
-    rtd::DTexture* dtexs = nullptr;
-    if ((st = dev_alloc(s, &da, n)) != RT_OK) return st;
-    if ((st = dev_alloc(s, &db, n)) != RT_OK) return st;
-    if ((st = dev_alloc(s, &dc, n)) != RT_OK) return st;
-    cudaStream_t stream = ctx->stream;
-    if (n) {
-        CUDA_TRY(cudaMemcpyAsync(da, ha.data(), n * sizeof(float4), cudaMemcpyHostToDevice, stream));
-        CUDA_TRY(cudaMemcpyAsync(db, hb.data(), n * sizeof(float4), cudaMemcpyHostToDevice, stream));
-        CUDA_TRY(cudaMemcpyAsync(dc, hc.data(), n * sizeof(uint4), cudaMemcpyHostToDevice, stream));
-    }
-    float lbvh_ms = 0.f;
-    uint32_t bvh_root = 0;
-    uint32_t n_nodes = 0;
-    if (mode == RT_BVH_HOST_SAH) {
-        n_nodes = uint32_t(nodes.size());
-        if ((st = dev_alloc(s, &dnodes, n_nodes)) != RT_OK) return st;
-        CUDA_TRY(cudaMemcpyAsync(dnodes, nodes.data(), n_nodes * sizeof(rtd::BvhNode), cudaMemcpyHostToDevice, stream));
-    } else if (mode == RT_BVH_GPU_LBVH) {
-        n_nodes = n - 1;
-        if ((st = dev_alloc(s, &dnodes, n_nodes)) != RT_OK) return st;
-        // Outsized primitives (the r = 1000 ground every scene of this renderer has) would sit deep in a Morton-ordered
-        // tree and inflate the boxes of all their ancestors, so every ray would walk that whole chain.  They are kept
-        // out of the LBVH and hung above its root instead: root -> (big_k, (... (big_0, LBVH root))).
-        std::vector<uint32_t> big, normal;
-        {
-            std::vector<float> radii(n);
-            for (uint32_t k = 0; k < n; ++k) radii[k] = std::fabs(ha[k].w);
-            std::vector<float> tmp(radii);
-            std::nth_element(tmp.begin(), tmp.begin() + n / 2, tmp.end());
-            const float limit = 32.f * tmp[n / 2];
-            for (uint32_t k = 0; k < n; ++k) (radii[k] > limit && big.size() < 32 ? big : normal).push_back(k);
-            if (normal.size() < 2) { // nothing sensible to separate
-                big.clear();
-                normal.clear();
-            }
-        }
-        const uint32_t m = big.empty() ? n : uint32_t(normal.size());
-        rtd::PoolBuffer<uint32_t> d_ids;
-        if (!big.empty()) {
-            CUDA_TRY(d_ids.alloc(m, stream));
-            CUDA_TRY(cudaMemcpyAsync(d_ids.get(), normal.data(), m * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
-        }
-        float rb[6];
-        cudaError_t e = rtd::lbvh_build(da, db, n_static, d_ids.get(), m, dnodes, stream, &lbvh_ms, &bstats.depth, rb);
-        if (e != cudaSuccess) {
-            set_error("GPU LBVH build failed: %s", cudaGetErrorString(e));
-            return RT_ERR_CUDA;
-        }
-        if (!big.empty()) {
-            std::vector<rth::NodeHost> chain(big.size());
-            rth::Box below{{rb[0], rb[1], rb[2]}, {rb[3], rb[4], rb[5]}};
-            int32_t below_ref = 0; // the LBVH root
-            for (size_t k = 0; k < big.size(); ++k) {
-                const rt_sphere& sp = desc->spheres[order[big[k]]];
-                const bool moving = (sp.flags & RT_SPHERE_MOVING) != 0;
-                rth::Box bb = rth::sphere_box(sp.center0, moving ? sp.center1 : sp.center0, sp.radius);
-                rth::NodeHost& nd = chain[k];
-                for (int a = 0; a < 3; ++a) {
-                    nd.lmin[a] = bb.lo[a];
-                    nd.lmax[a] = bb.hi[a];
-                    nd.rmin[a] = below.lo[a];
-                    nd.rmax[a] = below.hi[a];
-                    below.lo[a] = std::min(below.lo[a], bb.lo[a]);
-                    below.hi[a] = std::max(below.hi[a], bb.hi[a]);
-                }
-                nd.left = ~int32_t(big[k]);
-                nd.right = below_ref;
-                nd.pad0 = nd.pad1 = 0.f;
-                below_ref = int32_t(m - 1 + k);
-            }
-            CUDA_TRY(cudaMemcpyAsync(dnodes + (m - 1), chain.data(), chain.size() * sizeof(rtd::BvhNode), cudaMemcpyHostToDevice, stream));
-            CUDA_TRY(cudaStreamSynchronize(stream)); // `chain` is a pageable host buffer
-            bvh_root = uint32_t(below_ref);
-            bstats.depth += uint32_t(big.size());
-        }
-    }
-    rtd::BvhNodeCH* dnodes_ch = nullptr;
-    if (dnodes && n_nodes) { // the form the binary traversal reads
-        if ((st = dev_alloc(s, &dnodes_ch, n_nodes)) != RT_OK) return st;
-        cudaError_t e = rtd::bvh_nodes_ch(dnodes, n_nodes, dnodes_ch, stream);
-        if (e != cudaSuccess) {
-            set_error("BVH node conversion failed: %s", cudaGetErrorString(e));
-            return RT_ERR_CUDA;
-        }
-    }
-    rtd::BvhNode4* dnodes4 = nullptr;
-    rtd::BvhNode4Q* dnodes4q = nullptr;
-    uint32_t n_nodes4 = 0, root4 = 0;
-    if (dnodes && n_nodes) { // the 4-wide form the persistent-lane kernel walks (half the dependent node fetches per ray)
-        if ((st = dev_alloc(s, &dnodes4, n_nodes / 2 + 64)) != RT_OK) return st;
-        rtd::PoolBuffer<rtd::BvhNode4> scratch; // worst case (a degenerate chain) every binary node survives
-        CUDA_TRY(scratch.alloc(n_nodes, stream));
-        cudaError_t e = rtd::bvh_collapse4(dnodes, n_nodes, bvh_root, bstats.depth, scratch.get(), &n_nodes4, &root4, stream);
-        if (e == cudaSuccess && n_nodes4 <= n_nodes / 2 + 64) {
-            e = cudaMemcpyAsync(dnodes4, scratch.get(), size_t(n_nodes4) * sizeof(rtd::BvhNode4), cudaMemcpyDeviceToDevice, stream);
-        } else if (e == cudaSuccess) { // unusually deep tree: keep the big array itself
-            s->allocs.push_back(scratch.get());
-            dnodes4 = scratch.release();
-        }
-        if (e != cudaSuccess) {
-            set_error("4-wide BVH collapse failed: %s", cudaGetErrorString(e));
-            return RT_ERR_CUDA;
-        }
-        // ... and the 64-byte quantised form of the same nodes (kept only when every node is representable)
-        if (n_nodes4 && !getenv("RT_NO_BVH4Q")) {
-            if ((st = dev_alloc(s, &dnodes4q, n_nodes4)) != RT_OK) return st;
-            bool quant_ok = false;
-            e = rtd::bvh_quantize4(dnodes4, n_nodes4, dnodes4q, &quant_ok, stream);
-            if (e != cudaSuccess) {
-                set_error("4-wide BVH quantisation failed: %s", cudaGetErrorString(e));
-                return RT_ERR_CUDA;
-            }
-            s->nodes4q_mem = dnodes4q;
-            if (!quant_ok) dnodes4q = nullptr; // (the memory stays with the scene; the walk uses the 128-byte nodes)
-        }
-    }
-    if (bstats.depth > RT_BVH_STACK_DEPTH) {
-        set_error("BVH depth %u exceeds the traversal stack (%d)", bstats.depth, RT_BVH_STACK_DEPTH);
-        return RT_ERR_UNSUPPORTED;
-    }
-
-    std::vector<rtd::DMaterial> hm(desc->n_materials);
-    for (uint32_t i = 0; i < desc->n_materials; ++i) hm[i] = rtd::pack_material(desc->materials[i]);
-    std::vector<rtd::DTexture> ht(desc->n_textures);
-    for (uint32_t i = 0; i < desc->n_textures; ++i) {
-        const rt_texture& t = desc->textures[i];
-        ht[i] = rtd::DTexture{t.kind,      t.even,      t.odd,       t.image,   t.color1[0], t.color1[1],
-                              t.color1[2], t.density,   t.color2[0], t.color2[1], t.color2[2], t.hardness};
-    }
-    if ((st = dev_alloc(s, &dmats, hm.size())) != RT_OK) return st;
-    if ((st = dev_alloc(s, &dtexs, ht.size())) != RT_OK) return st;
-    if (!hm.empty()) CUDA_TRY(cudaMemcpyAsync(dmats, hm.data(), hm.size() * sizeof(rtd::DMaterial), cudaMemcpyHostToDevice, stream));
-    if (!ht.empty()) CUDA_TRY(cudaMemcpyAsync(dtexs, ht.data(), ht.size() * sizeof(rtd::DTexture), cudaMemcpyHostToDevice, stream));
-
-    // ---- image textures: float RGB -> float4 cudaArray + point-sampled texture object ----
-    for (uint32_t i = 0; i < desc->n_images; ++i) {
-        const rt_image& im = desc->images[i];
-        const size_t texels = size_t(im.width) * size_t(im.height);
-        rtd::PoolBuffer<float> d_rgb;
-        rtd::PoolBuffer<float4> d_rgba;
-        CUDA_TRY(d_rgb.alloc(texels * 3, stream));
-        cudaError_t e = d_rgba.alloc(texels, stream);
-        if (e != cudaSuccess) {
-            set_error("cudaMallocAsync(image staging) failed: %s", cudaGetErrorString(e));
-            return RT_ERR_OOM;
-        }
-        cudaArray_t arr = nullptr;
-        {
-            std::lock_guard<std::mutex> lock(ctx->cache_mutex);
-            for (size_t k = 0; k < ctx->array_cache.size(); ++k)
-                if (ctx->array_cache[k].width == im.width && ctx->array_cache[k].height == im.height) {
-                    arr = ctx->array_cache[k].arr;
-                    ctx->array_cache.erase(ctx->array_cache.begin() + long(k));
-                    break;
-                }
-        }
-        cudaChannelFormatDesc cd = cudaCreateChannelDesc<float4>();
-        e = cudaMemcpyAsync(d_rgb.get(), im.rgb, texels * 3 * sizeof(float), cudaMemcpyHostToDevice, stream);
-        if (e == cudaSuccess) {
-            rtd::launch_rgb_to_rgba(d_rgb.get(), d_rgba.get(), texels, ctx->sm_count, stream);
-            if (!arr) e = cudaMallocArray(&arr, &cd, size_t(im.width), size_t(im.height));
-        }
-        if (e == cudaSuccess) {
-            s->arrays.push_back(rt_context::CachedArray{im.width, im.height, arr});
-            e = cudaMemcpy2DToArrayAsync(arr, 0, 0, d_rgba.get(), size_t(im.width) * sizeof(float4), size_t(im.width) * sizeof(float4),
-                                         size_t(im.height), cudaMemcpyDeviceToDevice, stream);
-        }
-        if (e != cudaSuccess) {
-            set_error("image texture upload failed: %s", cudaGetErrorString(e));
-            return RT_ERR_CUDA;
-        }
-        cudaResourceDesc rd{};
-        rd.resType = cudaResourceTypeArray;
-        rd.res.array.array = arr;
-        cudaTextureDesc td{};
-        td.addressMode[0] = td.addressMode[1] = cudaAddressModeClamp;
-        td.filterMode = cudaFilterModePoint;
-        td.readMode = cudaReadModeElementType;
-        td.normalizedCoords = 0;
-        cudaTextureObject_t tex = 0;
-        CUDA_TRY(cudaCreateTextureObject(&tex, &rd, &td, nullptr));
-        s->texobjs.push_back(tex);
-        s->d.images[i] = rtd::DImage{tex, im.width, im.height};
-        s->info.device_bytes += texels * sizeof(float4);
-    }
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    CUDA_TRY(cudaGetLastError());
-
-    s->d.sph_a = da;
-    s->d.sph_b = db;
-    s->d.sph_c = dc;
-    s->d.n_spheres = n;
-    s->d.n_static = n_static;
-    s->d.nodes = dnodes;
-    s->d.nodes_ch = dnodes_ch;
-    s->d.nodes4 = dnodes4;
-    s->d.nodes4q = dnodes4q;
-    s->d.n_nodes4 = n_nodes4;
-    s->d.root4 = root4;
-    s->d.n_nodes = n_nodes;
-    s->d.root = bvh_root;
-    s->d.mats = dmats;
-    s->d.texs = dtexs;
-    s->d.n_list = 0;
-    if (mode == RT_BVH_NONE && n != 0 && n <= RT_LIST_MAX) { // the list in the constant bank (DScene::lst_*)
-        s->d.n_list = n;
-        for (uint32_t k = 0; k < n; ++k) {
-            s->d.lst_a[k] = ha[k];
-            s->d.lst_b[k] = hb[k];
-            memcpy(&s->d.lst_dt[k], &hc[k].x, 4);
-        }
-    }
-    s->d.has_noise = 0;
-    for (const auto& t : ht)
-        if (t.kind == RT_TEX_NOISE_PERLIN || t.kind == RT_TEX_NOISE_TURBULANCE || t.kind == RT_TEX_NOISE_MARBLE || t.kind == RT_TEX_WOOD) s->d.has_noise = 1;
-    rtd::make_camera(desc->camera, s->d.cam);
-    s->where.resize(n); // list ordinal -> device index
-    for (uint32_t k = 0; k < n; ++k) s->where[order[k]] = k;
-    s->sphere_material.resize(n);
-    for (uint32_t i = 0; i < n; ++i) s->sphere_material[i] = desc->spheres[i].material;
-    s->material_kind.resize(desc->n_materials);
-    for (uint32_t i = 0; i < desc->n_materials; ++i) s->material_kind[i] = desc->materials[i].kind;
-    s->n_textures = desc->n_textures;
-    rtd::find_lights(s);
-
-    const auto t_end = std::chrono::steady_clock::now();
-    s->info.n_spheres = n;
-    s->info.n_nodes = n_nodes;
-    s->info.bvh_mode = mode;
-    s->info.bvh_depth = bstats.depth;
-    s->info.sah_cost = bstats.sah_cost;
-    s->info.ms_build = mode == RT_BVH_GPU_LBVH ? lbvh_ms
-                                               : std::chrono::duration<float, std::milli>(t_build1 - t_build0).count();
-    s->info.ms_upload = std::chrono::duration<float, std::milli>(t_end - t_begin).count() -
-                        std::chrono::duration<float, std::milli>(t_build1 - t_build0).count();
-    guard.s = nullptr;
-    *out = s;
-    return RT_OK;
-} RT_API_CATCH
-
-void rt_scene_destroy(rt_scene* scene) {
-    if (!scene) return;
-    if (scene->ctx) cudaSetDevice(scene->ctx->device);
-    // the scene's kernels are ordered before these on the context stream
-    for (auto t : scene->texobjs) cudaDestroyTextureObject(t);
-    for (auto& a : scene->arrays) {
-        bool kept = false;
-        if (scene->ctx) {
-            std::lock_guard<std::mutex> lock(scene->ctx->cache_mutex);
-            if (scene->ctx->array_cache.size() < 8) {
-                scene->ctx->array_cache.push_back(a);
-                kept = true;
-            }
-        }
-        if (!kept) cudaFreeArray(a.arr);
-    }
-    for (auto p : scene->allocs) {
-        if (scene->ctx) cudaFreeAsync(p, scene->ctx->stream);
-        else cudaFree(p);
-    }
-    delete scene;
-}
-
-rt_status rt_scene_get_info(const rt_scene* scene, rt_scene_info* info) try {
-    ARG_CHECK(scene && info, "scene/info is NULL");
-    *info = scene->info;
     return RT_OK;
 } RT_API_CATCH
 

@@ -1,5 +1,5 @@
-// rt_internal.hpp — the opaque handles of include/rt_api.h, shared by the translation units that implement the C-ABI
-// (rt_api.cu: contexts, scenes, render entries; rt_multi.cu: the multi-GPU entries; rt_selftest.cu: the primitives' tests).
+// rt_internal.hpp — the opaque handles of include/rt_api.h, shared by the translation units that implement the C-ABI (rt_api.cu:
+// contexts, render entries; rt_scene.cu: scenes; rt_multi.cu: the multi-GPU entries; rt_selftest.cu: the primitives' tests).
 #pragma once
 
 #include <cuda_runtime.h>
@@ -58,14 +58,14 @@ struct rt_scene {
     std::vector<void*> allocs;
     std::vector<rt_context::CachedArray> arrays;
     std::vector<cudaTextureObject_t> texobjs;
-    // what rt_scene_update (rt_update.cu) needs of the creation description: the device index of every list ordinal, the
+    // what rt_scene_update needs of the creation description: the device index of every list ordinal, the
     // material of every sphere (list order), the kind of every material, and the texture count
     std::vector<uint32_t> where;
     std::vector<uint32_t> sphere_material;
     std::vector<uint32_t> material_kind;
     uint32_t n_textures = 0;
     rtd::BvhNode4Q* nodes4q_mem = nullptr; // the quantised nodes' allocation, also when d.nodes4q is nullptr
-    int* parents = nullptr; // rt_update.cu: parent of every inner node, then of every primitive (built on the first refit)
+    int* parents = nullptr; // parent of every inner node, then of every primitive (built on the first refit)
 };
 
 namespace rtd {
@@ -76,18 +76,6 @@ inline rt_status make_current(const rt_context* ctx) {
     return RT_OK;
 }
 
-// rt_api.cu, shared by rt_scene_create and rt_scene_update:
-// the per-sphere and per-material rules of a scene description
-rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials);
-rt_status check_material(const rt_material& m, uint32_t n_textures);
-// the device records (sph_a, sph_b, sph_c) of `count` spheres: record k is sphere spheres[src ? src[k] : k], whose list
-// ordinal is ordinal[k]
-void pack_spheres(const rt_sphere* spheres, const uint32_t* src, const uint32_t* ordinal, size_t count, float4* a, float4* b,
-                  uint4* c);
-DMaterial pack_material(const rt_material& m);
-// the emitter spheres for RT_RENDER_EMITTER_SAMPLING (DScene::lights: device indices, the first RT_MAX_LIGHTS in list order)
-// from the scene's sphere_material / material_kind mirrors
-void find_lights(rt_scene* s);
 // camera ctor (camera.h:7-31) in host float arithmetic
 void make_camera(const rt_camera& c, DCamera& out);
 } // namespace rtd

@@ -23,7 +23,52 @@ __device__ __forceinline__ float unflip_f(unsigned u) {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
-// Primitive bounds (prim_box, rt_lbvh.cuh) and their centroid bounds.
+// Bounds of primitive `prim` (sphere.h:142-146; moving: union of the boxes at both ends of the motion, sphere.h:192-202),
+// padded exactly like the host builder (rt_bvh_host.cpp sphere_box) so the conservative slab test never rejects a ray the
+// rounded sphere test accepts.  The LBVH build (k_prim_boxes) and the refit of a resident tree (k_refit_all) both use it.
+__device__ __forceinline__ void prim_box(const float4* __restrict__ sph_a, const float4* __restrict__ sph_b, uint32_t prim,
+                                         uint32_t n_static, float l[3], float h[3]) {
+    float4 a = __ldg(&sph_a[prim]);
+    float c0[3] = {a.x, a.y, a.z}, c1[3] = {a.x, a.y, a.z};
+    if (prim >= n_static) {
+        float4 b = __ldg(&sph_b[prim]);
+        c1[0] = __fadd_rz(a.x, b.x); // where moving_center() puts the sphere at the end of its motion
+        c1[1] = __fadd_rz(a.y, b.y);
+        c1[2] = __fadd_rz(a.z, b.z);
+    }
+    float ar = fabsf(a.w);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        float lk = fminf(c0[k], c1[k]) - ar, hk = fmaxf(c0[k], c1[k]) + ar;
+        float pad = ar * 6.1035156e-5f + (fabsf(lk) + fabsf(hk)) * 3.8146973e-6f;
+        l[k] = lk - pad;
+        h[k] = hk + pad;
+    }
+}
+
+// One step of the bottom-up refit, run by one thread per leaf: the thread writes its subtree's box (bl, bh) into its side of
+// node `parent` (the side whose child reference is `me`).  The first thread to reach a node returns false; the second, which
+// then sees both child boxes, returns true with their union in (bl, bh) and carries it on to the node's parent.
+__device__ __forceinline__ bool refit_step(BvhNode* nodes, int parent, int me, float4& bl, float4& bh, unsigned* visits) {
+    BvhNode* nd = nodes + parent;
+    volatile float* f = reinterpret_cast<volatile float*>(nd);
+    int left = reinterpret_cast<const int*>(&nd->lmin)[3];
+    if (left == me) {
+        f[0] = bl.x; f[1] = bl.y; f[2] = bl.z;
+        f[4] = bh.x; f[5] = bh.y; f[6] = bh.z;
+    } else {
+        f[8] = bl.x; f[9] = bl.y; f[10] = bl.z; f[11] = 0.f;
+        f[12] = bh.x; f[13] = bh.y; f[14] = bh.z; f[15] = 0.f;
+    }
+    __threadfence();
+    if (atomicAdd(&visits[parent], 1u) == 0u) return false; // sibling subtree not finished yet
+    __threadfence();
+    bl = make_float4(fminf(f[0], f[8]), fminf(f[1], f[9]), fminf(f[2], f[10]), 0.f);
+    bh = make_float4(fmaxf(f[4], f[12]), fmaxf(f[5], f[13]), fmaxf(f[6], f[14]), 0.f);
+    return true;
+}
+
+// Primitive bounds (prim_box) and their centroid bounds.
 __global__ void __launch_bounds__(256) k_prim_boxes(const float4* __restrict__ sph_a, const float4* __restrict__ sph_b,
                                                     const uint32_t* __restrict__ ids, uint32_t n, uint32_t n_static,
                                                     float4* __restrict__ lo, float4* __restrict__ hi,
@@ -176,6 +221,39 @@ __global__ void __launch_bounds__(256) k_depth(int n, const int* __restrict__ pa
     }
     d = __reduce_max_sync(0xffffffffu, d);
     if ((threadIdx.x & 31) == 0) atomicMax(max_depth, d);
+}
+
+// The parent table of a binary node array (host SAH tree, LBVH, and the chain of outsized spheres above the LBVH root alike:
+// one primitive per leaf, child < 0 is leaf ~prim): parent_inner[i] for every node, parent_leaf[p] for every primitive.
+// Both are -1 before this kernel; the root keeps -1.
+__global__ void __launch_bounds__(256) k_parents(const BvhNode* __restrict__ nodes, uint32_t n_nodes, int* __restrict__ parent_inner,
+                                                 int* __restrict__ parent_leaf) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_nodes) return;
+    const float4* np = reinterpret_cast<const float4*>(nodes + i);
+    const int child[2] = {__float_as_int(np[0].w), __float_as_int(np[1].w)};
+#pragma unroll
+    for (int c = 0; c < 2; ++c) {
+        if (child[c] >= 0) parent_inner[child[c]] = int(i);
+        else parent_leaf[~child[c]] = int(i);
+    }
+}
+
+// One thread per primitive: its padded box (prim_box, as the builders pad it), then up the tree with the visit-counter
+// protocol of the LBVH build's k_refit.  Every node is written on both sides, so no box of the old tree survives.
+__global__ void __launch_bounds__(256) k_refit_all(const float4* __restrict__ sph_a, const float4* __restrict__ sph_b, uint32_t n,
+                                                   uint32_t n_static, BvhNode* nodes, const int* __restrict__ parent_inner,
+                                                   const int* __restrict__ parent_leaf, unsigned* __restrict__ visits) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    float l[3], h[3];
+    prim_box(sph_a, sph_b, k, n_static, l, h);
+    float4 bl = make_float4(l[0], l[1], l[2], 0.f), bh = make_float4(h[0], h[1], h[2], 0.f);
+    int me = ~int(k);
+    for (int parent = parent_leaf[k]; parent >= 0; parent = parent_inner[parent]) {
+        if (!refit_step(nodes, parent, me, bl, bh, visits)) return;
+        me = parent;
+    }
 }
 
 // Binary -> 4-wide: node i of the 4-wide array is binary node i with each inner child replaced by that child's two
@@ -455,6 +533,27 @@ cudaError_t lbvh_build(const float4* sph_a, const float4* sph_b, uint32_t n_stat
     if (ms) RTD_TRY(cudaEventElapsedTime(ms, e0.ev, e1.ev));
     if (depth) *depth = d;
     return cudaSuccess;
+}
+
+cudaError_t bvh_parents(const BvhNode* nodes, uint32_t n_nodes, uint32_t n_prims, int* parents, uint32_t* levels, cudaStream_t st) {
+    PoolBuffer<unsigned> d_levels;
+    RTD_TRY(d_levels.alloc(1, st));
+    RTD_TRY(cudaMemsetAsync(parents, 0xff, (size_t(n_nodes) + n_prims) * sizeof(int), st));
+    RTD_TRY(cudaMemsetAsync(d_levels.get(), 0, sizeof(unsigned), st));
+    k_parents<<<(n_nodes + 255) / 256, 256, 0, st>>>(nodes, n_nodes, parents, parents + n_nodes);
+    k_depth<<<(n_prims + 255) / 256, 256, 0, st>>>(int(n_prims), parents, parents + n_nodes, d_levels.get());
+    RTD_TRY(cudaGetLastError());
+    RTD_TRY(cudaMemcpyAsync(levels, d_levels.get(), sizeof *levels, cudaMemcpyDeviceToHost, st));
+    return cudaStreamSynchronize(st);
+}
+
+cudaError_t bvh_refit(const float4* sph_a, const float4* sph_b, uint32_t n, uint32_t n_static, BvhNode* nodes, uint32_t n_nodes,
+                      const int* parents, cudaStream_t st) {
+    PoolBuffer<unsigned> visits;
+    RTD_TRY(visits.alloc(n_nodes, st));
+    RTD_TRY(cudaMemsetAsync(visits.get(), 0, n_nodes * sizeof(unsigned), st));
+    k_refit_all<<<(n + 255) / 256, 256, 0, st>>>(sph_a, sph_b, n, n_static, nodes, parents, parents + n_nodes, visits.get());
+    return cudaGetLastError();
 }
 
 } // namespace rtd

@@ -22,49 +22,11 @@ cudaError_t bvh_quantize4(const BvhNode4* nodes4, uint32_t n4, BvhNode4Q* out_q,
 cudaError_t bvh_collapse4(const BvhNode* nodes, uint32_t n_nodes, uint32_t root, uint32_t depth, BvhNode4* out, uint32_t* n_out,
                           uint32_t* root_out, cudaStream_t st);
 
-// Bounds of primitive `prim` (sphere.h:142-146; moving: union of the boxes at both ends of the motion, sphere.h:192-202),
-// padded exactly like the host builder (rt_bvh_host.cpp sphere_box) so the conservative slab test never rejects a ray the
-// rounded sphere test accepts.  The LBVH build (k_prim_boxes) and the scene update's refit (rt_update.cu) both use it.
-__device__ __forceinline__ void prim_box(const float4* __restrict__ sph_a, const float4* __restrict__ sph_b, uint32_t prim,
-                                         uint32_t n_static, float l[3], float h[3]) {
-    float4 a = __ldg(&sph_a[prim]);
-    float c0[3] = {a.x, a.y, a.z}, c1[3] = {a.x, a.y, a.z};
-    if (prim >= n_static) {
-        float4 b = __ldg(&sph_b[prim]);
-        c1[0] = __fadd_rz(a.x, b.x); // where moving_center() puts the sphere at the end of its motion
-        c1[1] = __fadd_rz(a.y, b.y);
-        c1[2] = __fadd_rz(a.z, b.z);
-    }
-    float ar = fabsf(a.w);
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        float lk = fminf(c0[k], c1[k]) - ar, hk = fmaxf(c0[k], c1[k]) + ar;
-        float pad = ar * 6.1035156e-5f + (fabsf(lk) + fabsf(hk)) * 3.8146973e-6f;
-        l[k] = lk - pad;
-        h[k] = hk + pad;
-    }
-}
-
-// One step of the bottom-up refit, run by one thread per leaf: the thread writes its subtree's box (bl, bh) into its side of
-// node `parent` (the side whose child reference is `me`).  The first thread to reach a node returns false; the second, which
-// then sees both child boxes, returns true with their union in (bl, bh) and carries it on to the node's parent.
-__device__ __forceinline__ bool refit_step(BvhNode* nodes, int parent, int me, float4& bl, float4& bh, unsigned* visits) {
-    BvhNode* nd = nodes + parent;
-    volatile float* f = reinterpret_cast<volatile float*>(nd);
-    int left = reinterpret_cast<const int*>(&nd->lmin)[3];
-    if (left == me) {
-        f[0] = bl.x; f[1] = bl.y; f[2] = bl.z;
-        f[4] = bh.x; f[5] = bh.y; f[6] = bh.z;
-    } else {
-        f[8] = bl.x; f[9] = bl.y; f[10] = bl.z; f[11] = 0.f;
-        f[12] = bh.x; f[13] = bh.y; f[14] = bh.z; f[15] = 0.f;
-    }
-    __threadfence();
-    if (atomicAdd(&visits[parent], 1u) == 0u) return false; // sibling subtree not finished yet
-    __threadfence();
-    bl = make_float4(fminf(f[0], f[8]), fminf(f[1], f[9]), fminf(f[2], f[10]), 0.f);
-    bh = make_float4(fmaxf(f[4], f[12]), fmaxf(f[5], f[13]), fmaxf(f[6], f[14]), 0.f);
-    return true;
-}
+// parent table of a finished binary node array: parents[i] of node i, then parents[n_nodes + p] of primitive p (root: -1);
+// levels: the depth of its deepest leaf (synchronises)
+cudaError_t bvh_parents(const BvhNode* nodes, uint32_t n_nodes, uint32_t n_prims, int* parents, uint32_t* levels, cudaStream_t st);
+// every box of the binary node array from the current primitives, bottom-up along the parent table; the topology stays
+cudaError_t bvh_refit(const float4* sph_a, const float4* sph_b, uint32_t n, uint32_t n_static, BvhNode* nodes, uint32_t n_nodes,
+                      const int* parents, cudaStream_t st);
 
 } // namespace rtd

@@ -340,16 +340,17 @@ RT_API_CATCH
 
 extern "C" int32_t rt_multi_size(const rt_multi* m) { return m ? m->n : 0; }
 
-extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) try {
-    ARG_CHECK(m && desc, "multi/desc is NULL");
+namespace {
+// call(k) for every member k, side by side on one host thread each; the first failing member's status, with its device
+// in the message
+template <class Call>
+rt_status each_member(rt_multi* m, Call&& call) {
     std::vector<rt_status> st(m->n, RT_OK);
     std::vector<std::string> msg(m->n);
     std::vector<std::thread> th;
     for (int k = 0; k < m->n; ++k)
-        th.emplace_back([&, k] { // uploads + BVH builds of the devices run side by side
-            if (m->scene[k]) rt_scene_destroy(m->scene[k]);
-            m->scene[k] = nullptr;
-            st[k] = rt_scene_create(m->ctx[k], desc, &m->scene[k]);
+        th.emplace_back([&, k] {
+            st[k] = call(k);
             if (st[k] != RT_OK) msg[k] = rt_last_error();
         });
     for (auto& t : th) t.join();
@@ -360,26 +361,22 @@ extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) 
         }
     return RT_OK;
 }
+} // namespace
+
+extern "C" rt_status rt_multi_set_scene(rt_multi* m, const rt_scene_desc* desc) try {
+    ARG_CHECK(m && desc, "multi/desc is NULL");
+    return each_member(m, [&](int k) { // uploads + BVH builds of the devices run side by side
+        if (m->scene[k]) rt_scene_destroy(m->scene[k]);
+        m->scene[k] = nullptr;
+        return rt_scene_create(m->ctx[k], desc, &m->scene[k]);
+    });
+}
 RT_API_CATCH
 
 extern "C" rt_status rt_multi_update_scene(rt_multi* m, const rt_scene_edit* edit) try {
     ARG_CHECK(m && edit, "multi/edit is NULL");
     for (int k = 0; k < m->n; ++k) ARG_CHECK(m->scene[k] != nullptr, "no scene: call rt_multi_set_scene first");
-    std::vector<rt_status> st(m->n, RT_OK);
-    std::vector<std::string> msg(m->n);
-    std::vector<std::thread> th;
-    for (int k = 0; k < m->n; ++k)
-        th.emplace_back([&, k] { // the updates of the devices run side by side
-            st[k] = rt_scene_update(m->ctx[k], m->scene[k], edit, nullptr);
-            if (st[k] != RT_OK) msg[k] = rt_last_error();
-        });
-    for (auto& t : th) t.join();
-    for (int k = 0; k < m->n; ++k)
-        if (st[k] != RT_OK) {
-            rtd::set_error("device %d: %s", m->ctx[k]->device, msg[k].c_str());
-            return st[k];
-        }
-    return RT_OK;
+    return each_member(m, [&](int k) { return rt_scene_update(m->ctx[k], m->scene[k], edit, nullptr); });
 }
 RT_API_CATCH
 

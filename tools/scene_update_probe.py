@@ -38,7 +38,7 @@ WALK_STEPS = (1, 10, 100)
 FRAME = dict(width=1920, height=1080, spp=16)
 PHASES = [  # (phase, substrings of the kernel / activity names it issues)
     ("records (copies + scatter)", ("k_scatter", "Memcpy HtoD")),
-    ("refit", ("k_refit_all", "k_parents", "k_levels", "Memset")),
+    ("refit", ("k_refit_all", "k_parents", "k_depth", "Memset")),
     ("centre/half-extent nodes", ("k_nodes_ch",)),
     ("4-wide collapse", ("k_collapse4", "k_mark4", "k_used4", "k_compact4", "scan", "Memcpy DtoD", "Memcpy DtoH")),
     ("quantisation", ("k_quantize4",)),
