@@ -290,6 +290,24 @@ typedef struct rt_scene_edit {
  * Returns when the update is complete.  ms_device (may be NULL): device time of the update.  A CUDA error during the
  * update (RT_ERR_CUDA / RT_ERR_OOM) leaves the scene unusable: destroy it. */
 rt_status rt_scene_update(rt_context* ctx, rt_scene* scene, const rt_scene_edit* edit, float* ms_device);
+/* rt_scene_update of an edit that has only spheres, read from DEVICE memory: for a simulation whose sphere state lives on
+ * the GPU (no copy to the host and back per step).  The records are checked, packed and scattered on the device; after
+ * RT_OK the scene equals rt_scene_create of its description with the edit applied, and what rt_scene_update of the same
+ * records gives.  Materials and the camera stay with rt_scene_update.
+ * sphere_index_dev: n_spheres list ordinals (uint32, 4-byte aligned); spheres_dev: n_spheres rt_sphere records (16-byte
+ * aligned).  Both are device or managed memory of ctx's device and at least n_spheres elements long (not checkable: the
+ * caller's guarantee).  n_spheres = 0 is a valid no-op without device work; the pointers may then be NULL.
+ * Checked on the host before any device work: NULLs, ctx not the scene's context, a pointer that is not device or managed
+ * memory of ctx's device (never handed to a kernel), the alignments.  Checked on the device before anything of the scene
+ * is written: the sphere rules of rt_scene_update (index in range, not repeated, RT_SPHERE_MOVING unchanged, material in
+ * range, centre / radius / times finite).  The failure reported is the one rt_scene_update would report: the lowest
+ * failing position, its first rule in that order.  RT_ERR_INVALID_ARG leaves the scene unchanged.
+ * Ordering: the records are read on ctx's stream after the work queued there before the call (a render enqueued before
+ * the call renders the old scene).  Records written on another stream (e.g. torch's current stream) must be ordered
+ * before the call by the caller: rt_context_set_stream to that stream, or a synchronise.  Returns when the update is
+ * complete; the caller may then overwrite both buffers.  ms_device and CUDA errors: as for rt_scene_update. */
+rt_status rt_scene_update_device(rt_context* ctx, rt_scene* scene, const uint32_t* sphere_index_dev,
+                                 const rt_sphere* spheres_dev, uint32_t n_spheres, float* ms_device);
 
 /* Parity hook: closest hit of scene.hit(r, tmin, FLT_MAX) (hitable_list.h:60-79)
  * for n caller-supplied rays.  use_bvh = 0 forces the brute-force list path, 1 walks the binary BVH

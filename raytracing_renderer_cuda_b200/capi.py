@@ -151,6 +151,7 @@ _SIGNATURES = {
     "rt_scene_destroy": (None, [_VP]),
     "rt_scene_get_info": (C.c_int, [_VP, C.POINTER(rt_scene_info)]),
     "rt_scene_update": (C.c_int, [_VP, _VP, C.POINTER(rt_scene_edit), C.POINTER(C.c_float)]),
+    "rt_scene_update_device": (C.c_int, [_VP, _VP, _VP, _VP, C.c_uint32, C.POINTER(C.c_float)]),
     "rt_trace_primary": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_float, C.c_int, _VP]),
     "rt_selftest_rz": (C.c_int, [_VP, _VP, _VP, C.c_size_t, _VP]),
     "rt_selftest_exclusive_sum": (C.c_int, [_VP, _VP, _VP, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
@@ -425,6 +426,33 @@ class Scene:
         del keep
         return ms.value
 
+    def update_device(self, sphere_index, spheres) -> float:
+        """rt_scene_update_device: replaces the spheres at list positions `sphere_index` (torch int32 / uint32, shape (n,))
+        with `spheres` (torch float32 (n, 12) or uint8 (n, 48) rt_sphere records, e.g. from sphere_records), both contiguous
+        CUDA tensors on the context's device.  The records are read on the context's stream: work of another stream that
+        writes them must be ordered first (Context.set_stream, or a synchronise).  Returns the device time in ms."""
+        import torch
+
+        if not (isinstance(sphere_index, torch.Tensor) and isinstance(spheres, torch.Tensor)):
+            raise TypeError("sphere_index and spheres must be torch tensors")
+        n = sphere_index.shape[0] if sphere_index.dim() == 1 else -1
+        args = (("sphere_index", sphere_index, (torch.int32, torch.uint32), (n,)),
+                ("spheres", spheres, (torch.float32, torch.uint8), (n, 12 if spheres.dtype == torch.float32 else 48)))
+        for name, t, dtypes, shape in args:
+            if t.dtype not in dtypes:
+                raise TypeError(f"{name}: dtype {t.dtype}, expected one of {dtypes}")
+            if tuple(t.shape) != shape:
+                raise ValueError(f"{name}: shape {tuple(t.shape)}, expected {shape}")
+        for name, t, _, _ in args:
+            if t.device != torch.device("cuda", self.ctx.device):
+                raise ValueError(f"{name}: on {t.device}, expected cuda:{self.ctx.device}")
+            if not t.is_contiguous():
+                raise ValueError(f"{name}: not contiguous")
+        ms = C.c_float()
+        _check(self.lib, self.lib.rt_scene_update_device(self.ctx._h, self._h, _VP(sphere_index.data_ptr() or None),
+                                                         _VP(spheres.data_ptr() or None), n, C.byref(ms)))
+        return ms.value
+
     def trace_primary(self, rays: np.ndarray, tmin: float = 1e-5, use_bvh: bool | int = True) -> np.ndarray:
         rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
         hits = np.zeros(rays.shape[0], dtype=HIT_DTYPE)
@@ -550,6 +578,36 @@ class Scene:
             self.close()
         except Exception:
             pass
+
+
+def sphere_records(center0, radius, center1=None, time0=0.0, time1=0.0, material=0, id=0, flags=None):
+    """rt_sphere records as a float32 (n, 12) torch tensor on center0's device (the input of Scene.update_device), built
+    with torch operations only.  center0 / center1: (n, 3); the other fields: (n,) tensors or scalars.  center1 defaults to
+    center0; flags defaults to RT_SPHERE_MOVING where center1 is given, else 0.  The uint32 fields are written through
+    an int32 view (values of 2^31 and above wrap, giving the same bits)."""
+    import torch
+
+    c0 = torch.as_tensor(center0)
+    n = c0.shape[0]
+    out = torch.empty((n, 12), dtype=torch.float32, device=c0.device)
+    bits = out.view(torch.int32)
+
+    def u32(v):
+        if isinstance(v, torch.Tensor):
+            v = v.to(device=c0.device, dtype=torch.int64)
+            return ((v + 2**31) % 2**32 - 2**31).to(torch.int32)
+        v = int(v) % 2**32
+        return v - 2**32 if v >= 2**31 else v
+
+    out[:, 0:3] = c0
+    out[:, 3] = radius
+    out[:, 4:7] = c0 if center1 is None else center1
+    out[:, 7] = time0
+    out[:, 8] = time1
+    bits[:, 9] = u32(material)
+    bits[:, 10] = u32(id)
+    bits[:, 11] = u32(RT_SPHERE_MOVING if center1 is not None else 0) if flags is None else u32(flags)
+    return out
 
 
 def scene_edit(sphere_index=None, spheres=None, material_index=None, materials=None, camera: "rt_camera | None" = None):

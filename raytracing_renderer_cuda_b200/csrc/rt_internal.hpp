@@ -58,14 +58,14 @@ struct rt_scene {
     std::vector<void*> allocs;
     std::vector<rt_context::CachedArray> arrays;
     std::vector<cudaTextureObject_t> texobjs;
-    // what rt_scene_update needs of the creation description: the device index of every list ordinal, the
-    // material of every sphere (list order), the kind of every material, and the texture count
+    // what rt_scene_update needs of the creation description: the device index of every list ordinal, and the material
+    // and texture counts
     std::vector<uint32_t> where;
-    std::vector<uint32_t> sphere_material;
-    std::vector<uint32_t> material_kind;
+    uint32_t n_materials = 0;
     uint32_t n_textures = 0;
     rtd::BvhNode4Q* nodes4q_mem = nullptr; // the quantised nodes' allocation, also when d.nodes4q is nullptr
     int* parents = nullptr; // parent of every inner node, then of every primitive (built on the first refit)
+    uint32_t* where_dev = nullptr; // `where` on the device (built on the first rt_scene_update_device, from sph_c.w)
 };
 
 namespace rtd {

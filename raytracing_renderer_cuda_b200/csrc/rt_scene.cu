@@ -1,7 +1,7 @@
 // rt_scene.cu — a scene's lifetime: rt_scene_create (validation, the packed sphere records, the binary tree, the node forms
 // derived from it, materials, textures and image arrays), rt_scene_update (edits of sphere records, material records and the
-// camera of a resident scene, and the refit of every node form of its tree on the device), rt_scene_get_info and
-// rt_scene_destroy.  An update keeps the tree's topology as it was built; only its boxes change (DESIGN.md "Scene updates").
+// camera of a resident scene, and the refit of every node form of its tree on the device), rt_scene_update_device (sphere
+// edits read, checked, packed and scattered on the device, then the same refit), rt_scene_get_info and rt_scene_destroy.  An update keeps the tree's topology as it was built; only its boxes change (DESIGN.md "Scene updates").
 #include <algorithm>
 #include <cfenv>
 #include <chrono>
@@ -13,6 +13,7 @@
 #include "rt_bvh_host.hpp"
 #include "rt_internal.hpp"
 #include "rt_lbvh.cuh"
+#include "rt_prims.cuh"
 
 namespace rtd {
 namespace {
@@ -41,7 +42,13 @@ rt_status dev_alloc(rt_scene* s, T** out, size_t count) {
     return RT_OK;
 }
 
-bool finite3(const float* v) { return std::isfinite(v[0]) && std::isfinite(v[1]) && std::isfinite(v[2]); }
+// (an exponent field below all ones: the same test in host and device code)
+__host__ __device__ bool finite1(float x) {
+    uint32_t u;
+    memcpy(&u, &x, 4);
+    return (u & 0x7f800000u) != 0x7f800000u;
+}
+__host__ __device__ bool finite3(const float* v) { return finite1(v[0]) && finite1(v[1]) && finite1(v[2]); }
 
 rt_status check_material(const rt_material& m, uint32_t n_textures) {
     ARG_CHECK(m.kind <= RT_MAT_EMITTER, "bad material kind");
@@ -50,12 +57,35 @@ rt_status check_material(const rt_material& m, uint32_t n_textures) {
     return RT_OK;
 }
 
-rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials) {
+// The rules of an edited sphere, in the order they are checked; a description's spheres are checked by the last two.
+// One definition for the host checks (check_sphere, check_edit) and the device check of rt_scene_update_device (k_check).
+enum SphereRule : uint32_t { SPH_OK, SPH_INDEX_RANGE, SPH_REPEATED, SPH_KIND, SPH_MATERIAL, SPH_NOT_FINITE };
+const char* const kSphereRuleMessage[] = {
+    "", "sphere index out of range", "sphere index repeated",
+    "an edit cannot make a static sphere moving or a moving one static", // (static spheres are stored before the moving ones)
+    "sphere material out of range", "sphere centre / radius / time is not finite"};
+
+__host__ __device__ uint32_t sphere_rule(const rt_sphere& sp, uint32_t n_materials) {
     // non-finite geometry would reach the builders' bin arithmetic (undefined for NaN / infinity) and the slab tests
-    ARG_CHECK(sp.material < n_materials, "sphere material out of range");
-    ARG_CHECK(finite3(sp.center0) && finite3(sp.center1) && std::isfinite(sp.radius) && std::isfinite(sp.time0) &&
-                  std::isfinite(sp.time1),
-              "sphere centre / radius / time is not finite");
+    if (!(sp.material < n_materials)) return SPH_MATERIAL;
+    if (!(finite3(sp.center0) && finite3(sp.center1) && finite1(sp.radius) && finite1(sp.time0) && finite1(sp.time1)))
+        return SPH_NOT_FINITE;
+    return SPH_OK;
+}
+
+// sphere `sp` replacing list ordinal `i` of a scene of `n` spheres; `repeated`: an earlier position of the edit holds `i`;
+// `stored_moving`: the sphere at `i` is stored as a moving one (both read only when i < n)
+__host__ __device__ uint32_t sphere_edit_rule(const rt_sphere& sp, uint32_t i, uint32_t n, bool repeated, bool stored_moving,
+                                              uint32_t n_materials) {
+    if (i >= n) return SPH_INDEX_RANGE;
+    if (repeated) return SPH_REPEATED;
+    if (((sp.flags & RT_SPHERE_MOVING) != 0) != stored_moving) return SPH_KIND;
+    return sphere_rule(sp, n_materials);
+}
+
+rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials) {
+    const uint32_t r = sphere_rule(sp, n_materials);
+    ARG_CHECK(r == SPH_OK, kSphereRuleMessage[r]);
     return RT_OK;
 }
 
@@ -86,7 +116,8 @@ rt_status validate_desc(const rt_scene_desc* d) {
 }
 
 // the device records (sph_a, sph_b, sph_c) of `count` spheres: record k is sphere spheres[src ? src[k] : k], whose list
-// ordinal is ordinal[k]
+// ordinal is ordinal[k].  k_apply packs the records of rt_scene_update_device on the device: the two packers must agree
+// bit for bit (a scene's hits may not depend on which entry wrote its records).
 void pack_spheres(const rt_sphere* spheres, const uint32_t* src, const uint32_t* ordinal, size_t count, float4* a, float4* b,
                   uint4* c) {
     {
@@ -119,14 +150,126 @@ DMaterial pack_material(const rt_material& m) {
     return DMaterial{m.kind, m.texture, m.albedo[0], m.albedo[1], m.albedo[2], m.param, 0.f, 0.f};
 }
 
-// the emitter spheres for RT_RENDER_EMITTER_SAMPLING (DScene::lights: device indices, the first RT_MAX_LIGHTS in list order)
-// from the scene's sphere_material / material_kind mirrors
-void find_lights(rt_scene* s) {
-    s->d.n_lights = 0;
-    const size_t n = s->where.size();
-    for (size_t i = 0; i < n && s->d.n_lights < RT_MAX_LIGHTS; ++i)
-        if (s->material_kind[s->sphere_material[i]] == RT_MAT_EMITTER) s->d.lights[s->d.n_lights++] = s->where[i];
-    for (uint32_t k = s->d.n_lights; k < RT_MAX_LIGHTS; ++k) s->d.lights[k] = 0;
+// ---- rt_scene_update_device: the edit's records are read from device memory, checked, packed and scattered there ----
+
+// one 48-byte rt_sphere as three 16-byte loads (the entry requires 16-byte aligned records)
+__device__ __forceinline__ rt_sphere load_sphere(const rt_sphere* __restrict__ spheres, uint32_t j) {
+    const float4* p = reinterpret_cast<const float4*>(spheres) + 3 * size_t(j);
+    const float4 r0 = p[0], r1 = p[1], r2 = p[2];
+    rt_sphere sp;
+    sp.center0[0] = r0.x, sp.center0[1] = r0.y, sp.center0[2] = r0.z, sp.radius = r0.w;
+    sp.center1[0] = r1.x, sp.center1[1] = r1.y, sp.center1[2] = r1.z, sp.time0 = r1.w;
+    sp.time1 = r2.x, sp.material = __float_as_uint(r2.y), sp.id = __float_as_uint(r2.z), sp.flags = __float_as_uint(r2.w);
+    return sp;
+}
+
+// where[list ordinal] = device index, from the ordinals the records carry
+__global__ void __launch_bounds__(256) k_where(const uint4* __restrict__ sph_c, uint32_t n, uint32_t* __restrict__ where) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n) where[sph_c[k].w] = k;
+}
+
+// claim[i] = the first edit position that names list ordinal i (claim starts at all ones)
+__global__ void __launch_bounds__(256) k_claim(const uint32_t* __restrict__ idx, uint32_t m, uint32_t n, uint32_t* __restrict__ claim) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < m && idx[j] < n) atomicMin(&claim[idx[j]], j);
+}
+
+// *verdict = min over the failing positions j of (j << 8 | rule): the lowest failing position and its first broken rule,
+// whatever order the threads run in (starts at all ones)
+__global__ void __launch_bounds__(256) k_check(const uint32_t* __restrict__ idx, const rt_sphere* __restrict__ spheres, uint32_t m,
+                                               uint32_t n, uint32_t n_static, uint32_t n_materials, const uint32_t* __restrict__ claim,
+                                               const uint32_t* __restrict__ where, unsigned long long* verdict) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= m) return;
+    const uint32_t i = idx[j];
+    const bool in = i < n;
+    const uint32_t rule = sphere_edit_rule(load_sphere(spheres, j), i, n, in && claim[i] < j, in && where[i] >= n_static, n_materials);
+    if (rule != SPH_OK) atomicMin(verdict, (static_cast<unsigned long long>(j) << 8) | rule);
+}
+
+// the checked records, packed as pack_spheres packs them, written at their device indices
+__global__ void __launch_bounds__(256) k_apply(const uint32_t* __restrict__ idx, const rt_sphere* __restrict__ spheres, uint32_t m,
+                                               const uint32_t* __restrict__ where, float4* __restrict__ a, float4* __restrict__ b,
+                                               uint4* __restrict__ c) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= m) return;
+    const uint32_t i = idx[j], k = where[i];
+    const rt_sphere sp = load_sphere(spheres, j);
+    a[k] = make_float4(sp.center0[0], sp.center0[1], sp.center0[2], sp.radius);
+    b[k] = make_float4(__fsub_rz(sp.center1[0], sp.center0[0]), __fsub_rz(sp.center1[1], sp.center0[1]),
+                       __fsub_rz(sp.center1[2], sp.center0[2]), sp.time0);
+    c[k] = make_uint4(__float_as_uint(__fsub_rn(sp.time1, sp.time0)), sp.material, sp.id, i);
+}
+
+// ---- the emitter list, derived on the device at creation and after every update ----
+
+// flag[list ordinal] = 1 when the sphere's material is an emitter
+__global__ void __launch_bounds__(256) k_emitter_flags(const uint4* __restrict__ sph_c, uint32_t n, const DMaterial* __restrict__ mats,
+                                                       uint32_t* __restrict__ flag) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const uint4 c = sph_c[k];
+    flag[c.w] = mats[c.y].kind == RT_MAT_EMITTER ? 1u : 0u;
+}
+
+// lights[rank] = device index of the emitter of that rank in list order (pos: the exclusive sum of the flags), first
+// RT_MAX_LIGHTS only
+__global__ void __launch_bounds__(256) k_lights(const uint4* __restrict__ sph_c, uint32_t n, const DMaterial* __restrict__ mats,
+                                                const uint32_t* __restrict__ pos, uint32_t* __restrict__ lights) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const uint4 c = sph_c[k];
+    if (mats[c.y].kind == RT_MAT_EMITTER && pos[c.w] < RT_MAX_LIGHTS) lights[pos[c.w]] = k;
+}
+
+uint32_t blocks(uint32_t n) { return (n + 255) / 256; }
+
+// the emitter spheres for RT_RENDER_EMITTER_SAMPLING (DScene::lights: device indices, the first RT_MAX_LIGHTS in list
+// order) from the device records and materials; returns after one read-back of the list
+rt_status find_lights(rt_scene* s, cudaStream_t st) {
+    DScene& d = s->d;
+    const uint32_t n = d.n_spheres;
+    d.n_lights = 0;
+    for (uint32_t k = 0; k < RT_MAX_LIGHTS; ++k) d.lights[k] = 0;
+    if (n == 0) return RT_OK;
+    PoolBuffer<uint32_t> buf; // flags, scan scratch, the list
+    const size_t scratch = prims::scan_scratch_elems(n);
+    CUDA_TRY(buf.alloc(n + scratch + RT_MAX_LIGHTS, st));
+    uint32_t* flag = buf.get();
+    uint32_t* lights = flag + n + scratch;
+    CUDA_TRY(cudaMemsetAsync(lights, 0xFF, RT_MAX_LIGHTS * sizeof(uint32_t), st)); // unused entries: all ones
+    k_emitter_flags<<<blocks(n), 256, 0, st>>>(d.sph_c, n, d.mats, flag);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(prims::exclusive_sum<uint32_t>(flag, flag, n, flag + n, st));
+    k_lights<<<blocks(n), 256, 0, st>>>(d.sph_c, n, d.mats, flag, lights);
+    CUDA_TRY(cudaGetLastError());
+    uint32_t h[RT_MAX_LIGHTS];
+    CUDA_TRY(cudaMemcpyAsync(h, lights, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    while (d.n_lights < RT_MAX_LIGHTS && h[d.n_lights] != ~0u) {
+        d.lights[d.n_lights] = h[d.n_lights];
+        ++d.n_lights;
+    }
+    return RT_OK;
+}
+
+// the constant-bank copy of a brute-force list scene (DScene::lst_*) from the device records
+rt_status read_list(rt_scene* s, cudaStream_t st) {
+    DScene& d = s->d;
+    if (d.n_list == 0) return RT_OK;
+    float4 a[RT_LIST_MAX], b[RT_LIST_MAX];
+    uint4 c[RT_LIST_MAX];
+    CUDA_TRY(cudaMemcpyAsync(a, d.sph_a, d.n_list * sizeof(float4), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(b, d.sph_b, d.n_list * sizeof(float4), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(c, d.sph_c, d.n_list * sizeof(uint4), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    for (uint32_t k = 0; k < d.n_list; ++k) {
+        d.lst_a[k] = a[k];
+        d.lst_b[k] = b[k];
+        memcpy(&d.lst_dt[k], &c[k].x, 4);
+    }
+    return RT_OK;
 }
 
 // the padded box of a sphere, over its whole motion when it moves
@@ -354,18 +497,14 @@ rt_status check_edit(const rt_context* ctx, const rt_scene* s, const rt_scene_ed
     ARG_CHECK(s->ctx == ctx, "the scene belongs to another context");
     ARG_CHECK(e->n_spheres == 0 || (e->sphere_index && e->spheres), "sphere_index/spheres is NULL");
     ARG_CHECK(e->n_materials == 0 || (e->material_index && e->materials), "material_index/materials is NULL");
-    const uint32_t n = s->d.n_spheres, n_mat = uint32_t(s->material_kind.size());
+    const uint32_t n = s->d.n_spheres, n_mat = s->n_materials;
     std::vector<bool> seen(e->n_spheres ? n : 0);
     for (uint32_t j = 0; j < e->n_spheres; ++j) {
         const uint32_t i = e->sphere_index[j];
-        ARG_CHECK(i < n, "sphere index out of range");
-        ARG_CHECK(!seen[i], "sphere index repeated");
+        const bool in = i < n;
+        const uint32_t r = sphere_edit_rule(e->spheres[j], i, n, in && seen[i], in && s->where[i] >= s->d.n_static, n_mat);
+        ARG_CHECK(r == SPH_OK, kSphereRuleMessage[r]);
         seen[i] = true;
-        // static spheres are stored before the moving ones: a sphere keeps its kind
-        ARG_CHECK(((e->spheres[j].flags & RT_SPHERE_MOVING) != 0) == (s->where[i] >= s->d.n_static),
-                  "an edit cannot make a static sphere moving or a moving one static");
-        const rt_status st = check_sphere(e->spheres[j], n_mat);
-        if (st != RT_OK) return st;
     }
     seen.assign(e->n_materials ? n_mat : 0, false);
     for (uint32_t j = 0; j < e->n_materials; ++j) {
@@ -414,15 +553,41 @@ rt_status upload_records(rt_scene* s, const rt_scene_edit* e, cudaStream_t st) {
         launch_scatter<DMaterial>(d_mats.get(), d_idx.get() + m, k, const_cast<DMaterial*>(s->d.mats), st);
     }
     CUDA_TRY(cudaGetLastError());
-    // the brute-force list's copy in the kernel parameters
-    for (uint32_t j = 0; j < m && s->d.n_list; ++j) {
-        const uint32_t i = idx[j];
-        s->d.lst_a[i] = a[j];
-        s->d.lst_b[i] = b[j];
-        memcpy(&s->d.lst_dt[i], &c[j].x, 4);
-    }
     // the host copy of the records goes out of scope: the copies from it must have been made
     CUDA_TRY(cudaStreamSynchronize(st));
+    return RT_OK;
+}
+
+// The sphere records of rt_scene_update_device, from device memory: checked on the device (the verdict comes back in one
+// copy; nothing of the scene is written before it), then packed and scattered.
+rt_status apply_device_records(rt_scene* s, const uint32_t* idx, const rt_sphere* spheres, uint32_t m, cudaStream_t st) {
+    DScene& d = s->d;
+    const uint32_t n = d.n_spheres;
+    ARG_CHECK(n != 0, kSphereRuleMessage[SPH_INDEX_RANGE]); // (every index of an edit of an empty scene is out of range)
+    if (!s->where_dev) { // first device update of this scene: list ordinal -> device index, kept with the scene
+        void* p = nullptr;
+        CUDA_TRY(cudaMallocFromPoolAsync(&p, size_t(n) * sizeof(uint32_t), s->ctx->pool, st));
+        s->allocs.push_back(p);
+        s->where_dev = static_cast<uint32_t*>(p);
+        k_where<<<blocks(n), 256, 0, st>>>(d.sph_c, n, s->where_dev);
+        CUDA_TRY(cudaGetLastError());
+    }
+    PoolBuffer<unsigned long long> verdict;
+    PoolBuffer<uint32_t> claim;
+    CUDA_TRY(verdict.alloc(1, st));
+    CUDA_TRY(claim.alloc(n, st));
+    CUDA_TRY(cudaMemsetAsync(verdict.get(), 0xFF, sizeof(unsigned long long), st));
+    CUDA_TRY(cudaMemsetAsync(claim.get(), 0xFF, size_t(n) * sizeof(uint32_t), st));
+    k_claim<<<blocks(m), 256, 0, st>>>(idx, m, n, claim.get());
+    k_check<<<blocks(m), 256, 0, st>>>(idx, spheres, m, n, d.n_static, s->n_materials, claim.get(), s->where_dev, verdict.get());
+    CUDA_TRY(cudaGetLastError());
+    unsigned long long v = 0;
+    CUDA_TRY(cudaMemcpyAsync(&v, verdict.get(), sizeof(v), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    ARG_CHECK(v == ~0ull, kSphereRuleMessage[v & 0xFF]);
+    k_apply<<<blocks(m), 256, 0, st>>>(idx, spheres, m, s->where_dev, const_cast<float4*>(d.sph_a), const_cast<float4*>(d.sph_b),
+                                       const_cast<uint4*>(d.sph_c));
+    CUDA_TRY(cudaGetLastError());
     return RT_OK;
 }
 
@@ -446,12 +611,33 @@ rt_status refit(rt_scene* s, cudaStream_t st) {
     return derive_forms(s, s->info.bvh_depth, st);
 }
 
+// The update both entries share: `write_records(stream)` enqueues the writes of the edit's records (or refuses the edit
+// before it writes anything), then the refit when spheres changed, inside the window ms_device times; then the host state
+// that depends on the records: the constant-bank list and the emitter list.  Returns when the update is complete.
+template <class WriteRecords>
+rt_status apply_update(rt_scene* s, bool spheres, WriteRecords&& write_records, float* ms_device) {
+    const cudaStream_t st = s->ctx->stream;
+    TimingEvent e0, e1;
+    CUDA_TRY(e0.create());
+    CUDA_TRY(e1.create());
+    CUDA_TRY(cudaEventRecord(e0.ev, st));
+    rt_status rs = write_records(st);
+    if (rs != RT_OK) return rs;
+    if (spheres && s->d.nodes && (rs = refit(s, st)) != RT_OK) return rs;
+    CUDA_TRY(cudaEventRecord(e1.ev, st));
+    CUDA_TRY(cudaEventSynchronize(e1.ev)); // (the reads below may enqueue nothing: a scene without spheres)
+    if (spheres && (rs = read_list(s, st)) != RT_OK) return rs;
+    if ((rs = find_lights(s, st)) != RT_OK) return rs;
+    if (ms_device) CUDA_TRY(cudaEventElapsedTime(ms_device, e0.ev, e1.ev));
+    return RT_OK;
+}
+
 } // namespace
 
 // every parameter of a camera finite (scene descriptions, frame sequences, rt_orbit_cameras)
 bool camera_finite(const rt_camera& c) {
-    return finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && std::isfinite(c.vfov) && std::isfinite(c.aspect) &&
-           std::isfinite(c.aperture) && std::isfinite(c.focus_dist) && std::isfinite(c.time0) && std::isfinite(c.time1);
+    return finite3(c.lookfrom) && finite3(c.lookat) && finite3(c.up) && finite1(c.vfov) && finite1(c.aspect) && finite1(c.aperture) &&
+           finite1(c.focus_dist) && finite1(c.time0) && finite1(c.time1);
 }
 
 } // namespace rtd
@@ -520,19 +706,14 @@ extern "C" rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc,
     if (s->d.nodes && (st = derive_forms(s, tree.stats.depth, stream)) != RT_OK) return st;
     if ((st = upload_materials(s, desc, stream)) != RT_OK) return st;
     if ((st = upload_images(s, desc, stream)) != RT_OK) return st;
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    CUDA_TRY(cudaGetLastError());
 
     // ---- what the kernels read besides the device arrays, the mirrors rt_scene_update needs, and the scene's info ----
-    s->d.n_list = 0;
-    if (mode == RT_BVH_NONE && n != 0 && n <= RT_LIST_MAX) { // the list in the constant bank (DScene::lst_*)
-        s->d.n_list = n;
-        for (uint32_t k = 0; k < n; ++k) {
-            s->d.lst_a[k] = ha[k];
-            s->d.lst_b[k] = hb[k];
-            memcpy(&s->d.lst_dt[k], &hc[k].x, 4);
-        }
-    }
+    // the list in the constant bank (DScene::lst_*) and the emitter list come from the device records, as after an update
+    s->d.n_list = mode == RT_BVH_NONE && n <= RT_LIST_MAX ? n : 0;
+    if ((st = read_list(s, stream)) != RT_OK) return st;
+    if ((st = find_lights(s, stream)) != RT_OK) return st;
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    CUDA_TRY(cudaGetLastError());
     s->d.has_noise = 0;
     for (uint32_t i = 0; i < desc->n_textures; ++i) {
         const uint32_t kind = desc->textures[i].kind;
@@ -541,12 +722,8 @@ extern "C" rt_status rt_scene_create(rt_context* ctx, const rt_scene_desc* desc,
     make_camera(desc->camera, s->d.cam);
     s->where.resize(n); // list ordinal -> device index
     for (uint32_t k = 0; k < n; ++k) s->where[order[k]] = k;
-    s->sphere_material.resize(n);
-    for (uint32_t i = 0; i < n; ++i) s->sphere_material[i] = desc->spheres[i].material;
-    s->material_kind.resize(desc->n_materials);
-    for (uint32_t i = 0; i < desc->n_materials; ++i) s->material_kind[i] = desc->materials[i].kind;
+    s->n_materials = desc->n_materials;
     s->n_textures = desc->n_textures;
-    find_lights(s);
 
     const auto t_end = std::chrono::steady_clock::now();
     s->info.n_spheres = n;
@@ -599,19 +776,30 @@ extern "C" rt_status rt_scene_update(rt_context* ctx, rt_scene* scene, const rt_
     if (edit->camera) make_camera(*edit->camera, scene->d.cam);
     if (edit->n_spheres == 0 && edit->n_materials == 0) return RT_OK;
     if ((st = make_current(ctx)) != RT_OK) return st;
-    const cudaStream_t stream = ctx->stream;
-    TimingEvent e0, e1;
-    CUDA_TRY(e0.create());
-    CUDA_TRY(e1.create());
-    CUDA_TRY(cudaEventRecord(e0.ev, stream));
-    if ((st = upload_records(scene, edit, stream)) != RT_OK) return st;
-    if (edit->n_spheres && scene->d.nodes && (st = refit(scene, stream)) != RT_OK) return st;
-    CUDA_TRY(cudaEventRecord(e1.ev, stream));
-    CUDA_TRY(cudaEventSynchronize(e1.ev));
-    if (ms_device) CUDA_TRY(cudaEventElapsedTime(ms_device, e0.ev, e1.ev));
-    for (uint32_t j = 0; j < edit->n_spheres; ++j) scene->sphere_material[edit->sphere_index[j]] = edit->spheres[j].material;
-    for (uint32_t j = 0; j < edit->n_materials; ++j) scene->material_kind[edit->material_index[j]] = edit->materials[j].kind;
-    find_lights(scene);
-    return RT_OK;
+    return apply_update(scene, edit->n_spheres != 0, [&](cudaStream_t s) { return upload_records(scene, edit, s); }, ms_device);
+}
+RT_API_CATCH
+
+extern "C" rt_status rt_scene_update_device(rt_context* ctx, rt_scene* scene, const uint32_t* sphere_index_dev,
+                                            const rt_sphere* spheres_dev, uint32_t n_spheres, float* ms_device) try {
+    if (ms_device) *ms_device = 0.f;
+    ARG_CHECK(ctx && scene, "ctx/scene is NULL");
+    ARG_CHECK(n_spheres == 0 || (sphere_index_dev && spheres_dev), "sphere_index_dev/spheres_dev is NULL");
+    ARG_CHECK(scene->ctx == ctx, "the scene belongs to another context");
+    if (n_spheres == 0) return RT_OK;
+    rt_status st = make_current(ctx);
+    if (st != RT_OK) return st;
+    // a pointer no kernel of ctx's device may read is refused here, never handed to a kernel
+    for (const void* p : {static_cast<const void*>(sphere_index_dev), static_cast<const void*>(spheres_dev)}) {
+        cudaPointerAttributes at{};
+        const cudaError_t e = cudaPointerGetAttributes(&at, p);
+        if (e != cudaSuccess) cudaGetLastError(); // (clears the error: the call only asked)
+        ARG_CHECK(e == cudaSuccess && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == ctx->device,
+                  "sphere_index_dev/spheres_dev is not device or managed memory of the context's device");
+    }
+    ARG_CHECK(reinterpret_cast<uintptr_t>(spheres_dev) % 16 == 0, "spheres_dev is not 16-byte aligned");
+    ARG_CHECK(reinterpret_cast<uintptr_t>(sphere_index_dev) % 4 == 0, "sphere_index_dev is not 4-byte aligned");
+    return apply_update(
+        scene, true, [&](cudaStream_t s) { return apply_device_records(scene, sphere_index_dev, spheres_dev, n_spheres, s); }, ms_device);
 }
 RT_API_CATCH
