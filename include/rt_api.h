@@ -86,6 +86,9 @@ enum {
                                         * the path value is weighted by p_reference / p_mixture (<= 2), so the image
                                         * converges to the frame rendered without the flag */
 #define RT_MAX_LIGHTS 16u             /* emitter spheres that are importance-sampled (first ones in list order) */
+#define RT_MAX_CHECKER_DEPTH 8        /* checker levels a texture may nest (checker of a checker ...) above its leaf; the
+                                       * shading code resolves at most this many, and rt_scene_create refuses deeper
+                                       * chains (RT_ERR_UNSUPPORTED) and cycles (RT_ERR_INVALID_ARG) */
 
 #define RT_SPHERE_MOVING 1u /* built by moving_sphere(...) (sphere.h:30-58) */
 #define RT_SPHERE_INSIDE 2u /* sphere(..., inside=true); stored, no effect (sphere.h:27,133-138) */
@@ -109,6 +112,10 @@ typedef struct rt_material {
     float param;     /* metal: roughness (clamped to <=1 at construction); dielectric: ri; emitter: intensity */
 } rt_material;
 
+/* A checker's children may be checkers themselves (texture.h:41-48 recurses).  rt_scene_create checks every texture of
+ * the description, used or not: a chain of more than RT_MAX_CHECKER_DEPTH checker levels is RT_ERR_UNSUPPORTED (the
+ * reference renders it; this library declines it rather than render it wrong), a checker that reaches itself is
+ * RT_ERR_INVALID_ARG (the reference cannot render it).  Both messages name the texture. */
 typedef struct rt_texture {
     uint32_t kind;   /* RT_TEX_* */
     int32_t even;    /* checker: texture index used when sines >= 0 */

@@ -269,7 +269,9 @@ float turbulence(V3 p) { // perlin_noise.h:142-153, defaults lacunacity 2, gain 
 // ------------------------------------------------------------------ textures (texture.h) ----
 V3 texture_value(const orc_scene& sc, int32_t ix, float u, float v, V3 p) {
     const rt_texture* t = &sc.textures[size_t(ix)];
-    for (int guard = 0; guard < 64 && t->kind == RT_TEX_CHECKER; ++guard) { // checker_texture::value (texture.h:41-48)
+    // checker_texture::value (texture.h:41-48), as far as the product resolves it: rt_scene_create refuses deeper chains and
+    // cycles, so a description it accepts never reaches the guard
+    for (int guard = 0; guard < RT_MAX_CHECKER_DEPTH && t->kind == RT_TEX_CHECKER; ++guard) {
         float sines = sinf(10 * p.x) * sinf(10 * p.y) * sinf(10 * p.z);
         t = &sc.textures[size_t(sines < 0.f ? t->odd : t->even)];
     }

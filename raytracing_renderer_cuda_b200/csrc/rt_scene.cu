@@ -89,6 +89,38 @@ rt_status check_sphere(const rt_sphere& sp, uint32_t n_materials) {
     return RT_OK;
 }
 
+// depth[i] = the checker levels above the leaves of texture i (0 for a leaf), by one depth-first walk over every texture
+// (children already checked in range).  The stack holds the path being walked, so a child on it closes a cycle.
+rt_status checker_depths(const rt_texture* t, uint32_t n, std::vector<uint32_t>& depth) {
+    enum : uint8_t { NEW, ON_PATH, DONE };
+    std::vector<uint8_t> state(n, NEW);
+    std::vector<uint32_t> path;
+    depth.assign(n, 0);
+    for (uint32_t root = 0; root < n; ++root) {
+        if (state[root] != NEW) continue;
+        path.push_back(root);
+        while (!path.empty()) {
+            const uint32_t i = path.back();
+            state[i] = ON_PATH;
+            if (t[i].kind == RT_TEX_CHECKER) {
+                const uint32_t even = uint32_t(t[i].even), odd = uint32_t(t[i].odd);
+                if (state[even] == ON_PATH || state[odd] == ON_PATH) {
+                    set_error("invalid argument: checker texture %u is its own descendant (a checker cycle)", i);
+                    return RT_ERR_INVALID_ARG;
+                }
+                if (state[even] == NEW || state[odd] == NEW) {
+                    path.push_back(state[even] == NEW ? even : odd);
+                    continue;
+                }
+                depth[i] = 1 + std::max(depth[even], depth[odd]);
+            }
+            state[i] = DONE;
+            path.pop_back();
+        }
+    }
+    return RT_OK;
+}
+
 rt_status validate_desc(const rt_scene_desc* d) {
     ARG_CHECK(d != nullptr, "desc is NULL");
     ARG_CHECK(d->n_spheres == 0 || d->spheres, "spheres is NULL");
@@ -107,11 +139,19 @@ rt_status validate_desc(const rt_scene_desc* d) {
                       "checker child out of range");
         if (t.kind == RT_TEX_IMAGE) ARG_CHECK(t.image >= 0 && uint32_t(t.image) < d->n_images, "image index out of range");
     }
-    rt_status st = RT_OK;
+    std::vector<uint32_t> depth;
+    rt_status st = checker_depths(d->textures, d->n_textures, depth);
     for (uint32_t i = 0; i < d->n_materials && st == RT_OK; ++i) st = check_material(d->materials[i], d->n_textures);
     for (uint32_t i = 0; i < d->n_spheres && st == RT_OK; ++i) st = check_sphere(d->spheres[i], d->n_materials);
     if (st != RT_OK) return st;
     ARG_CHECK(camera_finite(d->camera), "camera parameter is not finite");
+    // resolve_texture (rt_shade.cuh) follows RT_MAX_CHECKER_DEPTH levels; the reference renders deeper chains, so they are
+    // declined rather than rendered wrong (as trees deeper than RT_BVH_STACK_DEPTH are)
+    for (uint32_t i = 0; i < d->n_textures; ++i)
+        if (depth[i] > RT_MAX_CHECKER_DEPTH) {
+            set_error("texture %u nests %u checker levels, more than RT_MAX_CHECKER_DEPTH (%d)", i, depth[i], RT_MAX_CHECKER_DEPTH);
+            return RT_ERR_UNSUPPORTED;
+        }
     return RT_OK;
 }
 

@@ -137,10 +137,11 @@ RT_DEV DTexture load_tex(const DScene& sc, int32_t ix) {
 }
 
 // checker_texture::value (texture.h:41-48) only selects a child from p; children may be
-// checkers themselves.  Returns the index of the leaf texture and loads it into `t`.
+// checkers themselves.  Returns the index of the leaf texture and loads it into `t`.  rt_scene_create refuses chains
+// deeper than RT_MAX_CHECKER_DEPTH and cycles, so the loop always ends on a leaf.
 RT_DEV int32_t resolve_texture(const DScene& sc, int32_t ix, V3 p, DTexture& t) {
     t = load_tex(sc, ix);
-    for (int guard = 0; guard < 8 && t.kind == RT_TEX_CHECKER; ++guard) {
+    for (int guard = 0; guard < RT_MAX_CHECKER_DEPTH && t.kind == RT_TEX_CHECKER; ++guard) {
         float sines = __sinf(10 * p.x) * __sinf(10 * p.y) * __sinf(10 * p.z);
         ix = sines < 0.f ? t.odd : t.even;
         t = load_tex(sc, ix);

@@ -118,7 +118,7 @@ def test_random_scene_frame_matches_the_oracle_with_the_same_random_numbers(ctx,
     yardstick is tests/test_random_scene_sensitivity.py: the ORACLE against itself with round-to-nearest instead of
     round-toward-zero vector operators differs in 8.7 % / 0.55 % of the same scene's pixels and in <= 0.2 % of the others' —
     the scene is that sensitive to one ulp, whoever computes it; one shading step agrees ray by ray for every material of
-    it (tools/random_scene_probe.py: attenuation within 2.4e-5, no discrete flips, hits bit-identical)."""
+    it (tests/test_gpu_shading.py::test_random_documents_step_by_step)."""
     d = rt.SceneDesc.from_json(random_document(seed, n))
     w, h, spp = 64, 48, 6
     p = rt.default_params(width=w, height=h, spp=spp, tmin=1e-3, max_depth=max_depth)
